@@ -2,7 +2,7 @@
 """bench.py -- learner-side PPO throughput (GAE + normalisation + full update) of rlgym_ppo_b200 on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3]
-                    [--precision bf16|fp32] [--device cpu|cuda] [--no-cpu] [--no-sub]
+                    [--precision bf16|fp32] [--device cpu|cuda] [--no-cpu] [--no-sub] [--dump-outputs DIR]
 
 One "step" = one learner iteration at steady state on synthetic rollouts of the example shape (SURVEY.md 8d):
 Learner.add_new_experience on N_new fresh timesteps (value inference on N_new+1 states, GAE + reward normalisation,
@@ -23,6 +23,11 @@ steps: permutation gather, fwd/bwd, clip, Adam).
   cpu_baseline  the UNMODIFIED reference (baseline/_ref, pip-installed by build()) on this box's host cores, bounded
             sample (rank 0, N=1 only).
 
+The headline and the precision_fp32, c3 and strong sub-records time exactly --steps learner iterations each (c4 times its
+245 ticks, c5 its sweep).  `--dump-outputs DIR` writes what the last
+device-timed step handed its caller (see dump_outputs) as DIR/<name>.npy; the inputs depend on the arguments only, so two
+builds can be compared output for output.  The benchmark writes nothing into the source tree.
+
 `--impl reference` times that reference alone (all host threads; `--device cuda`: PyTorch eager on the B200, the same-box
 GPU comparator of BASELINE.md section 3) on this arm's config and prints the same JSON line.
 Multi-GPU (torchrun, one rank per GPU): weak scaling -- every rank contributes N_new timesteps and takes 1/R of every
@@ -39,6 +44,7 @@ from types import SimpleNamespace
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # the source tree may be read-only, and a run leaves nothing in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -302,6 +308,27 @@ class Rig:
         return {"rows_per_update": wl["batch"], "n_new": wl["n_new"], "n_params": n_params}
 
 
+def dump_outputs(rig, report, out_dir):
+    """What one step hands its caller, as out_dir/<name>.npy: the report's metrics (float64; the wall-clock
+    "PPO Batch Consumption Time" is not a result and is left out), both networks' updated parameters (float32) and the
+    value targets and advantages add_new_experience computed for the step's rollout (the newest n_new buffer rows).
+    The inputs are the same from run to run, the outputs are not bit-identical: weight gradients are summed with float
+    atomics, and Adam carries those last-bit differences forward.  Two runs of one build with --steps 20 --warmup 3
+    (26 learner iterations; B200 at its 1000 W power limit) differed by up to 1.1e-2 relative L2 on a weight tensor,
+    2.2e-3 on the advantages and 6.4e-3 relative on a report metric (the clip fraction)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"report." + k.lower().replace(" ", "_"): np.float64(v) for k, v in report.items()
+              if k != "PPO Batch Consumption Time"}
+    for net, module in (("policy", rig.ppo.policy), ("value_net", rig.ppo.value_net)):
+        for k, t in module.state_dict().items():
+            arrays[f"{net}.{k}"] = t.detach().float().cpu().numpy()
+    buf = rig.ns.experience_buffer
+    for field in ("values", "advantages"):
+        arrays["buffer." + field] = getattr(buf, field)[-rig.wl["n_new"]:].cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def gae_sweep(dev, peaks, log2s=(20, 22, 24, 26, 28), reps=5):
     """BASELINE configs[4] (C5): flat rollouts with random done masks, 28 algorithmic bytes per step, CUDA events around
     the C-ABI call, median of `reps`; inputs of 2^24 steps and more exceed the 126 MB L2."""
@@ -344,7 +371,7 @@ def sub_fp32(args, dev, rank, world, flush_buf, peaks):
     wl = WORKLOADS["c2"]
     rig = Rig(wl, dev, rank, world, "fp32")
     rig.fill_and_warm(3)
-    K = min(args.steps, 10)
+    K = args.steps
     dev_ms, _ = rig.timed_device(K, flush_buf)
     e2e_ms = rig.timed_e2e(K, 3)
     dev_ms, e2e_ms = rig.max_over_ranks(dev_ms, e2e_ms)
@@ -369,7 +396,7 @@ def sub_c3(args, dev, rank, world, flush_buf, peaks):
     wl = WORKLOADS["c3"]
     rig = Rig(wl, dev, rank, world, "bf16", n_pool=2)
     rig.fill_and_warm(2)
-    K = 2
+    K = args.steps
     dev_ms, _ = rig.timed_device(K, flush_buf)
     (dev_ms,) = rig.max_over_ranks(dev_ms)
     n_updates = wl["epochs"] * (wl["buffer"] // wl["batch"])
@@ -468,7 +495,7 @@ def sub_strong(args, dev, rank, world, flush_buf):
     wl = WORKLOADS["c2"]
     rig = Rig(wl, dev, rank, world, args.precision, dp_mode="replicated")
     rig.fill_and_warm(3)
-    K = min(args.steps, 10)
+    K = args.steps
     dev_ms, _ = rig.timed_device(K, flush_buf)
     e2e_ms = rig.timed_e2e(K, 3)
     dev_ms, e2e_ms = rig.max_over_ranks(dev_ms, e2e_ms)
@@ -511,6 +538,8 @@ def b200_arm(args, wl):
     calls0 = _lib.CALLS
     dev_ms, report = rig.timed_device(args.steps, flush_buf)
     calls = _lib.CALLS - calls0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(rig, report, args.dump_outputs)
     # ---- (2) end to end through the public API with host buffers ---------------------------------------------------
     e2e_ms = rig.timed_e2e(args.steps, n_warm)
     clocks = sampler.stop() if sampler else None
@@ -645,7 +674,12 @@ def main():
     ap.add_argument("--device", default="cpu", choices=["cpu", "cuda"], help="--impl reference: where the reference runs")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-sub", action="store_true", help="skip the sub-records (other configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last device-timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of this project's timed path (--impl b200)")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         reference_arm(args, wl)
