@@ -316,7 +316,8 @@ int rlppo_head_continuous_sample(const uint16_t* z, int64_t ldz, int z_parts, in
  *   rlppo_head_continuous_backward: d_logp, d_ent (mean over M*n elements, ref_oracle.py:473-478) and get_output's
  *     d_mean / d_std f32[M, n], back through the affine map of the std half and the Tanh.
  *   rlppo_value_head_backward[_split]: rlppo_value_head's training pass with dv = d_values[row] loaded:
- *     dH = dv * w (.) (H > 0);  dw[K] += sum_m dv*H;  db[1] += sum dv. */
+ *     dH = dv * w (.) (H > 0);  dw[K] += sum_m dv*H;  db[1] += sum dv.  d_values is the head's only upstream gradient
+ *     and is required (NULL: RLPPO_ERR_ARG); db may be NULL. */
 int rlppo_policy_head_backward(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
                                int64_t M, int n_actions, int K, const float* actions, const float* d_logp,
                                const float* d_ent, const float* d_probs, uint16_t* dz, int64_t lddz, void* stream);
