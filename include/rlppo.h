@@ -353,14 +353,18 @@ typedef struct rlppo_fused_net {
     int in_dim;                 /* observation width (<= 256) */
     int64_t in_ld;              /* row stride of x in elements (multiple of 8) */
     int hidden[4];              /* hidden widths */
-    const uint16_t* wq[5];      /* forward operands W_l bf16 [out_pad8, ld]; [n_hidden] = policy head (NULL for value) */
+    const uint16_t* wq[5];      /* forward operands W_l bf16 [out_pad8, ld]; [n_hidden] = policy head (NULL for value).
+                                   Columns past in_features are never read.  The head's rows n_actions .. out_pad8-1
+                                   are read and must be finite; no output depends on their values */
     int64_t wq_ld[5];
     const uint16_t* wt[5];      /* unused (kept for layout): the backward data GEMMs read wq[l] as an MN-major operand */
     int64_t wt_ld[5];
     const float* bias[5];       /* f32 biases; [n_hidden] = head bias (policy: n_actions, value: 1) */
     float* gbias[5];            /* only [n_hidden] of the value net (its head's scalar bias gradient) is written here;
                                    every other bias gradient comes from rlppo_wgrad_multi (item.db) */
-    uint16_t* h[4];             /* out (training): H_l bf16 [M, hidden_l], ld h_ld */
+    uint16_t* h[4];             /* out (training): H_l bf16 [M, hidden_l], ld h_ld.  Except the value net's
+                                   h[n_hidden-1]: that activation feeds only the in-kernel value head, so it is never
+                                   written and may be NULL */
     int64_t h_ld[4];
     uint16_t* dh[4];            /* out (training): dL/dH_l (ReLU-masked) bf16 [M, hidden_l] */
     int64_t dh_ld[4];
