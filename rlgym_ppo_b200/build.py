@@ -16,7 +16,7 @@ STAMP = os.path.join(HERE, "csrc", ".build_stamp")
 SOURCES = ["common.cu", "gae_scan.cu", "stats_ring.cu", "optim.cu", "mlp_tcgen05.cu", "mlp_fused.cu", "value_head.cu", "heads.cu", "host_rng.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]
-NVCC_FLAGS += os.environ.get("RLPPO_NVCC_EXTRA", "").split()     # experiments only (e.g. -DRLPPO_FINE_TRACE)
+NVCC_FLAGS += os.environ.get("RLPPO_NVCC_EXTRA", "").split()     # e.g. -DRLPPO_DEBUG_BAR (print the barrier a wait timed out on)
 
 
 def _nvcc():

@@ -31,7 +31,6 @@
 // k-blocks: 64 KB in flight per SM cannot cover the L2 latency) and the epilogue warps idle 27 % of the time.
 #include <type_traits>
 #include <math.h>
-#include <stdlib.h>
 
 #include "tc_common.cuh"
 
@@ -47,7 +46,7 @@ constexpr uint32_t KB_BYTES = TILE_M * KBLK * 2;   // 16 KB: one 64-column k-blo
 constexpr uint32_t ACT_BYTES = 4 * KB_BYTES;       // 64 KB
 constexpr uint32_t WST_BYTES = 256 * KBLK * 2;     // 32 KB: one k-block of a weight operand (<= 256 rows)
 constexpr uint32_t MN_CHUNK = 64 * KBLK * 2;       // 8 KB: 64 k-rows x 64 n-columns of an MN-major weight operand
-constexpr int MAX_NWST = 6;                        // ring stages (3 x 32 KB alone, up to 6 x 16 KB in a CTA pair)
+constexpr int MAX_NWST = 3;                        // weight ring stages of 32 KB
 constexpr int kThreads = 352;
 constexpr int kEpiThreads = 256;
 constexpr int MAXPH = 2 * MAXL + 1;
@@ -62,7 +61,7 @@ constexpr uint32_t ROWX_FLOATS = 1280;
 constexpr uint32_t MISC_DB = MISC_ROWX + ROWX_FLOATS * 4;          // 256 floats: column sums of the value head's weight gradient
 constexpr uint32_t MISC_MASK = MISC_DB + 256 * 4;                  // ReLU bit masks: [MAXL][4 k-blocks][256 threads] words
 constexpr uint32_t MISC_BARS = MISC_MASK + MAXL * 4 * kEpiThreads * 4;
-constexpr uint32_t MISC_BYTES = MISC_BARS + 384;     // 36 mbarriers + the TMEM slot + the item ring
+constexpr uint32_t MISC_BYTES = MISC_BARS + 384;     // 19 mbarriers + the TMEM slot + the item ring
 constexpr uint32_t SMEM_LIMIT = 232448;                            // 227 KB
 static_assert(ACT_BYTES + 2 * KB_BYTES + MISC_BYTES + 1024 + 3 * WST_BYTES <= SMEM_LIMIT,
               "an observation of <= 128 columns must leave room for a 3-stage weight ring (2 stages starve the MMA)");
@@ -123,16 +122,11 @@ struct NetP {
 struct Params {
     int64_t M;
     int num_tiles, in_kb, nwst;
-    int pair;                    // 1: launched as 2-CTA clusters (cta_group::2): see fused_mlp_kernel
-    int n_units;                 // work units per net: tiles, or tile PAIRS when pair
-    uint32_t wst_bytes;          // bytes of one ring stage (a whole weight k-block, or this CTA's half of it)
-    int n_nets;                  // work items = n_nets * num_tiles: item q is tile q % num_tiles of net q / num_tiles
+    int n_units;                 // work units per net: tiles (fused_mlp_kernel), or pairs of tiles (fused_duo_kernel)
+    int n_nets;                  // work items = n_nets * n_units: item q is unit q % n_units of net q / n_units
     NetP net[MAXNET];
     unsigned int* sched;         // [0] next item to hand out, [1] CTAs that have left (the last one zeroes both)
     uint32_t* mask_scratch;      // duo kernel: gridDim.x x 24 KB of ReLU mask words (L2-resident scratch)
-    int dbg_nostore;             // debug (RLPPO_FUSED_NOSTORE=1): timing experiment, outputs are NOT written
-    int dbg;                     // debug (RLPPO_DUO_DBG bits, duo kernel timing experiments, results are WRONG): 1 no MMAs, 2 no weight loads
-    unsigned long long* trace;   // debug (RLPPO_FUSED_TRACE=1): clock64 stamps of CTA 0, [role][event]
 };
 
 // ---- small PTX helpers local to this kernel -------------------------------------------------------------------
@@ -263,64 +257,32 @@ __device__ __forceinline__ void sts_chunk16_sw128(uint8_t* buf, int row, int chu
         *reinterpret_cast<uint4*>(kb + (((base16 + t) ^ (row & 7)) << 4)) = make_uint4(w[4 * t], w[4 * t + 1], w[4 * t + 2], w[4 * t + 3]);
 }
 
-#define RLPPO_TRACE(role, idx)                                                                  \
-    do {                                                                                        \
-        const int _i = (idx);                                                                   \
-        if (p.trace != nullptr && blockIdx.x == 0 && _i < 512) p.trace[(role) * 512 + _i] = clock64(); \
-    } while (0)
-
-// -DRLPPO_FINE_TRACE (experiments): clock stamps inside the epilogue loops of CTA 0's first tile, epilogue warp 2
-#ifdef RLPPO_FINE_TRACE
-#define EPI_T()                                                                                  \
-    do {                                                                                         \
-        if (p.trace != nullptr && blockIdx.x == 0 && it == 0 && warp == 2 && lane == 0 && tr5 < 500) p.trace[5 * 512 + tr5++] = clock64(); \
-    } while (0)
-#else
-#define EPI_T() do { } while (0)
-#endif
-
 struct EpiCtx {
     uint8_t* act;
     float* s_bias;
     float* s_rowx;
     uint32_t* s_mask;     // this thread's column of the mask planes: word (layer * 4 + kb) lives at s_mask[(layer*4+kb) * 256]
     uint64_t* a_ready;    // [4], one per k-block of the activation tile, 8 arrivals (epilogue warps)
-    uint64_t* a_mma;      // CTA pair: the LEADER's [4] barriers the MMA thread waits on (16 arrivals: both CTAs' warps)
-    uint32_t rank;        // CTA rank in the pair (0 = leader)
     int lane, quarter, half, row_in_tile;
 };
 
 // This warp's part of output k-block `kb` is written and its TMEM reads for it are done: one arrival per warp; the MMA
 // thread may then read that k-block as the next GEMM's A operand (and TMA-store it).
-template <bool PAIR>
 __device__ __forceinline__ void release_kb(const EpiCtx& e, int kb) {
     tc_fence_before();
     fence_proxy_async();
     __syncwarp();
-    if (e.lane == 0) {
-        mbar_arrive(e.a_ready + kb);                       // this CTA's store thread (and, alone, its MMA thread)
-        if (PAIR) mbar_arrive_cta(e.a_mma + kb, 0);       // the pair's MMA thread lives in the leader CTA
-    }
+    if (e.lane == 0) mbar_arrive(e.a_ready + kb);          // the store thread and the MMA thread wait on it
 }
 
-// PAIR: the launch consists of 2-CTA clusters.  Both CTAs of a pair run the same item sequence on two different 128-row
-// tiles (tile 2u + rank of unit u); ONE thread of the leader CTA issues tcgen05.mma.cta_group::2 over both tiles (M = 256),
-// and each CTA stages only ITS half of every weight k-block (N/2 rows, or N/2 columns of an MN-major operand): half the
-// L2 -> shared-memory weight traffic and half the operand reads of B per SM -- the fused kernel's epilogues share the
-// shared-memory pipe with exactly that traffic.  Roles per CTA: producer (own x tile, own weight halves), epilogue warps
-// and store thread (own tile, unchanged); warp 1 is the MMA issuer in the leader and a relay in the peer (tells the leader
-// when the peer's operand stages have landed).  Cross-CTA signals: remote mbarrier arrives (epilogue -> a_mma, relay ->
-// pfull / px_full, consumers -> tile_empty), multicast tcgen05.commit (stage free, x free, accumulator full).
-template <bool TRAIN, bool PAIR>
+template <bool TRAIN>
 __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_constant__ Maps maps, const Params p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
     uint8_t* act = smem + OFF_ACT;
     uint8_t* xst = smem + OFF_XST;
     uint8_t* wring = xst + p.in_kb * KB_BYTES;
-    uint8_t* misc = wring + p.nwst * p.wst_bytes;
-    const uint32_t rank = PAIR ? cluster_ctarank() : 0u;
-    const bool leader = rank == 0;
+    uint8_t* misc = wring + p.nwst * WST_BYTES;
     float* s_bias = reinterpret_cast<float*>(misc + MISC_BIAS);
     float* s_rowx = reinterpret_cast<float*>(misc + MISC_ROWX);
     float* s_db = reinterpret_cast<float*>(misc + MISC_DB);
@@ -334,19 +296,10 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
     uint64_t* st_done = acc_full + 2;       // [1]: the TMA stores of a phase's output have finished reading shared memory
     uint64_t* tile_full = st_done + 1;      // [2]: the producer has published the CTA's next tile index
     uint64_t* tile_empty = tile_full + 2;   // [2]: every consumer role has read it
-    uint64_t* a_mma = tile_empty + 2;       // [4] (pair, leader's copy is used): k-block ready in BOTH CTAs
-    uint64_t* pfull = a_mma + 4;            // [MAX_NWST] (pair, leader): the peer's half of ring stage i has landed
-    uint64_t* px_full = pfull + MAX_NWST;   // [1] (pair, leader): the peer's x tile has landed
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(px_full + 1);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tile_empty + 2);
     volatile int* tile_ring = reinterpret_cast<volatile int*>(tmem_slot + 1);   // [2]
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-#ifdef RLPPO_FINE_TRACE
-#define STAMP(slot) do { if (p.trace != nullptr && blockIdx.x == 0) p.trace[5 * 512 + (slot)] = clock64(); } while (0)
-#else
-#define STAMP(slot) do { } while (0)
-#endif
-    if (threadIdx.x == 0) STAMP(500);
     if (threadIdx.x == 0) {
         tma_prefetch_desc(&maps.x);
         for (int i = 0; i < MAX_NWST; ++i) {
@@ -362,19 +315,11 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
         const int consumers = TRAIN ? 10 : 9;           // warp 1's thread, (training) store thread, 8 epilogue warps
         for (int i = 0; i < 2; ++i) {
             mbar_init(&tile_full[i], 1);
-            mbar_init(&tile_empty[i], PAIR ? 2 * consumers + 1 : consumers);   // pair: + the peer's roles and its producer
-        }
-        if (PAIR) {
-            for (int i = 0; i < 4; ++i) mbar_init(&a_mma[i], 16);
-            for (int i = 0; i < MAX_NWST; ++i) mbar_init(&pfull[i], 1);
-            mbar_init(px_full, 1);
+            mbar_init(&tile_empty[i], consumers);
         }
         fence_barrier_init();
     }
-    if (warp == 1) {
-        if (PAIR) tmem_alloc_pair(tmem_slot, 512);
-        else tmem_alloc(tmem_slot, 512);
-    }
+    if (warp == 1) tmem_alloc(tmem_slot, 512);
     // PDL: everything above ran while the previous kernel of the stream was still draining; its outputs (x, parameters)
     // are read from here on.  All CTAs of this grid are resident, so the next kernel may be scheduled as SMs free up.
     pdl_wait();
@@ -401,15 +346,8 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
     for (int i = threadIdx.x; i < 256; i += kThreads) s_db[i] = 0.f;
     tc_fence_before();
     __syncthreads();
-    if (PAIR) cluster_sync_all();       // both CTAs' barriers are initialised before either one signals the other
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    if (threadIdx.x == 0) STAMP(501);
-    // a consumer role has read item slot `slot`: the leader's producer may reuse it once every role of BOTH CTAs has
-    auto ring_done = [&](int slot) {
-        if (leader) mbar_arrive(&tile_empty[slot]);
-        else mbar_arrive_cta(&tile_empty[slot], 0);
-    };
     // Work items (net, tile) are handed out dynamically from a global counter, the first net's tiles first (the policy
     // net's: they take longest, so the launch ends on the cheaper value tiles): 2 x 391 items over 148 CTAs instead of two
     // launches of 391 tiles that each end on a third, 64 %-full round.  The producer thread fetches the next item one
@@ -419,29 +357,16 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
         // ===================== TMA producer =====================
         if (lane == 0) {
             uint32_t ws = 0, wpar = 0;
-            int tr3 = 0;
             for (int it = 0;; ++it) {
                 const int slot = it & 1;
-                int q;
-                if (leader) {
-                    mbar_wait(&tile_empty[slot], ((it >> 1) & 1) ^ 1);
-                    q = (int)atomicAdd(p.sched, 1u);
-                    if (q >= p.n_nets * p.n_units) q = -1;
-                    tile_ring[slot] = q;
-                    mbar_arrive(&tile_full[slot]);
-                    if (PAIR) {                          // the same item for the peer CTA's roles
-                        st_shared_cta_s32(const_cast<int*>(tile_ring) + slot, 1, q);
-                        mbar_arrive_cta_release(&tile_full[slot], 1);
-                    }
-                } else {
-                    mbar_wait(&tile_full[slot], (it >> 1) & 1);
-                    q = tile_ring[slot];
-                    mbar_arrive_cta(&tile_empty[slot], 0);
-                }
+                mbar_wait(&tile_empty[slot], ((it >> 1) & 1) ^ 1);
+                int q = (int)atomicAdd(p.sched, 1u);
+                if (q >= p.n_nets * p.n_units) q = -1;
+                tile_ring[slot] = q;
+                mbar_arrive(&tile_full[slot]);
                 if (q < 0) break;
                 const int ni = q >= p.n_units ? 1 : 0;
-                const int unit = q - ni * p.n_units;
-                const int tile = PAIR ? 2 * unit + (int)rank : unit;      // out-of-range tiles load zeros, store nothing
+                const int tile = q - ni * p.n_units;
                 const NetP& np = p.net[ni];
                 mbar_wait(x_free, (it & 1) ^ 1);          // GEMM 0 of the previous tile has read the staging buffer
                 mbar_expect_tx(x_full, p.in_kb * KB_BYTES);
@@ -449,17 +374,15 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
                     tma_load_2d(&maps.x, x_full, xst + kb * KB_BYTES, kb * KBLK, tile * TILE_M);
                 for (int ph = 0; ph < np.n_ph; ++ph) {
                     const PhaseDesc& d = np.ph[ph];
-                    const int nh = PAIR ? d.N >> 1 : d.N;           // operand rows (columns if MN-major) this CTA stages
                     for (int kb = 0; kb < d.n_kb; ++kb) {
                         mbar_wait(&wempty[ws], wpar ^ 1);
-                        mbar_expect_tx(&wfull[ws], (uint32_t)nh * 128u);
-                        RLPPO_TRACE(3, tr3++);
-                        uint8_t* dst = wring + ws * p.wst_bytes;
+                        mbar_expect_tx(&wfull[ws], (uint32_t)d.N * 128u);
+                        uint8_t* dst = wring + ws * WST_BYTES;
                         if (d.b_mn) {
-                            for (int c = 0; c < (nh >> 6); ++c)
-                                tma_load_2d(&maps.w[ni][d.wmap], &wfull[ws], dst + c * MN_CHUNK, (int)rank * nh + c * 64, kb * KBLK);
+                            for (int c = 0; c < (d.N >> 6); ++c)
+                                tma_load_2d(&maps.w[ni][d.wmap], &wfull[ws], dst + c * MN_CHUNK, c * 64, kb * KBLK);
                         } else {
-                            tma_load_2d(&maps.w[ni][d.wmap], &wfull[ws], dst, kb * KBLK, (int)rank * nh);
+                            tma_load_2d(&maps.w[ni][d.wmap], &wfull[ws], dst, kb * KBLK, 0);
                         }
                         if (++ws == (uint32_t)p.nwst) {
                             ws = 0;
@@ -470,38 +393,11 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
             }
         }
     } else if (warp == 1) {
-        // ===================== MMA issuer (leader) / operand relay (peer of a pair) =====================
-        if (lane == 0 && !leader) {
-            // Peer CTA of a pair: its operand stages are filled by its own producer; tell the leader's MMA thread when each
-            // one has landed (the MMA reads both CTAs' shared memory).  Runs as far ahead as the loads do.
-            uint32_t ws = 0, wpar = 0;
-            for (int it = 0;; ++it) {
-                mbar_wait(&tile_full[it & 1], (it >> 1) & 1);
-                const int q = tile_ring[it & 1];
-                mbar_arrive_cta(&tile_empty[it & 1], 0);
-                if (q < 0) break;
-                const NetP& np = p.net[q >= p.n_units ? 1 : 0];
-                mbar_wait(x_full, it & 1);
-                mbar_arrive_cta(px_full, 0);
-                for (int ph = 0; ph < np.n_ph; ++ph) {
-                    const int n_kb = np.ph[ph].n_kb;
-                    for (int kb = 0; kb < n_kb; ++kb) {
-                        mbar_wait(&wfull[ws], wpar);
-                        mbar_arrive_cta(&pfull[ws], 0);
-                        if (++ws == (uint32_t)p.nwst) {
-                            ws = 0;
-                            wpar ^= 1;
-                        }
-                    }
-                }
-            }
-        }
-        if (lane == 0 && leader) {
+        // ===================== MMA issuer =====================
+        if (lane == 0) {
             uint32_t ws = 0, wpar = 0;
             uint32_t g = 0;                        // GEMMs issued so far: GEMM g accumulates into accumulator g & 1
             uint32_t apar = 0;                     // bit kb: parity of a_ready[kb] to wait for next (registers, not a local array)
-            uint64_t* const a_rdy = PAIR ? a_mma : a_ready;     // pair: k-blocks are ready when BOTH CTAs' warps said so
-            int tr0 = 0, tr4 = 0;
             for (int it = 0;; ++it) {
                 mbar_wait(&tile_full[it & 1], (it >> 1) & 1);
                 const int q = tile_ring[it & 1];
@@ -512,70 +408,55 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
                 for (int ph = 0; ph < np.n_ph; ++ph) {
                     const PhaseDesc& d = np.ph[ph];
                     if (d.n_kb > 0) {
-                        const uint32_t idesc = umma_idesc_bf16(PAIR ? 2 * TILE_M : TILE_M, d.N, 0, d.b_mn);
+                        const uint32_t idesc = umma_idesc_bf16(TILE_M, d.N, 0, d.b_mn);
                         const uint32_t d_tmem = tmem_base + (g & 1u) * 256u;
-                        RLPPO_TRACE(0, tr0++);   // MMA: start of (tile, ph)
                         for (int kb = 0; kb < d.n_kb; ++kb) {
                             uint32_t a_addr;
                             if (ph == 0) {
                                 if (kb == 0) {
                                     mbar_wait(x_full, it & 1);
-                                    if (PAIR) mbar_wait(px_full, it & 1);
                                     tc_fence_after();
-                                    if (it == 0) STAMP(502);
                                 }
                                 a_addr = smem_u32(xst + kb * KB_BYTES);
                             } else {
-                                mbar_wait(&a_rdy[kb], (apar >> kb) & 1u);   // k-block kb of the previous epilogue's output
+                                mbar_wait(&a_ready[kb], (apar >> kb) & 1u);   // k-block kb of the previous epilogue's output
                                 apar ^= 1u << kb;
                                 tc_fence_after();
                                 a_addr = smem_u32(act + kb * KB_BYTES);
                             }
                             mbar_wait(&wfull[ws], wpar);
-                            if (PAIR) mbar_wait(&pfull[ws], wpar);
                             tc_fence_after();
-                            RLPPO_TRACE(4, tr4++);
-                            const uint32_t b_addr = smem_u32(wring + ws * p.wst_bytes);
+                            const uint32_t b_addr = smem_u32(wring + ws * WST_BYTES);
 #pragma unroll
                             for (int k = 0; k < KBLK / 16; ++k) {
                                 const uint64_t ad = umma_smem_desc(a_addr + k * 32, 16, 1024);
                                 const uint64_t bd = d.b_mn ? umma_smem_desc(b_addr + k * (16 * 128), MN_CHUNK, 1024)
                                                            : umma_smem_desc(b_addr + k * 32, 16, 1024);
-                                if (PAIR) umma_bf16_pair(d_tmem, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
-                                else umma_bf16(d_tmem, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
+                                umma_bf16(d_tmem, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
                             }
-                            if (PAIR) umma_commit_pair(&wempty[ws]);
-                            else umma_commit(&wempty[ws]);
+                            umma_commit(&wempty[ws]);
                             if (++ws == (uint32_t)p.nwst) {
                                 ws = 0;
                                 wpar ^= 1;
                             }
                         }
-                        if (ph == 0) {                         // the staging buffers can take the next tiles' x
-                            if (PAIR) umma_commit_pair(x_free);
-                            else umma_commit(x_free);
-                        }
-                        RLPPO_TRACE(0, tr0++);   // MMA: all MMAs of (tile, ph) issued
-                        if (PAIR) umma_commit_pair(&acc_full[g & 1u]);
-                        else umma_commit(&acc_full[g & 1u]);
+                        if (ph == 0) umma_commit(x_free);      // the staging buffer can take the next tile's x
+                        umma_commit(&acc_full[g & 1u]);
                         ++g;
                     } else {
                         // GEMM-less phase (value net: dL/dH_L from the accumulator of the last forward GEMM, still in
                         // TMEM): consume the previous epilogue's releases, then hand the SAME accumulator back
-                        RLPPO_TRACE(0, tr0++);
                         for (int kb = 0; kb < d.wait_kb; ++kb) {
-                            mbar_wait(&a_rdy[kb], (apar >> kb) & 1u);
+                            mbar_wait(&a_ready[kb], (apar >> kb) & 1u);
                             apar ^= 1u << kb;
                         }
-                        RLPPO_TRACE(0, tr0++);
                         mbar_arrive(&acc_full[(g - 1u) & 1u]);
-                        if (PAIR) mbar_arrive_cta(&acc_full[(g - 1u) & 1u], 1);
                     }
                 }
                 // tail: the last epilogue's releases (barrier parity; also: every epilogue warp is done with both
                 // accumulators and the activation tile before the next tile's first GEMM / epilogue touch them)
                 for (int kb = 0; kb < np.tail_rel_kb; ++kb) {
-                    mbar_wait(&a_rdy[kb], (apar >> kb) & 1u);
+                    mbar_wait(&a_ready[kb], (apar >> kb) & 1u);
                     apar ^= 1u << kb;
                 }
             }
@@ -587,29 +468,24 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
         // next epilogue may overwrite that k-block in place.  The MMA thread never waits for stores.
         if (TRAIN && lane == 0) {
             uint32_t apar = 0;
-            int nst = 0;
             for (int it = 0;; ++it) {
                 mbar_wait(&tile_full[it & 1], (it >> 1) & 1);
                 const int q = tile_ring[it & 1];
-                ring_done(it & 1);
+                mbar_arrive(&tile_empty[it & 1]);
                 if (q < 0) break;
                 const int ni = q >= p.n_units ? 1 : 0;
-                const int unit = q - ni * p.n_units;
-                const int tile = PAIR ? 2 * unit + (int)rank : unit;
+                const int tile = q - ni * p.n_units;
                 const NetP& np = p.net[ni];
 #pragma unroll 1
                 for (int ph = 0; ph < np.n_ph; ++ph) {
                     const PhaseDesc& d = np.ph[ph];
                     const bool storing = d.out != NO_STORE;
-                    const bool skip = p.dbg_nostore != 0;
                     for (int kb = 0; kb < d.rel_kb; ++kb) {
                         mbar_wait(&a_ready[kb], (apar >> kb) & 1u);
                         apar ^= 1u << kb;
                         if (!storing) continue;
-                        RLPPO_TRACE(2, 2 * nst);
-                        if (!skip) tma_store_2d(&maps.out[ni][d.out], act + kb * KB_BYTES, kb * KBLK, tile * TILE_M);
+                        tma_store_2d(&maps.out[ni][d.out], act + kb * KB_BYTES, kb * KBLK, tile * TILE_M);
                         bulk_commit();
-                        ++nst;
                     }
                     if (d.rel_kb > 0) {
                         // ONE completion signal per phase, storing or not: the epilogue waits for it before its next phase, so
@@ -617,7 +493,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
                         // The next epilogue starts a whole GEMM (>= 1k cycles) after the last release: the reads are long done
                         if (storing) bulk_wait_read_all();
                         mbar_arrive(st_done);
-                        if (storing) RLPPO_TRACE(2, 2 * (nst - 1) + 1);
                     }
                 }
             }
@@ -631,8 +506,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
         e.s_rowx = s_rowx;
         e.s_mask = s_mask + (threadIdx.x - 64);
         e.a_ready = a_ready;
-        e.a_mma = a_mma;
-        e.rank = rank;
         e.lane = lane;
         e.quarter = warp & 3;
         e.half = (warp - 2) >> 2;
@@ -657,18 +530,14 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
                 pend = 0;
             }
         };
-        int tr1 = 0;
-        int tr5 = 0;
-        (void)tr5;
         for (int it = 0;; ++it) {
           mbar_wait(&tile_full[it & 1], (it >> 1) & 1);
           const int q = tile_ring[it & 1];
           __syncwarp();
-          if (lane == 0) ring_done(it & 1);
+          if (lane == 0) mbar_arrive(&tile_empty[it & 1]);
           if (q < 0) break;
           const int ni = q >= p.n_units ? 1 : 0;
-          const int unit = q - ni * p.n_units;
-          const int tile = PAIR ? 2 * unit + (int)rank : unit;
+          const int tile = q - ni * p.n_units;
           const NetP& np = p.net[ni];
           const float* s_bias_n = s_bias + ni * (int)BIAS_FLOATS;   // this net's bias table
           const int64_t row = (int64_t)tile * TILE_M + e.row_in_tile;
@@ -686,7 +555,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
                 mbar_wait(&acc_full[acc], (fpar >> acc) & 1u);
                 fpar ^= 1u << acc;
                 tc_fence_after();
-                if (warp == 2 && lane == 0) RLPPO_TRACE(1, tr1++);   // epilogue: accumulator of (tile, ph) complete
                 // the tile is overwritten in place: its last stores must have read it (and the store thread has seen every
                 // release of the previous phase)
                 if (TRAIN) wait_stores();
@@ -694,7 +562,7 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
                 uint8_t* dst = act;      // in place: the GEMM that read this tile has completed
                 const int li = d.layer;
 
-#define RLPPO_RELEASE_KB(j) release_kb<PAIR>(e, j)
+#define RLPPO_RELEASE_KB(j) release_kb(e, j)
 #define RLPPO_MASK_ST(l, kb, v) e.s_mask[((l) * 4 + (kb)) * kEpiThreads] = (v)
 #define RLPPO_MASK_LD(l, kb) e.s_mask[((l) * 4 + (kb)) * kEpiThreads]
 #include "fused_epilogue.inc"
@@ -702,7 +570,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
 #undef RLPPO_MASK_LD
 #undef RLPPO_RELEASE_KB
                 if (TRAIN && d.rel_kb > 0) pend = 1u;
-                if (warp == 2 && lane == 0) RLPPO_TRACE(1, tr1++);   // epilogue: (tile, ph) done
           }
         }
         // ---- metrics (the column sums are flushed by the whole CTA below) ----
@@ -733,12 +600,9 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
     }
     tc_fence_before();
     __syncthreads();
-    if (PAIR) cluster_sync_all();       // neither CTA leaves (or frees TMEM) while the other may still signal it / be read by an MMA
-    if (threadIdx.x == 0) STAMP(503);
     if (warp == 1) {
         tc_fence_after();
-        if (PAIR) tmem_dealloc_pair(tmem_base, 512);
-        else tmem_dealloc(tmem_base, 512);
+        tmem_dealloc(tmem_base, 512);
     }
     if (threadIdx.x == 0) {
         // every CTA has drawn its last (out-of-range) index by now: the last CTA to leave re-arms the scheduler words
@@ -762,10 +626,9 @@ __global__ void __launch_bounds__(kThreads, 1) fused_mlp_kernel(const __grid_con
 // ---------------------------------------------------------------------------------------------------------------
 // fused_duo_kernel: CTA pairs with TWO tiles in flight per CTA (training).
 //
-// The single-tile kernels above are a chain per tile: GEMM -> epilogue -> GEMM ..., in which the tensor core waits for the
-// epilogue's k-blocks and the epilogue warps wait for the GEMM's tail (and, in a CTA pair, for a cross-SM round trip) at
-// every phase boundary: ~13 k of a tile's 36 k cycles.  Here every CTA keeps two tiles ("slots") resident, each with its
-// own activation buffer (in place, as before) and its own 256-column TMEM accumulator, and all roles walk the same
+// The single-tile kernel above is a chain per tile: GEMM -> epilogue -> GEMM ..., in which the tensor core waits for the
+// epilogue's k-blocks and the epilogue warps wait for the GEMM's tail at every phase boundary: ~13 k of a tile's 36 k
+// cycles.  Here every CTA keeps two tiles ("slots") resident, each with its own activation buffer (in place, as before) and its own 256-column TMEM accumulator, and all roles walk the same
 // deterministic sequence  step n -> slot n & 1 -> that slot's next phase : while the eight epilogue warps work on one
 // slot, the GEMM of the other slot's next phase runs, so MMA time, weight latency and the pair's signalling latency hide
 // behind an epilogue instead of sitting between two of them.  What makes the second 64 KB buffer fit is the pair: each
@@ -852,11 +715,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
     if (warp == 1) tmem_alloc_pair(tmem_slot, 512);
     pdl_wait();
     pdl_trigger();
-    if (p.trace != nullptr && threadIdx.x == 0) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        p.trace[2048 + 2 * blockIdx.x] = t;      // per-CTA start / end (ns), every CTA
-    }
     for (int i = threadIdx.x; i < p.n_nets * (int)BIAS_FLOATS; i += kThreads) {
         const int ni = i >= (int)BIAS_FLOATS ? 1 : 0;
         const NetP& np = p.net[ni];
@@ -898,10 +756,9 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
         DUO_SET(w, items, s, DUO_SEL(w, items, s) + 1);
         return true;
     };
-#define DUO_WALK_BEGIN(w, traced)                                             \
+#define DUO_WALK_BEGIN(w)                                                     \
     for (int n = 0;; ++n) {                                                   \
         const int s = n & 1;                                                  \
-        if ((traced) && warp == 2 && lane == 0) RLPPO_TRACE(3, 4 * n);        \
         if (!DUO_SEL(w, alive, s)) {                                          \
             if (!DUO_SEL(w, alive, s ^ 1)) break;                             \
             continue;                                                         \
@@ -926,7 +783,7 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
         if (lane == 0) {
             DuoWalk w;
             uint32_t ws = 0, wpar = 0;
-            DUO_WALK_BEGIN(w, false)
+            DUO_WALK_BEGIN(w)
                 if (ph == 0) {
                     // the item's x tile, straight into the slot's activation buffer once the previous item's stores have read
                     // it: item k of the slot (k = items_s - 1) waits for completion k - 1 of x_free
@@ -960,9 +817,7 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
             DuoWalk w;
             uint32_t ws = 0, wpar = 0;
             uint32_t epi_cnt[2] = {0u, 0u};        // phases of slot s issued so far (every one ends with an epilogue)
-            int tr0 = 0;
-            DUO_WALK_BEGIN(w, false)
-                RLPPO_TRACE(0, tr0++);       // step start (before waiting for the slot's previous epilogue)
+            DUO_WALK_BEGIN(w)
                 const uint32_t d_tmem = tmem_base + (uint32_t)s * 256u;
                 uint8_t* act = smem + s * ACT_BYTES;
                 // this slot's previous epilogue, in both CTAs (every completion of a_done[s] is waited for, in order)
@@ -981,7 +836,7 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
                             const uint64_t ad = umma_smem_desc(a_addr + k * 32, 16, 1024);
                             const uint64_t bd = d.b_mn ? umma_smem_desc(b_addr + k * (16 * 128), MN_CHUNK, 1024)
                                                        : umma_smem_desc(b_addr + k * 32, 16, 1024);
-                            if (!(p.dbg & 1)) umma_bf16_pair(d_tmem, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
+                            umma_bf16_pair(d_tmem, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
                         }
                         umma_commit_pair(&wempty[ws]);
                         if (++ws == DUO_NST) {
@@ -996,7 +851,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
                     mbar_arrive_cta(&acc_full[s], 1);
                 }
                 ++epi_cnt[s];
-                RLPPO_TRACE(0, tr0++);       // all MMAs of the step issued
             DUO_WALK_END
         }
     } else if (warp == 10) {
@@ -1004,7 +858,7 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
         if (lane == 0) {
             DuoWalk w;
             uint32_t kpar = 0;                      // bit 4s + kb: parity of a_kb[s][kb] to wait for next
-            DUO_WALK_BEGIN(w, false)
+            DUO_WALK_BEGIN(w)
                 uint8_t* act = smem + s * ACT_BYTES;
                 // k-blocks are stored as the epilogue finishes them: a burst of four 16 KB stores at the end of a phase sat in
                 // the TMA queue ahead of the weight loads (r02aj: the launch is 10 % shorter with the stores switched off)
@@ -1013,7 +867,7 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
                     mbar_wait(&a_kb[b], (kpar >> b) & 1u);
                     kpar ^= 1u << b;
                     if (d.out != NO_STORE) {
-                        if (!p.dbg_nostore) tma_store_2d(&maps.out[ni][d.out], act + kb * KB_BYTES, kb * KBLK, tile_s * TILE_M);
+                        tma_store_2d(&maps.out[ni][d.out], act + kb * KB_BYTES, kb * KBLK, tile_s * TILE_M);
                         bulk_commit();
                     }
                 }
@@ -1033,8 +887,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
         e.s_bias = s_bias;
         e.s_rowx = s_rowx;
         e.a_ready = nullptr;
-        e.a_mma = nullptr;
-        e.rank = rank;
         e.lane = lane;
         e.quarter = warp & 3;
         e.half = (warp - 2) >> 2;
@@ -1048,9 +900,8 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
         // ReLU mask words of this thread's row half, [slot][hidden layer][k-block][thread]: a per-CTA scratch in global memory
         // (24 KB, lives in L2); a backward phase fetches its four words BEFORE it waits for its accumulator
         uint32_t* mask_g = p.mask_scratch + (size_t)blockIdx.x * (2 * DUO_MAXL * 4 * kEpiThreads) + (threadIdx.x - 64);
-        int tr1 = 0;
         DuoWalk w;
-        DUO_WALK_BEGIN(w, true)
+        DUO_WALK_BEGIN(w)
             uint8_t* act = smem + s * ACT_BYTES;
             e.act = act;
             e.s_mask = nullptr;
@@ -1058,7 +909,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
             const int64_t row = (int64_t)tile_s * TILE_M + e.row_in_tile;
             const bool row_ok = row < p.M;
             float dv_keep = s ? dv_slot1 : dv_slot0;
-            if (warp == 2 && lane == 0) RLPPO_TRACE(2, tr1);        // arrived at the step
             uint32_t mpre0 = 0u, mpre1 = 0u, mpre2 = 0u, mpre3 = 0u;
             if (d.kind == PH_DGRAD || d.kind == PH_VALUE_BWD) {
                 const uint32_t* mp = mask_g + (s * DUO_MAXL + d.layer) * 4 * kEpiThreads;
@@ -1070,7 +920,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
             mbar_wait(&acc_full[s], cnt[s] & 1u);
             ++cnt[s];
             tc_fence_after();
-            if (warp == 2 && lane == 0) RLPPO_TRACE(1, tr1++);      // accumulator complete
             if ((pend >> s) & 1u) {      // the slot's previous phase: its stores have read the tile, its releases were seen
                 mbar_wait(&st_done[s], (scnt >> s) & 1u);
                 scnt ^= 1u << s;
@@ -1079,10 +928,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
             const uint32_t trow = tmem_base + ((uint32_t)(e.quarter * 32) << 16) + (uint32_t)s * 256u;
             uint8_t* dst = act;
             const int li = d.layer;
-            const int it = 1;      // (fine-trace stamps of the single-tile kernels are off here)
-            int tr5 = 0;
-            (void)it;
-            (void)tr5;
     // k-blocks are handed to the store thread in pairs: one proxy fence (it waits for the warp's shared-memory writes, a few
     // hundred cycles with two warps per scheduler) per 128 columns instead of per 64
 #define RLPPO_RELEASE_KB(j)                                                  \
@@ -1105,17 +950,14 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
             if (s) dv_slot1 = dv_keep;
             else dv_slot0 = dv_keep;
             pend |= 1u << s;
-            if (warp == 2 && lane == 0) RLPPO_TRACE(3, 4 * n + 1);  // epilogue body done
             // the whole phase is done: the tile in act[s] is complete for the slot's next GEMM and for the store thread
             // (every k-block write above was followed by its own proxy fence + release)
             tc_fence_before();
             __syncwarp();
-            if (warp == 2 && lane == 0) RLPPO_TRACE(3, 4 * n + 2);  // fences done
             if (lane == 0) {
                 if (leader) mbar_arrive(&a_done[s]);
                 else mbar_arrive_cta(&a_done[s], 0);
             }
-            if (warp == 2 && lane == 0) RLPPO_TRACE(1, tr1++);      // phase done
         DUO_WALK_END
         if (e.half == 0) {
             for (int ni = 0; ni < p.n_nets; ++ni) {
@@ -1148,11 +990,6 @@ __global__ void __launch_bounds__(kThreads, 1) fused_duo_kernel(const __grid_con
 #undef DUO_SET
     tc_fence_before();
     __syncthreads();
-    if (p.trace != nullptr && threadIdx.x == 0) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        p.trace[2048 + 2 * blockIdx.x + 1] = t;
-    }
     cluster_sync_all();
     if (warp == 1) {
         tc_fence_after();
@@ -1298,34 +1135,19 @@ int build_net(bool POLICY, const rlppo_fused_net* net, int64_t M, int ni, Maps& 
     return RLPPO_OK;
 }
 
-// RLPPO_FUSED_PAIR=1: run the training launch as 2-CTA clusters (cta_group::2) when every GEMM splits evenly over the pair:
-// hidden widths 128 or 256 (the MN-major backward operands are staged in 64-column chunks per CTA).  OFF by default:
-// measured on B200 (profiles/README_r02.md) the pair's epilogues are faster (2.5k vs 2.9k cycles per phase: half the
-// weight traffic through each SM's shared memory) but every phase pays ~1.3k cycles more in cross-CTA signalling (remote
-// a_mma arrivals, multicast commits) on a chain that synchronises four times per 5k-cycle phase: 132 vs 123 us per launch.
-bool pair_ok(const rlppo_fused_net* const* nets, int n_nets) {
-    static const bool on = getenv("RLPPO_FUSED_PAIR") != nullptr && getenv("RLPPO_FUSED_PAIR")[0] == '1';
-    if (!on) return false;
-    for (int ni = 0; ni < n_nets; ++ni)
-        for (int l = 0; l < nets[ni]->n_hidden; ++l)
-            if (nets[ni]->hidden[l] != 128 && nets[ni]->hidden[l] != 256) return false;
-    return true;
-}
-
-template <bool TRAIN, bool PAIR>
+template <bool TRAIN>
 int launch_nets_t(const rlppo_fused_net* const* nets, const bool* is_policy, int n_nets, const uint16_t* x, int64_t M,
                   Params& p, cudaStream_t s) {
     Maps maps;
     p.M = M;
     p.num_tiles = (int)((M + TILE_M - 1) / TILE_M);
-    p.pair = PAIR ? 1 : 0;
-    p.n_units = PAIR ? (p.num_tiles + 1) / 2 : p.num_tiles;
+    p.n_units = p.num_tiles;
     p.n_nets = n_nets;
     p.in_kb = (nets[0]->in_dim + KBLK - 1) / KBLK;
     for (int ni = 0; ni < n_nets; ++ni) {
         RLPPO_CHECK_ARG(nets[ni]->in_dim == nets[0]->in_dim && nets[ni]->in_ld == nets[0]->in_ld,
                         "nets of one launch read the same x");
-        int rc = build_net<TRAIN>(is_policy[ni], nets[ni], M, ni, maps, p.net[ni], PAIR);
+        int rc = build_net<TRAIN>(is_policy[ni], nets[ni], M, ni, maps, p.net[ni], false);
         if (rc) return rc;
     }
     const rlppo_fused_net* net = nets[0];
@@ -1333,28 +1155,21 @@ int launch_nets_t(const rlppo_fused_net* const* nets, const bool* is_policy, int
     if (rc) return rc;
 
     // shared memory: activation tile + x staging (in_kb k-blocks) + as deep an operand ring as fits + misc
-    p.wst_bytes = PAIR ? WST_BYTES / 2 : WST_BYTES;
     const uint32_t fixed = ACT_BYTES + (uint32_t)p.in_kb * KB_BYTES + MISC_BYTES + 1024;
-    p.nwst = (int)((SMEM_LIMIT - fixed) / p.wst_bytes);
-    if (p.nwst > (PAIR ? MAX_NWST : 3)) p.nwst = PAIR ? MAX_NWST : 3;
+    p.nwst = (int)((SMEM_LIMIT - fixed) / WST_BYTES);
+    if (p.nwst > MAX_NWST) p.nwst = MAX_NWST;
     RLPPO_CHECK_ARG(p.nwst >= 2, "fused path: shared memory budget");
-    const uint32_t smem_bytes = fixed + (uint32_t)p.nwst * p.wst_bytes;
+    const uint32_t smem_bytes = fixed + (uint32_t)p.nwst * WST_BYTES;
     static bool configured = false;
-    auto kfn = fused_mlp_kernel<TRAIN, PAIR>;
+    auto kfn = fused_mlp_kernel<TRAIN>;
     if (!configured) {
         RLPPO_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_LIMIT));
         configured = true;
     }
     const int items = p.n_units * n_nets;
-    int grid;
-    if (PAIR) {
-        const int pairs = num_sms() / 2;
-        grid = 2 * (items < pairs ? items : pairs);
-    } else {
-        grid = items < num_sms() ? items : num_sms();
-    }
+    const int grid = items < num_sms() ? items : num_sms();
     // scheduler words: a pool of self-resetting {next tile, departures} pairs, handed out round-robin so that launches that
-    // may overlap (the two nets of a batch on two streams; consecutive launches under PDL) never share a pair
+    // may overlap (consecutive launches under PDL; launches a caller enqueues on different streams) never share a pair
     {
         constexpr int kSlots = 64;
         static unsigned int* d_sched[16] = {};
@@ -1368,45 +1183,13 @@ int launch_nets_t(const rlppo_fused_net* const* nets, const bool* is_policy, int
         }
         p.sched = d_sched[dev] + 2 * (next_slot[dev]++ % kSlots);
     }
-    static unsigned long long* d_trace = nullptr;
-    const bool tracing = getenv("RLPPO_FUSED_TRACE") != nullptr && TRAIN && p.net[0].policy;
-    p.dbg_nostore = getenv("RLPPO_FUSED_NOSTORE") != nullptr ? 1 : 0;
-    if (tracing) {
-        if (d_trace == nullptr) RLPPO_CUDA(cudaMalloc(&d_trace, 3072 * sizeof(unsigned long long)));
-        RLPPO_CUDA(cudaMemsetAsync(d_trace, 0, 3072 * sizeof(unsigned long long), s));
-        p.trace = d_trace;
-    }
-    RLPPO_CUDA(launch_pdl_cluster(kfn, dim3(grid), dim3(kThreads), smem_bytes, s, PAIR ? 2 : 1, maps, p));
-    if (tracing) {
-        static unsigned long long h[3072];
-        RLPPO_CUDA(cudaMemcpyAsync(h, d_trace, sizeof(h), cudaMemcpyDeviceToHost, s));
-        RLPPO_CUDA(cudaStreamSynchronize(s));
-        const unsigned long long t0 = h[0];
-        fprintf(stderr, "[fused trace] n_ph=%d tiles=%d\n", p.net[0].n_ph, p.num_tiles);
-        for (int i = 0; i + 1 < 512 && (i == 0 || h[i] != 0); i += 2)
-            fprintf(stderr, "  mma  #%d start=%llu issued+stored=+%llu\n", i / 2, h[i] - t0, h[i + 1] - h[i]);
-        for (int i = 0; i + 1 < 512 && h[512 + i] != 0; i += 2)
-            fprintf(stderr, "  epi  #%d start=%llu dur=%llu\n", i / 2, h[512 + i] - t0, h[512 + i + 1] - h[512 + i]);
-        for (int i = 0; i + 1 < 512 && h[1024 + i] != 0; i += 2)
-            fprintf(stderr, "  store #%d issued=%llu read_done=+%llu\n", i / 2, h[1024 + i] - t0, h[1024 + i + 1] - h[1024 + i]);
-        for (int i = 0; i < 512 && h[1536 + i] != 0; ++i)
-            fprintf(stderr, "  wload #%d issued=%llu\n", i, h[1536 + i] - t0);
-        for (int i = 0; i < 512 && h[2048 + i] != 0; ++i)
-            fprintf(stderr, "  wfull #%d at=%llu\n", i, h[2048 + i] - t0);
-        fprintf(stderr, "  stamps: entry=%lld prologue_done=%lld first_x=%lld exit=%lld (cycles rel. to first MMA start)\n",
-                (long long)(h[2560 + 500] - t0), (long long)(h[2560 + 501] - t0), (long long)(h[2560 + 502] - t0),
-                (long long)(h[2560 + 503] - t0));
-        for (int i = 0; i < 500 && h[2560 + i] != 0; ++i)
-            fprintf(stderr, "  fine #%d at=%llu (+%llu)\n", i, h[2560 + i] - t0, i ? h[2560 + i] - h[2560 + i - 1] : 0ull);
-    }
+    RLPPO_CUDA(launch_pdl(kfn, dim3(grid), dim3(kThreads), smem_bytes, s, maps, p));
     return RLPPO_OK;
 }
 
 // The training launch runs as CTA pairs with two tiles in flight per CTA (fused_duo_kernel) whenever the nets allow it
-// (<= 3 hidden layers of width 128 or 256); RLPPO_FUSED_DUO=0 falls back to the single-tile kernel.
+// (<= 3 hidden layers of width 128 or 256); other shapes run the single-tile kernel.
 bool duo_ok(const rlppo_fused_net* const* nets, int n_nets) {
-    static const bool off = getenv("RLPPO_FUSED_DUO") != nullptr && getenv("RLPPO_FUSED_DUO")[0] == '0';
-    if (off) return false;
     for (int ni = 0; ni < n_nets; ++ni) {
         if (nets[ni]->n_hidden > DUO_MAXL) return false;
         for (int l = 0; l < nets[ni]->n_hidden; ++l)
@@ -1420,12 +1203,9 @@ int launch_duo(const rlppo_fused_net* const* nets, const bool* is_policy, int n_
     Maps maps;
     p.M = M;
     p.num_tiles = (int)((M + TILE_M - 1) / TILE_M);
-    p.pair = 1;
     p.n_units = (p.num_tiles + 1) / 2;
     p.n_nets = n_nets;
     p.in_kb = (nets[0]->in_dim + KBLK - 1) / KBLK;
-    p.nwst = DUO_NST;
-    p.wst_bytes = DUO_STAGE;
     for (int ni = 0; ni < n_nets; ++ni) {
         RLPPO_CHECK_ARG(nets[ni]->in_dim == nets[0]->in_dim && nets[ni]->in_ld == nets[0]->in_ld,
                         "nets of one launch read the same x");
@@ -1449,7 +1229,7 @@ int launch_duo(const rlppo_fused_net* const* nets, const bool* is_policy, int n_
             RLPPO_CHECK_ARG(p.net[ni].ph[i].rel_kb > 0, "duo kernel: every phase must release at least one k-block");
     p.sched = nullptr;
     {
-        // four scratch areas handed out round-robin: launches on different streams may overlap (RLPPO_ONE_LAUNCH=0)
+        // four scratch areas handed out round-robin: launches a caller enqueues on different streams may overlap
         static uint32_t* d_mask[16] = {};
         static unsigned int next_area[16] = {};
         int dev = 0;
@@ -1458,40 +1238,7 @@ int launch_duo(const rlppo_fused_net* const* nets, const bool* is_policy, int n_
         if (d_mask[dev] == nullptr) RLPPO_CUDA(cudaMalloc(&d_mask[dev], 4 * area * sizeof(uint32_t)));
         p.mask_scratch = d_mask[dev] + (next_area[dev]++ % 4) * area;
     }
-    p.dbg_nostore = getenv("RLPPO_FUSED_NOSTORE") != nullptr ? 1 : 0;
-    p.dbg = getenv("RLPPO_DUO_DBG") != nullptr ? atoi(getenv("RLPPO_DUO_DBG")) : 0;
-    static unsigned long long* d_trace = nullptr;
-    const bool tracing = getenv("RLPPO_FUSED_TRACE") != nullptr;
-    if (tracing) {
-        if (d_trace == nullptr) RLPPO_CUDA(cudaMalloc(&d_trace, 3072 * sizeof(unsigned long long)));
-        RLPPO_CUDA(cudaMemsetAsync(d_trace, 0, 3072 * sizeof(unsigned long long), s));
-        p.trace = d_trace;
-    }
     RLPPO_CUDA(launch_pdl_cluster(fused_duo_kernel, dim3(grid), dim3(kThreads), (size_t)DUO_SMEM, s, 2, maps, p));
-    if (tracing) {
-        static unsigned long long h[3072];
-        RLPPO_CUDA(cudaMemcpyAsync(h, d_trace, sizeof(h), cudaMemcpyDeviceToHost, s));
-        RLPPO_CUDA(cudaStreamSynchronize(s));
-        const unsigned long long t0 = h[0];
-        fprintf(stderr, "[duo trace] items=%d (steps alternate slots 0/1)\n", items);
-        for (int i = 0; i + 1 < 100 && h[i + 1] != 0; i += 2)
-            fprintf(stderr, "  mma  step %d start=%llu issued=+%llu\n", i / 2, h[i] - t0, h[i + 1] - h[i]);
-        {
-            unsigned long long g0 = ~0ull, g1 = 0;
-            for (int b = 0; b < grid; ++b) {
-                if (h[2048 + 2 * b] < g0) g0 = h[2048 + 2 * b];
-                if (h[2048 + 2 * b + 1] > g1) g1 = h[2048 + 2 * b + 1];
-            }
-            fprintf(stderr, "  CTA spans (ns from the first start; start..end), kernel body %llu ns:\n", g1 - g0);
-            for (int b = 0; b < grid; b += 2)
-                fprintf(stderr, "   cluster %d: %llu..%llu%s", b / 2, h[2048 + 2 * b] - g0, h[2048 + 2 * b + 1] - g0, (b / 2) % 4 == 3 ? "\n" : "");
-            fprintf(stderr, "\n");
-        }
-        for (int i = 0; i + 1 < 100 && h[512 + i] != 0; i += 2)
-            fprintf(stderr, "  epi  step %d top=%llu arrive=%llu acc_full=%llu dur=%llu body_end=+%llu fences=+%llu arrives=+%llu\n", i / 2,
-                    h[1536 + 2 * i] - t0, h[1024 + i] - t0, h[512 + i] - t0, h[512 + i + 1] - h[512 + i],
-                    h[1536 + 2 * i + 1] - h[512 + i], h[1536 + 2 * i + 2] - h[1536 + 2 * i + 1], h[512 + i + 1] - h[1536 + 2 * i + 2]);
-    }
     return RLPPO_OK;
 }
 
@@ -1505,8 +1252,7 @@ int launch_nets(const rlppo_fused_net* const* nets, const bool* is_policy, int n
         if (rc) return rc;
     }
     if (TRAIN && duo_ok(nets, n_nets)) return launch_duo(nets, is_policy, n_nets, x, M, p, s);
-    if (TRAIN && pair_ok(nets, n_nets)) return launch_nets_t<TRAIN, TRAIN>(nets, is_policy, n_nets, x, M, p, s);
-    return launch_nets_t<TRAIN, false>(nets, is_policy, n_nets, x, M, p, s);
+    return launch_nets_t<TRAIN>(nets, is_policy, n_nets, x, M, p, s);
 }
 
 void fill_policy_train(NetP& n, int n_actions, const float* actions, const float* old_logp, const float* adv,

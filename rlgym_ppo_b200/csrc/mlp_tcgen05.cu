@@ -888,8 +888,6 @@ struct WLayer {
 struct WMultiParams {
     WLayer L[MAXW];
     int n_layers, total_items;
-    int dbg_nodrain;   // debug (RLPPO_WGRAD_NODRAIN=1): timing experiment, the accumulators are NOT added to dW
-    int dbg_nomma;     // debug (RLPPO_WGRAD_NOMMA=1): timing experiment, stages are released without issuing MMAs
 };
 
 __global__ void __launch_bounds__(kThreads, 1)
@@ -985,7 +983,7 @@ wgrad_multi_kernel(const __grid_constant__ WMaps maps, const WMultiParams p) {
                     tc_fence_after();
                     const uint32_t x_addr = smem_u32(smem + stage * STAGE);
                     const uint32_t b_addr = x_addr + 4 * CHUNK;
-                    for (int kt = 0; kt < (p.dbg_nomma ? 0 : n_kt); ++kt) {
+                    for (int kt = 0; kt < n_kt; ++kt) {
 #pragma unroll
                         for (int ks = 0; ks < BLOCK_K / UMMA_K; ++ks) {
                             const uint64_t ad = umma_smem_desc(x_addr + kt * 2 * CHUNK + ks * (UMMA_K * 128), CHUNK, 1024);
@@ -1035,7 +1033,7 @@ wgrad_multi_kernel(const __grid_constant__ WMaps maps, const WMultiParams p) {
                     phase ^= 1;
                 }
             }
-            if (want_db && !p.dbg_nodrain) {
+            if (want_db) {
                 const int n = it.n0 + ew * 64 + 2 * lane;
                 if (n < L.N) atomicAdd(L.db + n, s0 + s2);
                 if (n + 1 < L.N) atomicAdd(L.db + n + 1, s1 + s3);
@@ -1054,7 +1052,7 @@ wgrad_multi_kernel(const __grid_constant__ WMaps maps, const WMultiParams p) {
 #pragma unroll
                         for (int j = 0; j < 32; ++j) {
                             const int n = it.n0 + c * 32 + j;
-                            if (n < L.N && !p.dbg_nodrain) atomicAdd(L.dw + (int64_t)n * L.lddw + k, v[j]);
+                            if (n < L.N) atomicAdd(L.dw + (int64_t)n * L.lddw + k, v[j]);
                         }
                     }
                 }
@@ -1460,10 +1458,6 @@ int rlppo_wgrad_multi(const rlppo_wgrad_item* h_items, int n_items, void* stream
         first += tiles * L.splits;
     }
     p.total_items = first;
-    static const bool nodrain = getenv("RLPPO_WGRAD_NODRAIN") != nullptr;
-    p.dbg_nodrain = nodrain ? 1 : 0;
-    static const bool nomma = getenv("RLPPO_WGRAD_NOMMA") != nullptr;
-    p.dbg_nomma = nomma ? 1 : 0;
     constexpr uint32_t SMEM = 3 * 8 * 8192 + 256 + 1024;
     static bool configured = false;
     if (!configured) {

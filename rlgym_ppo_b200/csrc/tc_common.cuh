@@ -212,13 +212,6 @@ __device__ __forceinline__ uint32_t mapa_u32(const void* p, uint32_t cta) {
 __device__ __forceinline__ void mbar_arrive_cta(uint64_t* bar, uint32_t cta) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(mapa_u32(bar, cta)) : "memory");
 }
-// the same with release at cluster scope: publishes this thread's earlier st.shared::cluster to the waiter
-__device__ __forceinline__ void mbar_arrive_cta_release(uint64_t* bar, uint32_t cta) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(mapa_u32(bar, cta)) : "memory");
-}
-__device__ __forceinline__ void st_shared_cta_s32(int* p, uint32_t cta, int v) {
-    asm volatile("st.shared::cluster.s32 [%0], %1;" ::"r"(mapa_u32(p, cta)), "r"(v) : "memory");
-}
 // 2-D tile load into THIS CTA's shared memory whose completion (complete_tx) is counted on the mbarrier at the same offset
 // in the pair's leader CTA: the leader's MMA thread waits on ONE barrier for both CTAs' operand halves (the form
 // CUTLASS's SM100_TMA_2SM_LOAD uses; tools/microbench/cta_pair_gemm.cu tma_mode 1).

@@ -165,8 +165,7 @@ class PPOLearner(object):
         self.clip_range = clip_range
         self.ent_coef = ent_coef
         self.cumulative_model_updates = 0
-        # RLPPO_MAX_CHUNK_ROWS: experiment knob (rows of a batch processed per fused-kernel launch; see profiles/README_r02.md)
-        self.max_chunk_rows = int(os.environ.get("RLPPO_MAX_CHUNK_ROWS", max_chunk_rows))
+        self.max_chunk_rows = int(max_chunk_rows)
 
         # ---- data parallelism ---------------------------------------------------------------------------------
         # Data-parallel modes (world_size > 1; one process per GPU, NCCL through torch.distributed):
@@ -193,24 +192,6 @@ class PPOLearner(object):
         self._graph_warm = set()
         self._idx_cur = None
         self._perm_dev = None
-        # RLPPO_GRAPH_COLLECTIVES=1: capture the NCCL allreduces inside the whole-call graph when data parallel.  Off by
-        # default: measured on 2 x B200 it buys 1 % (the step is bound by the collectives' latency, not by their launch)
-        # and process-group teardown hangs with captured NCCL work outstanding.  Default: two graphs per optimiser step
-        # with an eager allreduce between them.
-        self.graph_collectives = os.environ.get("RLPPO_GRAPH_COLLECTIVES", "0") == "1"
-        # RLPPO_TWO_STREAMS=0: policy and value chains of a batch on one stream (see _train_chunk)
-        self.two_streams = os.environ.get("RLPPO_TWO_STREAMS", "1") == "1"
-        # RLPPO_ONE_LAUNCH=0: the two nets of a batch as two fused launches (two streams) instead of one (see _train_chunk)
-        self.one_launch = os.environ.get("RLPPO_ONE_LAUNCH", "1") == "1"
-        self._side_stream = None
-        # RLPPO_GATHER_PREFETCH=1 (experiment, off by default): the gather of batch i + 1 (independent of the weights) runs on
-        # a second stream -- a parallel branch of the captured graph -- beside the weight-gradient and optimiser launches of
-        # batch i, into the other of two minibatch buffer sets (see _learn_body).  Measured on B200 at the example shape
-        # (profiles/r02be_timeline_prefetch.txt): the 24 us gather does run under the weight-gradient kernel, which then
-        # takes 92 instead of 80 us -- both stream the same HBM -- and the step is unchanged (0.935 vs 0.933 ms).
-        self.gather_prefetch = os.environ.get("RLPPO_GATHER_PREFETCH", "0") == "1"
-        self._gather_stream = None
-        self._mb_alt = None
 
     def _setup_peers(self, dev, n):
         """Gradient arena + flag block in symmetric memory (torch.distributed._symmetric_memory: CUDA peer mappings over
@@ -255,10 +236,9 @@ class PPOLearner(object):
             self._gsum = torch.zeros(n, dtype=torch.float32, device=dev)
 
     # ---- workspaces ----------------------------------------------------------------------------------------
-    def _minibatch_buffers(self, rows, slot=0):
-        """The gathered minibatch (bf16 observation rows + the per-sample scalars).  Two sets exist when the next batch is
-        gathered while the current one trains (slot 1, see _learn_body)."""
-        cur = self._mb if slot == 0 else self._mb_alt
+    def _minibatch_buffers(self, rows):
+        """The gathered minibatch (bf16 observation rows + the per-sample scalars)."""
+        cur = self._mb
         if cur is None or cur["rows"] < rows:
             dev = self._params.device
             f = lambda: torch.empty(rows, dtype=torch.float32, device=dev)  # noqa: E731
@@ -273,10 +253,7 @@ class PPOLearner(object):
                 cur["x"] = torch.zeros((rows, 3 * ps.in_ps), dtype=torch.bfloat16, device=dev)
             else:
                 cur["x"] = torch.zeros((rows, ps.in_pad), dtype=torch.bfloat16, device=dev)
-            if slot == 0:
-                self._mb = cur
-            else:
-                self._mb_alt = cur
+            self._mb = cur
         return cur
 
     def _gather(self, exp, idx, M, mb):
@@ -315,62 +292,27 @@ class PPOLearner(object):
         self._views_sig = sig
 
     # ---- one chunk of one batch: gather -> fwd -> fused heads -> bwd (grads accumulate) -------------------------
-    def _train_chunk(self, exp, idx, M, mb=None, after_fused=None):
-        """`mb`: a minibatch buffer set that already holds the gathered rows (gather prefetch); None: gather here.
-        `after_fused`: called once the fused forward/backward launch is enqueued (where the next batch's gather forks off)."""
+    def _train_chunk(self, exp, idx, M):
         self._sync_operand_views()
-        if mb is None:
-            mb = self._minibatch_buffers(M)
-            self._gather(exp, idx, M, mb)
+        mb = self._minibatch_buffers(M)
+        self._gather(exp, idx, M, mb)
         x = mb["x"]
         # (1/mb) * (mb/B), ppo_learner.py:172-177; B = the number of samples one optimiser step averages over
         inv_b = 1.0 / float(parallel.samples_per_step(self.batch_size, self.world_size, self.dp_mode))
         metrics = self._step_metrics()
         n = 1
-        both_fused = self.policy_type == 0 and self.policy._stack.fused_ok and self.value_net._stack.fused_ok
-        if both_fused and self.one_launch:
+        if self.policy_type == 0 and self.policy._stack.fused_ok and self.value_net._stack.fused_ok:
             # Both nets in ONE persistent launch: 2 x ceil(M/128) work items (policy tiles first) dealt out over
-            # one CTA per SM, then every weight (and bias) gradient of both nets in one launch.  Two launches on two
-            # streams (RLPPO_ONE_LAUNCH=0) each end on a partly filled round of tiles: 391 tiles over 148 CTAs.
+            # one CTA per SM, then every weight (and bias) gradient of both nets in one launch.  Two launches, one per
+            # net, would each end on a partly filled round of tiles: 391 tiles over 148 CTAs.
             ps, vs = self.policy._stack, self.value_net._stack
             wp, wv = ps.workspace(M), vs.workspace(M)
             ops.policy_value_train_fused(ps.fused_net(x.stride(0), wp, policy_head=True), vs.fused_net(x.stride(0), wv), x, M,
                                          self.policy.n_actions, mb["actions"], mb["old_logp"], mb["adv"], inv_b,
                                          float(self.clip_range), float(self.ent_coef), vs.w[-1], mb["targets"], vs.gw[-1],
                                          metrics)
-            if after_fused is not None:
-                after_fused()
             ops.wgrad_multi(ps.fused_wgrad_items(x, wp, head_dy=wp["dz"]) + vs.fused_wgrad_items(x, wv), M)
             self.launches += 3
-            return
-        if after_fused is not None:
-            after_fused()
-        if both_fused and self.two_streams and _lib._TIMING is None:
-            # The two nets are independent until the optimiser step: the value net's chain (fused kernel, weight
-            # gradients) runs on a second stream -- a parallel branch of the captured graph.  Each kernel is persistent
-            # with one CTA per SM, so the branches do not share SMs; they fill each other's tails (391 tiles over 148 CTAs
-            # leave a third of the SMs idle for the last tile round) and prologue / drain phases.
-            main = torch.cuda.current_stream()
-            if self._side_stream is None:
-                self._side_stream = torch.cuda.Stream(device=self._params.device)
-            side = self._side_stream
-            fork, join = torch.cuda.Event(), torch.cuda.Event()
-            fork.record(main)
-            side.wait_event(fork)
-            with torch.cuda.stream(side):
-                st = self.value_net._stack
-                ws = st.workspace(M)
-                ops.value_train_fused(st.fused_net(x.stride(0), ws), x, M, st.w[-1], mb["targets"], inv_b, st.gw[-1], metrics)
-                ops.wgrad_multi(st.fused_wgrad_items(x, ws), M)
-                join.record(side)
-            st = self.policy._stack
-            ws = st.workspace(M)
-            ops.policy_train_fused(st.fused_net(x.stride(0), ws, policy_head=True), x, M, self.policy.n_actions,
-                                   mb["actions"], mb["old_logp"], mb["adv"], inv_b, float(self.clip_range),
-                                   float(self.ent_coef), metrics)
-            ops.wgrad_multi(st.fused_wgrad_items(x, ws, head_dy=ws["dz"]), M)
-            main.wait_event(join)
-            self.launches += 5
             return
         wg_items = []
         for net, is_policy in ((self.policy, True), (self.value_net, False)):
@@ -524,7 +466,6 @@ class PPOLearner(object):
         """Everything a captured graph bakes in: buffer identity, workspace generations (addresses), scalar arguments."""
         return (exp.uid, local, chunk, float(self.clip_range), float(self.ent_coef), self.batch_size, self.world_size,
                 self.dp_mode, self.dp_collective, self.precision, self.policy_type, self.policy._stack.fused_ok, self.value_net._stack.fused_ok, getattr(self, "_mb_gen", 0),
-                self.gather_prefetch,
                 getattr(self.policy._stack, "ws_gen", 0), getattr(self.value_net._stack, "ws_gen", 0))
 
     def _learn_body(self, exp, n_batches, local, chunk, tail=True):
@@ -537,40 +478,8 @@ class PPOLearner(object):
         steps = [(epoch, parallel.rank_rows(k, B, self.rank, R, self.dp_mode)[0])
                  for epoch in range(self.n_epochs) for k in range(n_batches)]
         idx_of = lambda i: self._perm_dev[steps[i][0], steps[i][1]:steps[i][1] + local]  # noqa: E731
-        if self.gather_prefetch and chunk == local and len(steps) > 1:
-            # Software pipeline over the optimiser steps: while step i runs its fused / weight-gradient / optimiser launches
-            # (persistent, one CTA per SM, with idle SMs in every tail), the rows of step i + 1 are gathered on a second
-            # stream into the other buffer set.  The gather reads only the rings and the permutation, never the weights.
-            main = torch.cuda.current_stream()
-            if self._gather_stream is None:
-                self._gather_stream = torch.cuda.Stream(device=self._params.device)
-            side = self._gather_stream
-            sets = (self._minibatch_buffers(local, 0), self._minibatch_buffers(local, 1))
-            self._gather(exp, idx_of(0), local, sets[0])
-            for i in range(len(steps)):
-                joins = []
-
-                def prefetch(i=i, joins=joins):
-                    # Forked BEHIND the fused launch of step i (an event waits for everything before it): the gather shares
-                    # the SMs with the weight-gradient and optimiser launches -- its 128-thread CTAs fit beside their CTAs.
-                    # Forked ahead of the fused launch it only runs first: a persistent CTA needs a whole SM's shared memory
-                    # and waits for the gather's CTAs to drain (timeline r02bd).
-                    fork, join = torch.cuda.Event(), torch.cuda.Event()
-                    fork.record(main)
-                    side.wait_event(fork)
-                    with torch.cuda.stream(side):
-                        self._gather(exp, idx_of(i + 1), local, sets[(i + 1) & 1])
-                        join.record(side)
-                    joins.append(join)
-
-                self._grads.zero_()                                     # ppo_learner.py:131-132
-                self._train_chunk(exp, None, local, mb=sets[i & 1], after_fused=prefetch if i + 1 < len(steps) else None)
-                self._optimizer_step()
-                for join in joins:
-                    main.wait_event(join)
-        else:
-            for i in range(len(steps)):
-                self._batch_body(exp, idx_of(i), local, chunk)
+        for i in range(len(steps)):
+            self._batch_body(exp, idx_of(i), local, chunk)
         ops.sqdiff(self._before, self._params, self._seg, self._tail[8:8 + len(self._seg) - 1])
         if tail:
             self._tail_host.copy_(self._tail, non_blocking=True)      # metric sums are global already (see __init__)
@@ -614,8 +523,7 @@ class PPOLearner(object):
         n_iterations = E * n_batches
 
         p2p = R > 1 and self.dp_collective in ("p2p", "p2p2")
-        whole = (self.use_cuda_graph and _lib._TIMING is None and n_batches > 0
-                 and (R == 1 or p2p or self.graph_collectives))
+        whole = self.use_cuda_graph and _lib._TIMING is None and n_batches > 0 and (R == 1 or p2p)
         if whole:
             # data parallel over peer memory: the graph holds the WHOLE call, the report readback included
             tail = True

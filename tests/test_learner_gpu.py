@@ -719,20 +719,3 @@ def test_fused_training_launch_back_to_back(pkg, M):
     torch.cuda.synchronize()
     assert torch.isfinite(logp).all() and torch.equal(logp, first)
     assert torch.isfinite(lr._grads).all() and torch.isfinite(metrics).all()
-
-
-@pytest.mark.parametrize("env", [{"RLPPO_FUSED_DUO": "0"}, {"RLPPO_FUSED_DUO": "0", "RLPPO_FUSED_PAIR": "1"}],
-                         ids=["single_cta", "cta_pair"])
-def test_other_fused_launch_forms_match(pkg, env):
-    """The default training launch is fused_duo_kernel (2-CTA clusters, tcgen05.mma.cta_group::2, two tiles in flight per
-    CTA).  The two other forms -- one tile per CTA (RLPPO_FUSED_DUO=0) and one tile per CTA of a pair (+ RLPPO_FUSED_PAIR=1)
-    -- must give the same results: the fused-vs-layerwise, golden and partition tests re-run in a fresh process with the
-    switches set (they are read once per process)."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-m", "pytest", "tests/test_learner_gpu.py", "-m", "gpu", "-x", "-q", "-k",
-                        "fused_kernels_match_layerwise or policy_and_value_golden or ppo_learner_golden or row_partition"],
-                       cwd=root, env=dict(os.environ, **env), capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
