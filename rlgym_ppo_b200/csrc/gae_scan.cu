@@ -5,24 +5,16 @@
 //   aA = f32(gamma*lambda)*(1-done)*(1-trunc),  bA = delta_t (f32),  aR = gamma*(1-done)*(1-trunc),  bR = r_t.
 // A done/truncated step has a = 0, which is the segment reset.  Composition (a,b)o(c,d) = (a*c, b + a*d)
 // is associative, so the recurrence is a suffix scan: thread-serial over 4 steps, warp shuffle scan over
-// lanes, one warp over the 16 warp aggregates, and decoupled look-back across tiles (tile 0 is the END of
-// the rollout; tile ids are handed out by an atomic ticket so a tile only ever waits on tiles that are
-// already running).  Carries are f64 (HBM-bound kernel; the fp64 work is free) which also reproduces the
+// lanes, a scan over the 8 warp aggregates of a 1024-step tile, and decoupled look-back across tiles (tile 0 is
+// the END of the rollout).  Carries are f64 (HBM-bound kernel; the fp64 work is free) which also reproduces the
 // reference's f64 accumulation; delta is formed with the reference's f32 rounding points.
 //
 // HBM traffic: reads r, done, trunc, V (16 B/step with f32 flags), writes adv, vtarget, ret (12 B/step).
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "common.cuh"
 
 namespace {
-
-constexpr int kThreads = 512;
-constexpr int kItems = 4;
-constexpr int kTile = kThreads * kItems;  // 2048 steps per CTA
-constexpr int kWarps = kThreads / 32;
 
 struct Aff {
     double aA, bA, aR, bR;
@@ -51,208 +43,12 @@ __device__ __forceinline__ Aff warp_suffix_scan(Aff x, int lane) {
     return x;
 }
 
+// Both record arrays hold one 4-double map per tile slot.
 struct Workspace {
-    int* counter;   // ticket
-    int* status;    // per tile: 0 = nothing, 1 = aggregate published, 2 = inclusive published
-    double* agg;    // per tile 4 doubles: map of this tile alone
-    double* incl;   // per tile 4 doubles: map of this tile and every tile to its right
+    double* agg;    // per tile: map of this tile alone
+    double* gagg;   // per group of 32 CTAs: map of the group's tiles of one iteration, slot = the group's first tile
 };
 
-template <bool TRUNC64, bool VEC, bool STORE>
-__global__ void __launch_bounds__(kThreads)
-gae_scan_kernel(const float* __restrict__ rew, const float* __restrict__ done, const void* __restrict__ trunc,
-                const float* __restrict__ val, int64_t n, double gamma, float gl32,
-                const float* __restrict__ ret_std, float* __restrict__ adv, float* __restrict__ vt,
-                float* __restrict__ ret, double* __restrict__ ret_head, int64_t n_head,
-                const double* __restrict__ carry_in, double* __restrict__ summary_out, Workspace ws,
-                int n_tiles) {
-    __shared__ int s_tile;
-    __shared__ double s_warp[kWarps][4];
-    __shared__ double s_carry[2];
-
-    if (threadIdx.x == 0) s_tile = atomicAdd(ws.counter, 1);
-    __syncthreads();
-    const int tile = s_tile;
-    const int chunk = n_tiles - 1 - tile;
-    const int lane = threadIdx.x & 31;
-    const int warp = threadIdx.x >> 5;
-    const int64_t base = (int64_t)chunk * kTile + (int64_t)threadIdx.x * kItems;
-
-    float r[kItems], d[kItems], v[kItems + 1];
-    double tr[kItems];
-    const bool full = base + kItems <= n;
-    if (VEC && full) {
-        const float4 r4 = __ldg(reinterpret_cast<const float4*>(rew + base));
-        const float4 d4 = __ldg(reinterpret_cast<const float4*>(done + base));
-        const float4 v4 = __ldg(reinterpret_cast<const float4*>(val + base));
-        r[0] = r4.x; r[1] = r4.y; r[2] = r4.z; r[3] = r4.w;
-        d[0] = d4.x; d[1] = d4.y; d[2] = d4.z; d[3] = d4.w;
-        v[0] = v4.x; v[1] = v4.y; v[2] = v4.z; v[3] = v4.w;
-        v[4] = __ldg(val + base + 4);
-        if (TRUNC64) {
-            const double2 t0 = __ldg(reinterpret_cast<const double2*>(static_cast<const double*>(trunc) + base));
-            const double2 t1 = __ldg(reinterpret_cast<const double2*>(static_cast<const double*>(trunc) + base + 2));
-            tr[0] = t0.x; tr[1] = t0.y; tr[2] = t1.x; tr[3] = t1.y;
-        } else {
-            const float4 t4 = __ldg(reinterpret_cast<const float4*>(static_cast<const float*>(trunc) + base));
-            tr[0] = t4.x; tr[1] = t4.y; tr[2] = t4.z; tr[3] = t4.w;
-        }
-    } else {
-#pragma unroll
-        for (int i = 0; i < kItems; ++i) {
-            const int64_t t = base + i;
-            const bool ok = t < n;
-            r[i] = ok ? __ldg(rew + t) : 0.f;
-            d[i] = ok ? __ldg(done + t) : 0.f;
-            v[i] = (t <= n) ? __ldg(val + t) : 0.f;   // values has n+1 entries
-            tr[i] = !ok ? 0.0
-                        : (TRUNC64 ? __ldg(static_cast<const double*>(trunc) + t)
-                                   : (double)__ldg(static_cast<const float*>(trunc) + t));
-        }
-        v[kItems] = (base + kItems <= n) ? __ldg(val + base + kItems) : 0.f;
-    }
-    const bool has_std = ret_std != nullptr;
-    const float stdv = has_std ? __ldg(ret_std) : 1.f;
-
-    // per-step maps; steps past the end are identities so the carry passes through them
-    Aff f[kItems];
-#pragma unroll
-    for (int i = 0; i < kItems; ++i) {
-        if (base + i < n) {
-            const float nd = __fsub_rn(1.0f, d[i]);                              // torch_functions.py:59
-            const double nt = 1.0 - tr[i];                                       // :60
-            float nr = r[i];
-            if (has_std) {                                                        // :62-65
-                nr = __fdiv_rn(r[i], stdv);
-                nr = fminf(fmaxf(nr, -10.f), 10.f);
-            }
-            const float gv = (float)(gamma * (double)v[i + 1]);
-            const float pred = __fadd_rn(nr, __fmul_rn(gv, nd));                 // :67
-            const float delta = __fsub_rn(pred, v[i]);                           // :68
-            f[i].aA = (double)__fmul_rn(gl32, nd) * nt;                          // :72
-            f[i].bA = (double)delta;
-            f[i].aR = gamma * (double)nd * nt;                                   // :69
-            f[i].bR = (double)r[i];
-        } else {
-            f[i] = aff_identity();
-        }
-    }
-    Aff agg = f[kItems - 1];
-#pragma unroll
-    for (int i = kItems - 2; i >= 0; --i) agg = compose(f[i], agg);
-
-    // warp-level suffix scan of the thread aggregates
-    const Aff incl_w = warp_suffix_scan(agg, lane);
-    Aff excl = shfl_down(incl_w, 1);
-    if (lane == 31) excl = aff_identity();
-    if (lane == 0) {
-        s_warp[warp][0] = incl_w.aA; s_warp[warp][1] = incl_w.bA;
-        s_warp[warp][2] = incl_w.aR; s_warp[warp][3] = incl_w.bR;
-    }
-    __syncthreads();
-
-    if (warp == 0) {
-        Aff w = aff_identity();
-        if (lane < kWarps) w = Aff{s_warp[lane][0], s_warp[lane][1], s_warp[lane][2], s_warp[lane][3]};
-        const Aff wi = warp_suffix_scan(w, lane);       // lanes >= kWarps hold identities
-        Aff we = shfl_down(wi, 1);                      // exclusive: warps to the right of `lane`
-        if (lane == 31) we = aff_identity();
-        if (lane < kWarps) {
-            s_warp[lane][0] = we.aA; s_warp[lane][1] = we.bA; s_warp[lane][2] = we.aR; s_warp[lane][3] = we.bR;
-        }
-        const Aff tile_agg = shfl_idx(wi, 0);
-
-        // ---- decoupled look-back: map of everything to the right of this tile ----
-        Aff right = aff_identity();
-        if (tile > 0) {
-            if (lane == 0) {
-                double* a = ws.agg + (size_t)tile * 4;
-                a[0] = tile_agg.aA; a[1] = tile_agg.bA; a[2] = tile_agg.aR; a[3] = tile_agg.bR;
-                __threadfence();
-                rlppo::st_release_s32(ws.status + tile, 1);
-            }
-            int look = tile - 1;
-            bool finished = false;
-            while (!finished) {
-                const int j = look - lane;
-                int st = 2;
-                Aff m = aff_identity();   // j < 0: nothing to the right of tile 0
-                if (j >= 0) {
-                    const long long t0 = clock64();
-                    do {
-                        st = rlppo::ld_acquire_s32(ws.status + j);
-                        if (st == 0 && clock64() - t0 > 8000000000LL) __trap();   // watchdog (~4 s)
-                    } while (st == 0);
-                    const double* src = (st == 2 ? ws.incl : ws.agg) + (size_t)j * 4;
-                    m = Aff{__ldcg(src), __ldcg(src + 1), __ldcg(src + 2), __ldcg(src + 3)};
-                }
-                const unsigned done_mask = __ballot_sync(0xffffffffu, st == 2);
-                const int upto = done_mask ? (__ffs(done_mask) - 1) : 31;
-                for (int l = 0; l <= upto; ++l) right = compose(right, shfl_idx(m, l));
-                finished = done_mask != 0;
-                look -= 32;
-            }
-        }
-        const Aff incl = compose(tile_agg, right);
-        if (lane == 0) {
-            double* o = ws.incl + (size_t)tile * 4;
-            o[0] = incl.aA; o[1] = incl.bA; o[2] = incl.aR; o[3] = incl.bR;
-            __threadfence();
-            rlppo::st_release_s32(ws.status + tile, 2);
-            const double cA = carry_in ? carry_in[0] : 0.0;
-            const double cR = carry_in ? carry_in[1] : 0.0;
-            s_carry[0] = fma(right.aA, cA, right.bA);
-            s_carry[1] = fma(right.aR, cR, right.bR);
-            if (summary_out != nullptr && tile == n_tiles - 1) {
-                summary_out[0] = incl.aA; summary_out[1] = incl.bA;
-                summary_out[2] = incl.aR; summary_out[3] = incl.bR;
-            }
-        }
-    }
-    if (!STORE) return;
-    __syncthreads();
-
-    // value just right of this thread's 4 steps
-    const Aff wr = Aff{s_warp[warp][0], s_warp[warp][1], s_warp[warp][2], s_warp[warp][3]};
-    const Aff e = compose(excl, wr);
-    double xA = fma(e.aA, s_carry[0], e.bA);
-    double xR = fma(e.aR, s_carry[1], e.bR);
-    float oa[kItems], ov[kItems], orr[kItems];
-    double r64[kItems];
-#pragma unroll
-    for (int i = kItems - 1; i >= 0; --i) {
-        xA = fma(f[i].aA, xA, f[i].bA);
-        xR = fma(f[i].aR, xR, f[i].bR);
-        oa[i] = (float)xA;                       // :76
-        ov[i] = (float)((double)v[i] + xA);      // :77
-        orr[i] = (float)xR;
-        r64[i] = xR;
-    }
-    if (VEC && full) {
-        *reinterpret_cast<float4*>(adv + base) = make_float4(oa[0], oa[1], oa[2], oa[3]);
-        *reinterpret_cast<float4*>(vt + base) = make_float4(ov[0], ov[1], ov[2], ov[3]);
-        *reinterpret_cast<float4*>(ret + base) = make_float4(orr[0], orr[1], orr[2], orr[3]);
-    } else {
-#pragma unroll
-        for (int i = 0; i < kItems; ++i)
-            if (base + i < n) {
-                adv[base + i] = oa[i];
-                vt[base + i] = ov[i];
-                ret[base + i] = orr[i];
-            }
-    }
-    if (ret_head != nullptr && base < n_head) {
-#pragma unroll
-        for (int i = 0; i < kItems; ++i)
-            if (base + i < n_head && base + i < n) ret_head[base + i] = r64[i];
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// History -- v2 (removed; see profiles/README_r01.md): the same scan with the tile's inputs staged in shared memory by bulk
-// async copies, one 2048-step tile per CTA, 4 CTAs/SM: 3.0 TB/s at 2^28 steps, latency-bound (every tile still paid
-// ticket -> loads -> look-back -> stores back to back).  The helpers below are what v3 kept from it.
-// ---------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_addr_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
@@ -260,14 +56,13 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gsrc, uint3
                  "l"(gsrc), "r"(bytes), "r"(smem_addr_u32(bar))
                  : "memory");
 }
-// Tile records without flags or fences: a record (aggregate or inclusive map, 4 doubles) is written with two 16-byte
-// relaxed gpu-scope vector stores and polled with two relaxed gpu-scope vector loads.  The workspace is pre-set to
-// all-ones bytes -- a NaN pattern no computation produces -- and a record counts as arrived when none of its four
-// doubles is that pattern (each 8-byte element is single-copy atomic, so nothing torn can pass the test).  The accesses
-// must be STRONG (.relaxed.gpu), not plain .cg: a weak load may be served by the reader's own L2 partition and never
-// observe the other die's store.  (The first version published a status word with __threadfence() + st.release and
-// polled it with ld.acquire: ncu showed 12 % of all stall samples on the CCTL.IVALL the acquire emits, plus a dependent
-// second load per look-back round.)
+// Tile records without flags or fences: a record (4 doubles) is written with two 16-byte relaxed gpu-scope vector
+// stores and polled with two relaxed gpu-scope vector loads.  The workspace is pre-set to all-ones bytes -- a NaN
+// pattern no computation produces -- and a record counts as arrived when none of its four doubles is that pattern (each
+// 8-byte element is single-copy atomic, so nothing torn can pass the test).  The accesses must be STRONG (.relaxed.gpu),
+// not plain .cg: a weak load may be served by the reader's own L2 partition and never observe the other die's store.
+// (A status word published with __threadfence() + st.release and polled with ld.acquire cost 12 % of all stall samples
+// on the CCTL.IVALL the acquire emits, plus a dependent second load per look-back round.)
 __device__ __forceinline__ void rec_store(double* rec, const Aff& m) {
     asm volatile("st.relaxed.gpu.global.v2.f64 [%0], {%1, %2};" ::"l"(rec), "d"(m.aA), "d"(m.bA) : "memory");
     asm volatile("st.relaxed.gpu.global.v2.f64 [%0], {%1, %2};" ::"l"(rec + 2), "d"(m.aR), "d"(m.bR) : "memory");
@@ -290,7 +85,7 @@ struct StepMaps {
     float gl32, stdv;
     bool has_std;
     // multipliers of local step j exactly as the reference writes them (torch_functions.py:59-60, 69, 72): the generic
-    // path, for flags that are not exactly +0 / 1 and for the ragged tile
+    // path, for flags that are not exactly +0 / 1 and for tiles that are not staged
     __device__ __forceinline__ void mults(int j, double& aA, double& aR) const {
         const float dj = d[j];
         const double trj = TRUNC64 ? static_cast<const double*>(t)[j] : (double)static_cast<const float*>(t)[j];
@@ -315,61 +110,51 @@ struct StepMaps {
 };
 
 // ---------------------------------------------------------------------------------------------------------
-// v3: persistent, software-pipelined scan.
+// Persistent, software-pipelined scan.
 //
-// ncu on v2 (one tile per CTA, 4 CTAs/SM, 2^26 steps): a tile's lifetime was 11.5 us, of which 22 % waiting for its own
-// ticket + loads, 33 % in the look-back (store -> L2 -> poll round trips, 256-thread shuffle scans, block barriers) and
-// only 37 % in the two compute phases -- latency-bound at 40 % of the DRAM bandwidth however the phases were trimmed.
-// Here a CTA lives for the whole launch and overlaps the three latencies with compute:
+// With one tile per CTA the scan is latency-bound (a tile waits for its loads, then its look-back, then its stores, at
+// 40 % of the DRAM bandwidth however the phases are trimmed).  Here a CTA lives for the whole launch and overlaps the
+// three latencies with compute:
 //   * 3 CTAs per SM; CTA b takes tiles b, b+G, b+2G, ... (tile 0 = the END of the rollout, 1024 steps per tile).
 //   * warp 8 (one thread): producer.  Keeps a 3-stage ring of {r, done, V(+halo), truncated} tiles filled with bulk
 //     async copies (mbarrier full/empty per stage), so tile k+1 and k+2 are in flight while tile k is scanned.
 //   * warps 0-7: compute.  A(k): flags -> delta -> thread/warp/block aggregates, everything phase B needs moved to
 //     REGISTERS (r, V, delta, live mask, the thread's exclusive map) and the stage handed back at once.
 //     B(k-1) runs AFTER A(k): by then the look-back of tile k-1 has had a whole A phase to finish.
-//   * warp 9: look-back.  Publishes the tile aggregate, walks the predecessors' records 32 at a time (strong relaxed
-//     vector loads, sentinel-initialised records as in v2), stops at the first inclusive record -- at the latest at this
-//     CTA's own previous tile, G tiles back, whose inclusive map it still holds in registers, so a CTA never depends on
-//     another CTA's look-back, only on aggregates -- publishes the inclusive record and hands the carry to the compute
-//     warps through shared memory.
+//   * warp 9: look-back.  Publishes the group aggregates, gathers the records right of the tile, composes them with
+//     this CTA's own previous tile's inclusive map, which it still holds in registers, and hands the carry to the
+//     compute warps through shared memory.
+// A tile is staged only when the launch allows it (every input pointer, and every output pointer when storing, is
+// 16-byte aligned) and all of its 1024 steps and the 4-float V halo exist.  Other tiles take bounds-checked global loads
+// with the reference's expressions as written.
 // Co-residency: the grid is min(tiles, 3 x SMs) CTAs; a CTA waits only for aggregates of lower-numbered tiles, which
 // lower-numbered CTAs (scheduled first) or earlier iterations produce, so a partially resident grid still progresses.
 // ---------------------------------------------------------------------------------------------------------
-#ifndef RLPPO_GAE3_STEPS
-#define RLPPO_GAE3_STEPS 4               // steps per thread (4 or 8)
-#endif
-#ifndef RLPPO_GAE3_CTAS
-#define RLPPO_GAE3_CTAS 3                // resident CTAs per SM
-#endif
-#ifndef RLPPO_GAE3_STAGES
-#define RLPPO_GAE3_STAGES 3
-#endif
-constexpr int kI3 = RLPPO_GAE3_STEPS;
-constexpr int kTile3 = 1024;             // steps per tile
-constexpr int kC3 = kTile3 / kI3;        // compute threads
-constexpr int kT3 = kC3 + 32;            // + look-back warp
-constexpr int kW3 = kC3 / 32;
-constexpr int kStages3 = RLPPO_GAE3_STAGES;
-constexpr int kCtasPerSm3 = RLPPO_GAE3_CTAS;
-static_assert(kI3 == 4 || kI3 == 8, "4 or 8 steps per thread");
-constexpr uint32_t kVBytes3 = kTile3 * 4u + 16u;            // V tile + 4-float halo (only the first is used)
-constexpr uint32_t kOffD3 = kTile3 * 4u;
-constexpr uint32_t kOffV3 = 2u * kTile3 * 4u;
-constexpr uint32_t kOffT3 = kOffV3 + kVBytes3;
-__host__ __device__ constexpr uint32_t stage_bytes3(bool t64) { return kOffT3 + kTile3 * (t64 ? 8u : 4u); }
+constexpr int kItems = 4;                 // steps per thread
+constexpr int kTile = 1024;               // steps per tile
+constexpr int kCompute = kTile / kItems;  // compute threads
+constexpr int kThreads = kCompute + 32;   // + look-back warp
+constexpr int kWarps = kCompute / 32;
+constexpr int kStages = 3;
+constexpr int kCtasPerSm = 3;
+constexpr uint32_t kVBytes = kTile * 4u + 16u;            // V tile + 4-float halo (only the first is used)
+constexpr uint32_t kOffD = kTile * 4u;
+constexpr uint32_t kOffV = 2u * kTile * 4u;
+constexpr uint32_t kOffT = kOffV + kVBytes;
+__host__ __device__ constexpr uint32_t stage_bytes(bool t64) { return kOffT + kTile * (t64 ? 8u : 4u); }
 
-__device__ __forceinline__ void mbar_init3(uint64_t* b, uint32_t cnt) {
+__device__ __forceinline__ void mbar_init(uint64_t* b, uint32_t cnt) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr_u32(b)), "r"(cnt) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive3(uint64_t* b) {
+__device__ __forceinline__ void mbar_arrive(uint64_t* b) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_addr_u32(b)) : "memory");
 }
-__device__ __forceinline__ void mbar_expect_tx3(uint64_t* b, uint32_t bytes) {
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* b, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr_u32(b)), "r"(bytes) : "memory");
 }
-// Waiters back off with nanosleep: the event trace of the first version showed the look-back warp taking 11 us for a
-// 300-instruction shuffle scan -- the scheduler kept issuing the 24 hot-spinning compute warps of the SM instead.
-__device__ __forceinline__ void mbar_wait3(uint64_t* b, uint32_t parity) {
+// Waiters back off with nanosleep: without it the look-back warp took 11 us for a 300-instruction shuffle scan -- the
+// scheduler kept issuing the 24 hot-spinning compute warps of the SM instead.
+__device__ __forceinline__ void mbar_wait(uint64_t* b, uint32_t parity) {
     for (;;) {
         uint32_t ok;
         asm volatile(
@@ -385,74 +170,64 @@ __device__ __forceinline__ void mbar_wait3(uint64_t* b, uint32_t parity) {
 }
 
 // what phase B needs of a tile, per thread, in registers
-struct Pending3 {
-    float r[kI3], v[kI3], dl[kI3];
+struct Pending {
+    float r[kItems], v[kItems], dl[kItems];
     Aff e;            // map of everything right of this thread's steps inside the tile
-    uint32_t live;    // bit i: step i continues the recurrence (fast threads)
-    bool fast;        // flags all exactly 0 / 1 and the tile is a full, staged one
+    // bit i < kItems: step i continues the recurrence; bit kItems (kFast): the flags are all exactly 0 / 1 and the tile
+    // is a staged one.  One word, not a word and a flag: two of these are live at the 72-register cap of 3 CTAs/SM.
+    uint32_t live;
 };
 
 template <bool TRUNC64, bool STORE>
-__global__ void __launch_bounds__(kT3, kCtasPerSm3)
+__global__ void __launch_bounds__(kThreads, kCtasPerSm)
 gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, const void* __restrict__ trunc,
                  const float* __restrict__ val, int64_t n, double gamma, float gl32,
                  const float* __restrict__ ret_std, float* __restrict__ adv, float* __restrict__ vt,
                  float* __restrict__ ret, double* __restrict__ ret_head, int64_t n_head,
                  const double* __restrict__ carry_in, double* __restrict__ summary_out, Workspace ws, int n_tiles,
-                 unsigned long long* __restrict__ trace, int early_poll) {
-    extern __shared__ __align__(128) uint8_t sm3[];
-    __shared__ uint64_t s_full[kStages3], s_aggr[2], s_carr[2];
-    __shared__ double s_wagg[2][kW3][4];
+                 bool can_stage) {
+    extern __shared__ __align__(128) uint8_t smem[];
+    __shared__ uint64_t s_full[kStages], s_aggr[2], s_carr[2];
+    __shared__ double s_wagg[2][kWarps][4];
     __shared__ double s_agg[2][4];
     __shared__ double s_carry[2][2];
 
-    // debug (RLPPO_GAE_TRACE=<file>): globaltimer stamps of three CTAs, [cta slot][tile k < 128][event]
-    const int tr_slot = trace == nullptr ? -1
-                        : (blockIdx.x == 0 ? 0 : ((int)blockIdx.x == (int)gridDim.x / 2 ? 1 : (blockIdx.x == gridDim.x - 1 ? 2 : -1)));
-    auto stamp = [&](int k, int ev) {
-        if (tr_slot >= 0 && k < 128) {
-            unsigned long long now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            trace[(tr_slot * 128 + k) * 8 + ev] = now;
-        }
-    };
-    constexpr uint32_t kStage = stage_bytes3(TRUNC64);
+    constexpr uint32_t kStage = stage_bytes(TRUNC64);
     constexpr uint32_t kTB = TRUNC64 ? 8u : 4u;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int G = gridDim.x;
     const int K = (n_tiles - (int)blockIdx.x + G - 1) / G;      // tiles of this CTA (grid <= n_tiles)
     if (tid == 0) {
-        for (int i = 0; i < kStages3; ++i) {
-            mbar_init3(&s_full[i], 1);
+        for (int i = 0; i < kStages; ++i) {
+            mbar_init(&s_full[i], 1);
         }
         for (int i = 0; i < 2; ++i) {
-            mbar_init3(&s_aggr[i], 1);
-            mbar_init3(&s_carr[i], 1);
+            mbar_init(&s_aggr[i], 1);
+            mbar_init(&s_carr[i], 1);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
 
-    // a tile is staged by bulk copies iff all of its 1024 steps and the 4-float V halo exist
-    auto base_of = [&](int k) { return (int64_t)(n_tiles - 1 - ((int)blockIdx.x + k * G)) * kTile3; };
-    auto staged = [&](int64_t base0) { return base0 + kTile3 + 4 <= n + 1; };
+    auto base_of = [&](int k) { return (int64_t)(n_tiles - 1 - ((int)blockIdx.x + k * G)) * kTile; };
+    auto staged = [&](int64_t base0) { return can_stage && base0 + kTile + 4 <= n + 1; };
 
-    // stage s takes tile k: four bulk copies (one thread); a ragged tile is not staged, its barrier completes at once
+    // stage s takes tile k: four bulk copies (one thread); a tile that is not staged completes its barrier at once
     auto produce = [&](int k) {
-        const int s = k % kStages3;
+        const int s = k % kStages;
         const int64_t base0 = base_of(k);
         if (staged(base0)) {
-            uint8_t* st = sm3 + s * kStage;
-            mbar_expect_tx3(&s_full[s], 2u * kTile3 * 4u + kVBytes3 + kTile3 * kTB);
-            bulk_g2s(st, rew + base0, kTile3 * 4u, &s_full[s]);
-            bulk_g2s(st + kOffD3, done + base0, kTile3 * 4u, &s_full[s]);
-            bulk_g2s(st + kOffV3, val + base0, kVBytes3, &s_full[s]);
-            bulk_g2s(st + kOffT3, static_cast<const uint8_t*>(trunc) + base0 * kTB, kTile3 * kTB, &s_full[s]);
+            uint8_t* st = smem + s * kStage;
+            mbar_expect_tx(&s_full[s], 2u * kTile * 4u + kVBytes + kTile * kTB);
+            bulk_g2s(st, rew + base0, kTile * 4u, &s_full[s]);
+            bulk_g2s(st + kOffD, done + base0, kTile * 4u, &s_full[s]);
+            bulk_g2s(st + kOffV, val + base0, kVBytes, &s_full[s]);
+            bulk_g2s(st + kOffT, static_cast<const uint8_t*>(trunc) + base0 * kTB, kTile * kTB, &s_full[s]);
         } else {
-            mbar_arrive3(&s_full[s]);
+            mbar_arrive(&s_full[s]);
         }
     };
-    if (warp == kW3) {
+    if (warp == kWarps) {
         // ===================== look-back =====================
         // Two-level, chain-free.  CTAs form groups of 32 consecutive block ids; the last CTA of a group also publishes
         // the group's aggregate (its own tile's map composed with its 31 peers') in the second record array.  The map of
@@ -463,9 +238,9 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
         //   S4  aggregates of the higher peers of iteration k-1          block ids group end .. bid+1
         //   then this CTA's own previous tile t-G, whose INCLUSIVE map is still in registers.
         // At most 31 + NG-1 records (<= 64: two per lane), all of them published right after a phase A -- no record
-        // depends on another CTA's look-back, so nothing propagates serially along the rollout.  (The first version
-        // walked 32 predecessors per round until it met an inclusive record: the inclusive frontier advanced 32 tiles
-        // per L2 round trip, 2^26 steps took 2048 round trips = 757 us whatever the memory system did.)
+        // depends on another CTA's look-back, so nothing propagates serially along the rollout.  (Walking predecessors
+        // until an inclusive record turns up advances the inclusive frontier by 32 tiles per L2 round trip: 2^26 steps
+        // took 2048 round trips = 757 us whatever the memory system did.)
         const double cA = carry_in ? carry_in[0] : 0.0;
         const double cR = carry_in ? carry_in[1] : 0.0;
         const int bid = (int)blockIdx.x;
@@ -473,27 +248,22 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
         const int g = bid >> 5, l = bid & 31;
         const int gend = ((32 * g + 31 < G - 1) ? 32 * g + 31 : G - 1) - 32 * g;   // local index of the group's last CTA
         const bool group_last = l == gend;
-        double* const gagg = ws.incl;          // second record array: group aggregates, slot = tile id of the group's first tile
         Aff prev_incl = aff_identity();
         for (int k = 0; k < K; ++k) {
             const int t = bid + k * G;
-            // The polls below do not need this tile's own aggregate: they start while the compute warps are still in
-            // phase A, and the aggregate is only waited for where it is consumed.
-            Aff tile_agg;
-            auto wait_own = [&]() {
-                mbar_wait3(&s_aggr[k & 1], (k >> 1) & 1);
-                tile_agg = Aff{s_agg[k & 1][0], s_agg[k & 1][1], s_agg[k & 1][2], s_agg[k & 1][3]};
-                if (lane == 0) stamp(k, 4);
-            };
-            if (!early_poll) wait_own();
+            mbar_wait(&s_aggr[k & 1], (k >> 1) & 1);
+            // read where consumed, not held in registers across the polls (the kernel is at its register cap); the
+            // compute warps rewrite s_agg[k & 1] only after lane 0 has handed this tile's carry over, and lane 0 is the
+            // only lane whose maps are used
+            auto tile_agg = [&]() { return Aff{s_agg[k & 1][0], s_agg[k & 1][1], s_agg[k & 1][2], s_agg[k & 1][3]}; };
             // the record at position p of the nearest-first list (nullptr: none)
             auto rec_at = [&](int p) -> const double* {
                 if (p < l) return ws.agg + (size_t)(t - 1 - p) * 4;
                 p -= l;
-                if (p < g) return gagg + (size_t)(k * G + 32 * (g - 1 - p)) * 4;
+                if (p < g) return ws.gagg + (size_t)(k * G + 32 * (g - 1 - p)) * 4;
                 p -= g;
                 if (k == 0) return nullptr;
-                if (p < NG - 1 - g) return gagg + (size_t)((k - 1) * G + 32 * (NG - 1 - p)) * 4;
+                if (p < NG - 1 - g) return ws.gagg + (size_t)((k - 1) * G + 32 * (NG - 1 - p)) * 4;
                 p -= NG - 1 - g;
                 if (p < gend - l) return ws.agg + (size_t)((k - 1) * G + 32 * g + gend - p) * 4;
                 return nullptr;
@@ -508,8 +278,8 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
                 // The group aggregate must not wait for anything but the peers' aggregates (positions 0 .. l-1): publishing
                 // it only after the group records of S2/S3 had arrived chained the groups serially, 14 hops per iteration.
                 // Warp-uniform polling loops (every lane iterates until the last record is in): lanes that leave a
-                // divergent spin loop one by one stayed diverged through the shuffle scans below -- the event trace
-                // showed 11 us from "all records arrived" to "carry handed over" for ~400 instructions.
+                // divergent spin loop one by one stay diverged through the shuffle scans below, 11 us from "all records
+                // arrived" to "carry handed over" for ~400 instructions.
                 Aff s1 = aff_identity();
                 const double* ps = lane < l ? ws.agg + (size_t)(t - 1 - lane) * 4 : nullptr;
                 bool need_s = ps != nullptr;
@@ -525,8 +295,7 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
                     const Aff y = shfl_down(s1, off);
                     s1 = compose(s1, y);                       // lanes past the end pull in garbage; lane 0 is exact
                 }
-                if (early_poll) wait_own();
-                if (lane == 0) rec_store(gagg + (size_t)(k * G + 32 * g) * 4, compose(tile_agg, s1));
+                if (lane == 0) rec_store(ws.gagg + (size_t)(k * G + 32 * g) * 4, compose(tile_agg(), s1));
             }
             for (;;) {
                 Aff xa, xb;
@@ -545,8 +314,6 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
                 if (clock64() - t0 > 8000000000LL) __trap();   // watchdog (~4 s)
                 __nanosleep(100);
             }
-            if (lane == 0) stamp(k, 5);
-            if (early_poll && !group_last) wait_own();
             Aff right = compose(ma, mb);
 #pragma unroll
             for (int off = 1; off < 32; off <<= 1) {   // adjacent pairs first: the maps do not commute
@@ -554,7 +321,7 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
                 right = compose(right, y);                     // exact on lane 0 (shfl_down past the end returns own value)
             }
             if (k > 0) right = compose(right, prev_incl);      // lane 0 is the only consumer from here on
-            const Aff incl = compose(tile_agg, right);
+            const Aff incl = compose(tile_agg(), right);
             prev_incl = incl;
             if (lane == 0) {
                 s_carry[k & 1][0] = fma(right.aA, cA, right.bA);
@@ -563,8 +330,7 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
                     summary_out[0] = incl.aA; summary_out[1] = incl.bA;
                     summary_out[2] = incl.aR; summary_out[3] = incl.bR;
                 }
-                mbar_arrive3(&s_carr[k & 1]);       // release: the carry stores above are visible to the waiters
-                stamp(k, 6);
+                mbar_arrive(&s_carr[k & 1]);       // release: the carry stores above are visible to the waiters
             }
             __syncwarp();
         }
@@ -576,77 +342,66 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
     sm.gamma = gamma; sm.gl32 = gl32; sm.gl64 = (double)gl32;
     sm.has_std = ret_std != nullptr;
     sm.stdv = sm.has_std ? __ldg(ret_std) : 1.f;
-    double g4A = (sm.gl64 * sm.gl64) * (sm.gl64 * sm.gl64);            // multiplier of kI3 live steps
-    double g4R = (gamma * gamma) * (gamma * gamma);
-    if (kI3 == 8) {
-        g4A *= g4A;
-        g4R *= g4R;
-    }
-    constexpr uint32_t kAllLive = (1u << kI3) - 1u;
-    const int j0 = tid * kI3;
+    const double g4A = (sm.gl64 * sm.gl64) * (sm.gl64 * sm.gl64);      // multiplier of kItems live steps
+    const double g4R = (gamma * gamma) * (gamma * gamma);
+    constexpr uint32_t kAllLive = (1u << kItems) - 1u, kFast = 1u << kItems;
+    const int j0 = tid * kItems;
 
     // ---- phase A of tile k: everything up to the tile aggregate; the inputs phase B needs end up in `P` ----
-    auto phaseA = [&](int k, Pending3& P) {
-        const int s = k % kStages3;
+    auto phaseA = [&](int k, Pending& P) {
+        const int s = k % kStages;
         const int64_t base0 = base_of(k);
         const bool tile_staged = staged(base0);
-        const uint8_t* st = sm3 + s * kStage;
-        mbar_wait3(&s_full[s], (k / kStages3) & 1);
-        if (tid == 0) stamp(k, 0);
+        const uint8_t* st = smem + s * kStage;
+        mbar_wait(&s_full[s], (k / kStages) & 1);
         Aff agg;
-        P.fast = tile_staged;
         P.live = 0;
         if (tile_staged) {
-            // 16-byte shared-memory accesses, kI3 / 4 per array (at 8 steps per thread the 32-byte thread stride makes them
-            // 2-way bank conflicts: 5 arrays per tile, not what bounds the kernel)
             // flags stay in their storage type: the 0/1 fast path only compares them, and an f32 -> f64 conversion per step
             // (quarter-rate pipe) made the f32-flag scan SLOWER than the f64-flag one although it reads 4 bytes less
             using TFlag = typename std::conditional<TRUNC64, double, float>::type;
-            float dd[kI3], vn[kI3 + 1];
-            TFlag tt[kI3];
-#pragma unroll
-            for (int q = 0; q < kI3 / 4; ++q) {
-                const float4 r4 = *reinterpret_cast<const float4*>(st + (size_t)(j0 + 4 * q) * 4);
-                const float4 d4 = *reinterpret_cast<const float4*>(st + kOffD3 + (size_t)(j0 + 4 * q) * 4);
-                const float4 v4 = *reinterpret_cast<const float4*>(st + kOffV3 + (size_t)(j0 + 4 * q) * 4);
-                P.r[4 * q] = r4.x; P.r[4 * q + 1] = r4.y; P.r[4 * q + 2] = r4.z; P.r[4 * q + 3] = r4.w;
-                dd[4 * q] = d4.x; dd[4 * q + 1] = d4.y; dd[4 * q + 2] = d4.z; dd[4 * q + 3] = d4.w;
-                vn[4 * q] = v4.x; vn[4 * q + 1] = v4.y; vn[4 * q + 2] = v4.z; vn[4 * q + 3] = v4.w;
-                if (TRUNC64) {
-                    const double2 t0 = *reinterpret_cast<const double2*>(st + kOffT3 + (size_t)(j0 + 4 * q) * 8);
-                    const double2 t1 = *reinterpret_cast<const double2*>(st + kOffT3 + (size_t)(j0 + 4 * q) * 8 + 16);
-                    tt[4 * q] = t0.x; tt[4 * q + 1] = t0.y; tt[4 * q + 2] = t1.x; tt[4 * q + 3] = t1.y;
-                } else {
-                    const float4 t4 = *reinterpret_cast<const float4*>(st + kOffT3 + (size_t)(j0 + 4 * q) * 4);
-                    tt[4 * q] = t4.x; tt[4 * q + 1] = t4.y; tt[4 * q + 2] = t4.z; tt[4 * q + 3] = t4.w;
-                }
+            float dd[kItems], vn[kItems + 1];
+            TFlag tt[kItems];
+            const float4 r4 = *reinterpret_cast<const float4*>(st + (size_t)j0 * 4);
+            const float4 d4 = *reinterpret_cast<const float4*>(st + kOffD + (size_t)j0 * 4);
+            const float4 v4 = *reinterpret_cast<const float4*>(st + kOffV + (size_t)j0 * 4);
+            P.r[0] = r4.x; P.r[1] = r4.y; P.r[2] = r4.z; P.r[3] = r4.w;
+            dd[0] = d4.x; dd[1] = d4.y; dd[2] = d4.z; dd[3] = d4.w;
+            vn[0] = v4.x; vn[1] = v4.y; vn[2] = v4.z; vn[3] = v4.w;
+            if (TRUNC64) {
+                const double2 t0 = *reinterpret_cast<const double2*>(st + kOffT + (size_t)j0 * 8);
+                const double2 t1 = *reinterpret_cast<const double2*>(st + kOffT + (size_t)j0 * 8 + 16);
+                tt[0] = t0.x; tt[1] = t0.y; tt[2] = t1.x; tt[3] = t1.y;
+            } else {
+                const float4 t4 = *reinterpret_cast<const float4*>(st + kOffT + (size_t)j0 * 4);
+                tt[0] = t4.x; tt[1] = t4.y; tt[2] = t4.z; tt[3] = t4.w;
             }
-            vn[kI3] = *reinterpret_cast<const float*>(st + kOffV3 + (size_t)(j0 + kI3) * 4);
+            vn[kItems] = *reinterpret_cast<const float*>(st + kOffV + (size_t)(j0 + kItems) * 4);
             bool ok = true;
 #pragma unroll
-            for (int i = 0; i < kI3; ++i) {
+            for (int i = 0; i < kItems; ++i) {
                 P.v[i] = vn[i];
                 const bool dz = dd[i] == 0.f, tz = tt[i] == (TFlag)0;
                 ok = ok && (dz || dd[i] == 1.f) && (tz || tt[i] == (TFlag)1);
                 P.live |= (dz && tz ? 1u : 0u) << i;
                 P.dl[i] = sm.delta_of(P.r[i], dd[i], vn[i], vn[i + 1]);
             }
-            P.fast = ok;
             if (ok) {
                 // multipliers are 0 or a constant: only the additive parts need arithmetic
                 double bA = 0.0, bR = 0.0;
 #pragma unroll
-                for (int i = kI3 - 1; i >= 0; --i) {
+                for (int i = kItems - 1; i >= 0; --i) {
                     const bool lv = (P.live >> i) & 1u;
                     bA = fma(lv ? sm.gl64 : 0.0, bA, (double)P.dl[i]);
                     bR = fma(lv ? gamma : 0.0, bR, (double)P.r[i]);
                 }
                 const bool all = P.live == kAllLive;
                 agg = Aff{all ? g4A : 0.0, bA, all ? g4R : 0.0, bR};
+                P.live |= kFast;
             } else {
                 agg = aff_identity();
 #pragma unroll
-                for (int i = kI3 - 1; i >= 0; --i) {
+                for (int i = kItems - 1; i >= 0; --i) {
                     const float nd = __fsub_rn(1.0f, dd[i]);                              // :59
                     const double nt = 1.0 - (double)tt[i];                                // :60
                     const Aff f = Aff{(double)__fmul_rn(gl32, nd) * nt, (double)P.dl[i],  // :72
@@ -655,16 +410,16 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
                 }
             }
         } else {
-            // ragged tile: bounds-checked global loads, the reference's expressions as written; steps past the end are
-            // identity maps so that the carry passes through them
-            const int cnt = (int)((n - base0) < (int64_t)kTile3 ? (n - base0) : (int64_t)kTile3);
+            // tile not staged: bounds-checked global loads, the reference's expressions as written; steps past the end
+            // are identity maps so that the carry passes through them
+            const int cnt = (int)((n - base0) < (int64_t)kTile ? (n - base0) : (int64_t)kTile);
             sm.r = rew + base0; sm.d = done + base0; sm.v = val + base0;
             sm.t = static_cast<const uint8_t*>(trunc) + base0 * kTB;
             agg = aff_identity();
 #pragma unroll
-            for (int i = 0; i < kI3; ++i) P.r[i] = P.v[i] = P.dl[i] = 0.f;
+            for (int i = 0; i < kItems; ++i) P.r[i] = P.v[i] = P.dl[i] = 0.f;
 #pragma unroll
-            for (int i = kI3 - 1; i >= 0; --i)
+            for (int i = kItems - 1; i >= 0; --i)
                 if (j0 + i < cnt) {
                     Aff f;
                     sm.mults(j0 + i, f.aA, f.aR);
@@ -684,48 +439,46 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
             wagg[warp][0] = incl_w.aA; wagg[warp][1] = incl_w.bA;
             wagg[warp][2] = incl_w.aR; wagg[warp][3] = incl_w.bR;
         }
-        asm volatile("bar.sync 1, %0;" ::"n"(kC3) : "memory");
+        asm volatile("bar.sync 1, %0;" ::"n"(kCompute) : "memory");
         // every compute warp has read stage s into registers by now: refill it with the tile three ahead
-        if (tid == 0 && k + kStages3 < K) {
+        if (tid == 0 && k + kStages < K) {
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy reads before the async-proxy refill
-            produce(k + kStages3);
+            produce(k + kStages);
         }
         // every warp scans the 8 warp aggregates itself (lanes 0-7): no second barrier
         Aff w = aff_identity();
-        if (lane < kW3) w = Aff{wagg[lane][0], wagg[lane][1], wagg[lane][2], wagg[lane][3]};
+        if (lane < kWarps) w = Aff{wagg[lane][0], wagg[lane][1], wagg[lane][2], wagg[lane][3]};
 #pragma unroll
-        for (int off = 1; off < kW3; off <<= 1) {
+        for (int off = 1; off < kWarps; off <<= 1) {
             const Aff y = shfl_down(w, off);
-            if (lane + off < kW3) w = compose(w, y);
+            if (lane + off < kWarps) w = compose(w, y);
         }
         // lane l < 8 now holds warps l..7; this warp's exclusive = lane warp+1 (identity for the last warp)
         Aff we = shfl_idx(w, (warp + 1) & 31);
-        if (warp == kW3 - 1) we = aff_identity();
+        if (warp == kWarps - 1) we = aff_identity();
         if (tid == 0) {
             // published from here, not by the look-back warp: that one may still be busy with the previous tile
             rec_store(ws.agg + (size_t)((int)blockIdx.x + k * G) * 4, w);
             s_agg[k & 1][0] = w.aA; s_agg[k & 1][1] = w.bA; s_agg[k & 1][2] = w.aR; s_agg[k & 1][3] = w.bR;
-            mbar_arrive3(&s_aggr[k & 1]);
-            stamp(k, 1);
+            mbar_arrive(&s_aggr[k & 1]);
         }
         P.e = compose(excl, we);
     };
 
     // ---- phase B of tile k: apply the carry, write the outputs ----
-    auto phaseB = [&](int k, const Pending3& P) {
+    auto phaseB = [&](int k, const Pending& P) {
         const int64_t base0 = base_of(k);
-        mbar_wait3(&s_carr[k & 1], (k >> 1) & 1);     // also the flow control that keeps s_agg / s_aggr two tiles deep
-        if (tid == 0) stamp(k, 2);
+        mbar_wait(&s_carr[k & 1], (k >> 1) & 1);     // also the flow control that keeps s_agg / s_aggr two tiles deep
         if (!STORE) return;
         const double carryA = s_carry[k & 1][0], carryR = s_carry[k & 1][1];
         double xA = fma(P.e.aA, carryA, P.e.bA);
         double xR = fma(P.e.aR, carryR, P.e.bR);
         const int64_t gbase = base0 + j0;
         const bool head = ret_head != nullptr && gbase < n_head;
-        float oa[kI3], ov[kI3], orr[kI3];
-        if (P.fast) {
+        if (P.live & kFast) {
+            float oa[kItems], ov[kItems], orr[kItems];
 #pragma unroll
-            for (int i = kI3 - 1; i >= 0; --i) {
+            for (int i = kItems - 1; i >= 0; --i) {
                 const bool lv = (P.live >> i) & 1u;
                 xA = fma(lv ? sm.gl64 : 0.0, xA, (double)P.dl[i]);
                 xR = fma(lv ? gamma : 0.0, xR, (double)P.r[i]);
@@ -734,20 +487,17 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
                 ov[i] = (float)((double)P.v[i] + xA);           // :77
                 orr[i] = (float)xR;
             }
-#pragma unroll
-            for (int q = 0; q < kI3 / 4; ++q) {
-                *reinterpret_cast<float4*>(adv + gbase + 4 * q) = make_float4(oa[4 * q], oa[4 * q + 1], oa[4 * q + 2], oa[4 * q + 3]);
-                *reinterpret_cast<float4*>(vt + gbase + 4 * q) = make_float4(ov[4 * q], ov[4 * q + 1], ov[4 * q + 2], ov[4 * q + 3]);
-                *reinterpret_cast<float4*>(ret + gbase + 4 * q) = make_float4(orr[4 * q], orr[4 * q + 1], orr[4 * q + 2], orr[4 * q + 3]);
-            }
+            *reinterpret_cast<float4*>(adv + gbase) = make_float4(oa[0], oa[1], oa[2], oa[3]);
+            *reinterpret_cast<float4*>(vt + gbase) = make_float4(ov[0], ov[1], ov[2], ov[3]);
+            *reinterpret_cast<float4*>(ret + gbase) = make_float4(orr[0], orr[1], orr[2], orr[3]);
         } else {
-            // generic flags / ragged tile: the multipliers again, from global memory (rare)
-            const int cnt = (int)((n - base0) < (int64_t)kTile3 ? (n - base0) : (int64_t)kTile3);
+            // generic flags / tile not staged: the multipliers again, from global memory (rare)
+            const int cnt = (int)((n - base0) < (int64_t)kTile ? (n - base0) : (int64_t)kTile);
             StepMaps<TRUNC64> g = sm;
             g.r = rew + base0; g.d = done + base0; g.v = val + base0;
             g.t = static_cast<const uint8_t*>(trunc) + base0 * kTB;
 #pragma unroll
-            for (int i = kI3 - 1; i >= 0; --i)
+            for (int i = kItems - 1; i >= 0; --i)
                 if (j0 + i < cnt) {
                     double aA, aR;
                     g.mults(j0 + i, aA, aR);
@@ -759,13 +509,12 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
                     ret[gbase + i] = (float)xR;
                 }
         }
-        if (tid == 0) stamp(k, 3);
     };
 
     // A(k) runs one tile ahead of B(k-1); two register sets alternate (unrolled by two: no dynamic indexing)
     if (tid == 0)
-        for (int kk = 0; kk < kStages3 && kk < K; ++kk) produce(kk);
-    Pending3 P0, P1;
+        for (int kk = 0; kk < kStages && kk < K; ++kk) produce(kk);
+    Pending P0, P1;
     phaseA(0, P0);
     int k = 1;
     for (; k + 1 < K; k += 2) {
@@ -783,21 +532,8 @@ gae_scan3_kernel(const float* __restrict__ rew, const float* __restrict__ done, 
     }
 }
 
-inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
-struct WsLayout {
-    size_t status_off, agg_off, incl_off, total, clear_bytes;
-};
-WsLayout ws_layout(int64_t n) {
-    const size_t n_tiles = (size_t)((n + kTile3 - 1) / kTile3);   // the finest tiling any of the kernels uses
-    WsLayout L;
-    L.status_off = 16;
-    L.clear_bytes = align_up(16 + n_tiles * sizeof(int), 16);
-    L.agg_off = align_up(L.clear_bytes, 256);
-    L.incl_off = L.agg_off + n_tiles * 4 * sizeof(double);
-    L.total = L.incl_off + n_tiles * 4 * sizeof(double);
-    return L;
-}
+// the two record arrays of n steps' tiles (see Workspace)
+size_t ws_bytes_for(int64_t n) { return 2 * (size_t)((n + kTile - 1) / kTile) * 4 * sizeof(double); }
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
@@ -806,82 +542,40 @@ int launch_gae(const float* rew, const float* done, const void* trunc, int trunc
                int64_t n, double gamma, double lambda, const float* ret_std, float* adv, float* vtarget,
                float* ret, double* ret_head64, int64_t n_head, const double* carry_in, double* summary_out,
                void* wsp, size_t ws_bytes, cudaStream_t s) {
-    const WsLayout L = ws_layout(n);
-    if (ws_bytes < L.total || wsp == nullptr) {
-        rlppo::set_error("gae workspace too small: %zu < %zu", ws_bytes, L.total);
+    const size_t need = ws_bytes_for(n);
+    if (ws_bytes < need || wsp == nullptr) {
+        rlppo::set_error("gae workspace too small: %zu < %zu", ws_bytes, need);
         return RLPPO_ERR_WORKSPACE;
     }
     RLPPO_CHECK_ARG(aligned16(wsp), "gae workspace must be 16-byte aligned");
     const int n_tiles = (int)((n + kTile - 1) / kTile);
-    char* base = static_cast<char*>(wsp);
-    Workspace ws{reinterpret_cast<int*>(base), reinterpret_cast<int*>(base + L.status_off),
-                 reinterpret_cast<double*>(base + L.agg_off), reinterpret_cast<double*>(base + L.incl_off)};
-    RLPPO_CUDA(cudaMemsetAsync(base, 0, L.clear_bytes, s));
+    Workspace ws{static_cast<double*>(wsp), static_cast<double*>(wsp) + (size_t)n_tiles * 4};
+    RLPPO_CUDA(cudaMemsetAsync(wsp, 0xFF, need, s));   // every record unset (see rec_load)
     const float gl32 = (float)(gamma * lambda);
-    bool vec = aligned16(rew) && aligned16(done) && aligned16(trunc) && aligned16(values);
-    if (STORE) vec = vec && aligned16(adv) && aligned16(vtarget) && aligned16(ret);
-#define RLPPO_GAE_LAUNCH(T64, V)                                                                         \
-    gae_scan_kernel<T64, V, STORE><<<n_tiles, kThreads, 0, s>>>(rew, done, trunc, values, n, gamma, gl32, \
-                                                                ret_std, adv, vtarget, ret, ret_head64,  \
-                                                                n_head, carry_in, summary_out, ws, n_tiles)
-    if (vec) {
-        // persistent pipelined kernel (v3): 1024-step tiles, records pre-set to the all-ones sentinel
-        const int n_tiles3 = (int)((n + kTile3 - 1) / kTile3);
-        const size_t smem = (size_t)kStages3 * stage_bytes3(trunc_is_f64 != 0);
-        RLPPO_CUDA(cudaMemsetAsync(base + L.agg_off, 0xFF, L.total - L.agg_off, s));
-        // debug trace (see the kernel): RLPPO_GAE_TRACE=<file> dumps the stamps of this launch after a synchronise
-        static const char* trace_env = getenv("RLPPO_GAE_TRACE");
-        static const char* trace_path = (trace_env != nullptr && trace_env[0] != 0) ? trace_env : nullptr;
-        static unsigned long long* trace_dev = nullptr;
-        constexpr size_t kTraceWords = 3 * 128 * 8;
-        if (trace_path != nullptr) {
-            if (trace_dev == nullptr) RLPPO_CUDA(cudaMalloc(&trace_dev, kTraceWords * 8));
-            RLPPO_CUDA(cudaMemsetAsync(trace_dev, 0, kTraceWords * 8, s));
+    bool can_stage = aligned16(rew) && aligned16(done) && aligned16(trunc) && aligned16(values);
+    if (STORE) can_stage = can_stage && aligned16(adv) && aligned16(vtarget) && aligned16(ret);
+    const size_t smem = (size_t)kStages * stage_bytes(trunc_is_f64 != 0);
+    static bool configured[2] = {false, false};
+    static int resident[2] = {0, 0};
+    auto launch = [&](auto kfn, int which) -> cudaError_t {
+        if (!configured[which]) {
+            cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                 (int)(kStages * stage_bytes(true)));
+            if (e != cudaSuccess) return e;
+            // every CTA of the grid must be able to be resident at once (see the kernel's header comment)
+            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident[which], kfn, kThreads, kStages * stage_bytes(true));
+            if (e != cudaSuccess) return e;
+            if (resident[which] < 1) return cudaErrorLaunchOutOfResources;
+            configured[which] = true;
         }
-        static const int early_poll = getenv("RLPPO_GAE_EARLY") != nullptr ? atoi(getenv("RLPPO_GAE_EARLY")) : 0;
-        static bool configured3[2] = {false, false};
-        static int resident3[2] = {0, 0};
-        auto launch3 = [&](auto kfn, int which) -> cudaError_t {
-            if (!configured3[which]) {
-                cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                     (int)(kStages3 * stage_bytes3(true)));
-                if (e != cudaSuccess) return e;
-                // every CTA of the grid must be able to be resident at once (see the kernel's header comment)
-                e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident3[which], kfn, kT3,
-                                                                  kStages3 * stage_bytes3(true));
-                if (e != cudaSuccess) return e;
-                if (resident3[which] < 1) return cudaErrorLaunchOutOfResources;
-                configured3[which] = true;
-            }
-            int cap = resident3[which] * rlppo::num_sms();
-            static const char* grid_env = getenv("RLPPO_GAE_GRID");      // experiments only: fewer persistent CTAs
-            if (grid_env != nullptr && atoi(grid_env) > 0 && atoi(grid_env) < cap) cap = atoi(grid_env);
-            const int grid = n_tiles3 < cap ? n_tiles3 : cap;
-            kfn<<<grid, kT3, smem, s>>>(rew, done, trunc, values, n, gamma, gl32, ret_std, adv, vtarget, ret, ret_head64,
-                                       n_head, carry_in, summary_out, ws, n_tiles3, trace_dev, early_poll);
-            return cudaSuccess;
-        };
-        if (trunc_is_f64) RLPPO_CUDA(launch3(gae_scan3_kernel<true, STORE>, 1));
-        else RLPPO_CUDA(launch3(gae_scan3_kernel<false, STORE>, 0));
-        if (trace_path != nullptr) {
-            static unsigned long long host[kTraceWords];
-            RLPPO_CUDA(cudaStreamSynchronize(s));
-            RLPPO_CUDA(cudaMemcpy(host, trace_dev, sizeof(host), cudaMemcpyDeviceToHost));
-            if (FILE* f = fopen(trace_path, "w")) {
-                for (size_t i = 0; i < kTraceWords; i += 8) {
-                    fprintf(f, "%zu %zu", i / 8 / 128, (i / 8) % 128);
-                    for (int e = 0; e < 8; ++e) fprintf(f, " %llu", host[i + e]);
-                    fprintf(f, "\n");
-                }
-                fclose(f);
-            }
-        }
-    } else if (trunc_is_f64) {
-        RLPPO_GAE_LAUNCH(true, false);
-    } else {
-        RLPPO_GAE_LAUNCH(false, false);
-    }
-#undef RLPPO_GAE_LAUNCH
+        const int cap = resident[which] * rlppo::num_sms();
+        const int grid = n_tiles < cap ? n_tiles : cap;
+        kfn<<<grid, kThreads, smem, s>>>(rew, done, trunc, values, n, gamma, gl32, ret_std, adv, vtarget, ret, ret_head64,
+                                         n_head, carry_in, summary_out, ws, n_tiles, can_stage);
+        return cudaSuccess;
+    };
+    if (trunc_is_f64) RLPPO_CUDA(launch(gae_scan3_kernel<true, STORE>, 1));
+    else RLPPO_CUDA(launch(gae_scan3_kernel<false, STORE>, 0));
     RLPPO_LAUNCH_CHECK();
     return RLPPO_OK;
 }
@@ -909,7 +603,7 @@ int rlppo_gae_compose_carry(const double* summaries, int rank, int world, double
     return RLPPO_OK;
 }
 
-size_t rlppo_gae_workspace_bytes(int64_t n) { return ws_layout(n < 1 ? 1 : n).total; }
+size_t rlppo_gae_workspace_bytes(int64_t n) { return ws_bytes_for(n < 1 ? 1 : n); }
 
 int rlppo_gae_f32(const float* rew, const float* done, const void* trunc, int trunc_is_f64, const float* values,
                   int64_t n, double gamma, double lambda, const float* ret_std, float* adv, float* vtarget,

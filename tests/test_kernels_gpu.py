@@ -111,35 +111,62 @@ def test_gae_fractional_and_negative_zero_flags(ops, trunc_dtype):
             assert (got != want).mean() < 1e-3, (name, "bit mismatch rate", float((got != want).mean()))
 
 
+def _assert_vs_oracle(outs, want, case):
+    """(vt, adv, ret) device tensors against the oracle's (vt, adv, ret): 1e-5 scale-aware, bit mismatches < 1e-3."""
+    for name, got, w in zip(("vt", "adv", "ret"), outs, want):
+        got, w = got.cpu().numpy(), w.astype(np.float32)
+        err = np.abs(got - w) / np.maximum(np.abs(w), 1.0)
+        assert err.max() <= 1e-5, (case, name, float(err.max()))
+        assert (got != w).mean() < 1e-3, (case, name, "bit mismatch rate", float((got != w).mean()))
+
+
 def test_gae_unaligned_views_and_carry(ops):
-    """Misaligned pointers take the scalar path; carry_in + chunk summaries reproduce the unsharded scan."""
-    rng = np.random.RandomState(3)
-    n = 10007
-    rew = (rng.randn(n) * 0.1).astype(np.float32)
-    done = (rng.rand(n) < 0.002).astype(np.float32)
-    trunc = np.zeros(n, np.float32)
-    val = rng.randn(n + 1).astype(np.float32)
-    vt0, adv0, ret0 = O.gae_nep50_c(rew, done, trunc, val, 0.99, 0.95, None)
-    pad = lambda a: dev(np.concatenate([[0], a]).astype(a.dtype))[1:]  # noqa: E731  4-byte-offset views
-    vt, adv, ret = ops.gae(pad(rew), pad(done), pad(trunc), pad(val), 0.99, 0.95, None)
-    assert np.allclose(adv.cpu().numpy(), adv0, rtol=1e-6, atol=1e-6)
-    assert np.allclose(ret.cpu().numpy(), ret0, rtol=1e-6, atol=1e-6)
-    # two shards: right shard first, its first values are the left shard's carry
-    cut = 6000
-    r, d, t, v = dev(rew), dev(done), dev(trunc), dev(val)
-    vt_r, adv_r, ret_r = ops.gae(r[cut:].clone(), d[cut:].clone(), t[cut:].clone(), v[cut:].clone(), 0.99, 0.95, None)
-    summ = ops.gae_chunk_summary(r[cut:].clone(), d[cut:].clone(), t[cut:].clone(), v[cut:].clone(), 0.99, 0.95, None)
-    torch.cuda.synchronize()
-    s = summ.cpu().numpy()
-    assert abs(s[1] - float(adv0[cut])) < 1e-5 and abs(s[3] - float(ret0[cut])) < 1e-5
-    # carry = exact f64 values right of the cut; take them from the f64 oracle
-    _, _, ret64 = O.gae_fp64(rew, done, trunc, val, 0.99, 0.95, None)
-    carry = dev(np.asarray([s[1], s[3]], np.float64))
-    vt_l, adv_l, ret_l = ops.gae(r[:cut].clone(), d[:cut].clone(), t[:cut].clone(), v[:cut + 1].clone(), 0.99, 0.95,
-                                 None, carry_in=carry)
-    assert np.allclose(adv_l.cpu().numpy(), adv0[:cut], rtol=1e-6, atol=1e-6)
-    assert np.allclose(ret_l.cpu().numpy(), ret0[:cut], rtol=1e-6, atol=1e-6)
-    assert np.allclose(adv_r.cpu().numpy(), adv0[cut:], rtol=1e-6, atol=1e-6)
+    """Misaligned inputs, misaligned `out=` buffers and chunk summaries of misaligned views take the bounds-checked path
+    on every tile; carry_in + chunk summaries reproduce the unsharded scan.  600001 steps > 444 CTAs x 1024: CTAs take
+    several tiles."""
+    for n, cut in ((10007, 6000), (600001, 360000)):
+        for trunc_dtype in (np.float32, np.float64):
+            case = (n, trunc_dtype.__name__)
+            rng = np.random.RandomState(3)
+            rew = (rng.randn(n) * 0.1).astype(np.float32)
+            done = (rng.rand(n) < 0.002).astype(np.float32)
+            val = rng.randn(n + 1).astype(np.float32)
+            trunc = ((rng.rand(n) < 1 / 1500) * (1 - done)).astype(trunc_dtype)
+            vt0, adv0, ret0 = O.gae_nep50_c(rew, done, trunc, val, 0.99, 0.95, None)
+            pad = lambda a: dev(np.concatenate([[0], a]).astype(a.dtype))[1:]  # noqa: E731  4-byte-offset views
+            vt, adv, ret = ops.gae(pad(rew), pad(done), pad(trunc), pad(val), 0.99, 0.95, None)
+            assert np.allclose(adv.cpu().numpy(), adv0, rtol=1e-6, atol=1e-6), case
+            assert np.allclose(ret.cpu().numpy(), ret0, rtol=1e-6, atol=1e-6), case
+            _assert_vs_oracle((vt, adv, ret), (vt0, adv0, ret0), case)
+            # aligned inputs, outputs at a 4-byte offset
+            out = tuple(torch.zeros(n + 1, dtype=torch.float32, device=DEV)[1:] for _ in range(3))
+            ops.gae(dev(rew), dev(done), dev(trunc), dev(val), 0.99, 0.95, None, out=out)
+            _assert_vs_oracle(out, (vt0, adv0, ret0), case)
+            # two shards: right shard first, its first values are the left shard's carry
+            r, d, t, v = dev(rew), dev(done), dev(trunc), dev(val)
+            vt_r, adv_r, ret_r = ops.gae(r[cut:].clone(), d[cut:].clone(), t[cut:].clone(), v[cut:].clone(), 0.99, 0.95,
+                                         None)
+            _assert_vs_oracle((vt_r, adv_r, ret_r), (vt0[cut:], adv0[cut:], ret0[cut:]), case)
+            summ = ops.gae_chunk_summary(r[cut:].clone(), d[cut:].clone(), t[cut:].clone(), v[cut:].clone(), 0.99, 0.95,
+                                         None)
+            s = summ.cpu().numpy()
+            assert abs(s[1] - float(adv0[cut])) < 1e-5 and abs(s[3] - float(ret0[cut])) < 1e-5, case
+            summ_u = ops.gae_chunk_summary(pad(rew[cut:]), pad(done[cut:]), pad(trunc[cut:]), pad(val[cut:]), 0.99, 0.95,
+                                           None)
+            s_u = summ_u.cpu().numpy()
+            assert abs(s_u[1] - float(adv0[cut])) < 1e-5 and abs(s_u[3] - float(ret0[cut])) < 1e-5, case
+            assert np.allclose(s_u, s, rtol=1e-12, atol=1e-12), case
+            # carry = the right shard's values at its first step: bA and bR of its summary
+            carry = dev(np.asarray([s[1], s[3]], np.float64))
+            vt_l, adv_l, ret_l = ops.gae(r[:cut].clone(), d[:cut].clone(), t[:cut].clone(), v[:cut + 1].clone(), 0.99,
+                                         0.95, None, carry_in=carry)
+            assert np.allclose(adv_l.cpu().numpy(), adv0[:cut], rtol=1e-6, atol=1e-6), case
+            assert np.allclose(ret_l.cpu().numpy(), ret0[:cut], rtol=1e-6, atol=1e-6), case
+            assert np.allclose(adv_r.cpu().numpy(), adv0[cut:], rtol=1e-6, atol=1e-6), case
+            _assert_vs_oracle((vt_l, adv_l, ret_l), (vt0[:cut], adv0[:cut], ret0[:cut]), case)
+            # the left shard again from misaligned views, with the same carry
+            _assert_vs_oracle(ops.gae(pad(rew[:cut]), pad(done[:cut]), pad(trunc[:cut]), pad(val[:cut + 1]), 0.99, 0.95,
+                                      None, carry_in=carry), (vt0[:cut], adv0[:cut], ret0[:cut]), case)
 
 
 def test_gae_linearity_full_size(ops):
