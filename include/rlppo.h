@@ -467,6 +467,37 @@ int rlppo_norm_clip_adam_peers2(float* params, const float* const* h_peer_grads,
 int rlppo_sqdiff(const float* a, const float* b, const int64_t* h_seg_off, int n_seg, float* out,
                  void* stream);
 
+/* ---- wide discrete head: DiscreteFF with 257 <= n_actions <= 4096 -------------------------------------------------
+ * The fused epilogue of rlppo_policy_head_* holds a row's logits in one TMEM tile (<= 256 actions).  Wider softmax
+ * policies run their last Linear as rlppo_linear_fwd_split (relu = 0, out_parts = 3: fp32-exact logits as split bf16
+ * parts, as the (f-4) heads above) and these per-row kernels over it, one warp per row.  The z view is as for the (f-4)
+ * heads and must allow 16-byte accesses: z 16-byte aligned, ldz and z_pstride multiples of 8, every part pad8(n_actions)
+ * columns wide.  The arithmetic is that of the epilogue forms (p = clamp(softmax(z), 1e-11, 1)); only the order of the
+ * row sums differs.  Every entry point checks 257 <= n_actions <= 4096.
+ *   _sample (DiscreteFF.get_action / get_output, discrete_policy.py:35-62): as rlppo_policy_head_sample: inverse-CDF
+ *     draw against u * (total clamped mass), u from u_inject f32[M] or Philox4x32-10(seed, offset + row), subsequence 0,
+ *     u = (x >> 8) / 2^24; deterministic != 0: per-row argmax (first of ties), logp = log clamp(1/S).  Outputs (any may be
+ *     NULL, not all): actions_out f32[M], actions_i64_out int64[M], logp_out f32[M], probs_out f32[M, n_actions] (the
+ *     unclamped softmax).
+ *   _train (get_backprop_data :64-80 + the PPO loss block ppo_learner.py:146-180): as rlppo_policy_head_train, with
+ *     actions f32[M] (clamped to [0, n_actions-1]), d(logits) written as dz_parts bf16 parts of dz_cols columns
+ *     (dz_cols a multiple of 8 >= pad8(n_actions), dz_pstride apart; columns past n_actions zeroed), metrics f32[8] as
+ *     there ([0..4] accumulated), logp_out optional f32[M].
+ *   _backward (autograd, discrete_policy.py:35-80): as rlppo_policy_head_backward: d_logp f32[M], d_ent f32[1] (of the
+ *     mean entropy), d_probs f32[M, n_actions] (of get_output's unclamped softmax), each optional; dz as for _train. */
+int rlppo_head_discrete_sample(const uint16_t* z, int64_t ldz, int z_parts, int64_t z_pstride, int64_t M, int n_actions,
+                               const float* u_inject, uint64_t seed, uint64_t offset, int deterministic,
+                               float* actions_out, int64_t* actions_i64_out, float* logp_out, float* probs_out,
+                               void* stream);
+int rlppo_head_discrete_train(const uint16_t* z, int64_t ldz, int z_parts, int64_t z_pstride, int64_t M, int n_actions,
+                              const float* actions, const float* old_logp, const float* adv, float inv_batch, float clip,
+                              float ent_coef, uint16_t* dz, int64_t lddz, int dz_parts, int64_t dz_pstride, int dz_cols,
+                              float* logp_out, float* metrics, void* stream);
+int rlppo_head_discrete_backward(const uint16_t* z, int64_t ldz, int z_parts, int64_t z_pstride, int64_t M,
+                                 int n_actions, const float* actions, const float* d_logp, const float* d_ent,
+                                 const float* d_probs, uint16_t* dz, int64_t lddz, int dz_parts, int64_t dz_pstride,
+                                 int dz_cols, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

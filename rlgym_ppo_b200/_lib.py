@@ -89,6 +89,9 @@ _SIGS = {
     "rlppo_norm_clip_adam_peers2": ([_P, _P, _P, _P, _I, _I, _P, _P, _P, _I, _P, _P, _P, _D, _D, _D, _D, _P, _I, _P,
                                      ctypes.c_size_t, _P], _I),
     "rlppo_sqdiff": ([_P, _P, _P, _I, _P, _P], _I),
+    "rlppo_head_discrete_sample": ([_P, _L, _I, _L, _L, _I, _P, _U64, _U64, _I, _P, _P, _P, _P, _P], _I),
+    "rlppo_head_discrete_train": ([_P, _L, _I, _L, _L, _I, _P, _P, _P, _F, _F, _F, _P, _L, _I, _L, _I, _P, _P, _P], _I),
+    "rlppo_head_discrete_backward": ([_P, _L, _I, _L, _L, _I, _P, _P, _P, _P, _P, _L, _I, _L, _I, _P], _I),
 }
 
 EXPORTED = tuple(_SIGS)

@@ -71,8 +71,13 @@ class TickInference(object):
             ops.u64_add(self.offset_dev, self.S)
         elif hasattr(pol, "n_actions"):                 # DiscreteFF, layer by layer
             h = st.forward_hidden(ws["x"], self.S, ws)
-            st.policy_head_sample(h, self.S, pol.n_actions, seed=pol._seed, offset=pol._offset, actions_out=self.act_dev,
-                                  logp_out=self.logp_dev)
+            if pol.wide:                                # above 256 actions: logits + per-row sampling kernel
+                z, parts, ps = st.logits(h, self.S, ws)
+                ops.head_discrete_sample(z, parts, ps, self.S, pol.n_actions, seed=pol._seed, offset=pol._offset,
+                                         actions_out=self.act_dev, logp_out=self.logp_dev)
+            else:
+                st.policy_head_sample(h, self.S, pol.n_actions, seed=pol._seed, offset=pol._offset,
+                                      actions_out=self.act_dev, logp_out=self.logp_dev)
             pol._offset += self.S
         else:                                           # MultiDiscreteFF / ContinuousPolicy: logits + per-row head kernel
             h = st.forward_hidden(ws["x"], self.S, ws)

@@ -10,6 +10,8 @@
 // UPSTREAM instantiations (rlppo_head_*_backward): the same backward into the logits with the PPO block replaced by
 // loaded upstream gradients of get_backprop_data's outputs (d_logp f32[M], d_ent f32[1] of the mean entropy) and, for
 // the continuous head, of get_output's (mean, std) -- any of them NULL.
+// The wide discrete head (DiscreteFF with 257..4096 actions, head_discrete_kernel below) is the same kind of tail for
+// the softmax policy whose rows are too wide for the fused epilogue of the head GEMM: one warp per row.
 #include <math.h>
 
 #include "common.cuh"
@@ -295,6 +297,318 @@ __global__ void head_ct_kernel(ZView z, int64_t M, int n_act, float var_m, float
     metrics_add(metrics, ent, r, ok);
 }
 
+// ---- Discrete, wide (257..4096 actions) ---------------------------------------------------------------------------
+// DiscreteFF (discrete_policy.py:22-80) for action spaces too wide for the head GEMM's fused epilogue, where a row's
+// logits must fit one TMEM tile (<= 256 columns).  The last Linear writes its logits as split parts (rlppo_linear_fwd_split)
+// and this kernel is the per-row tail, one warp per row (grid-stride over the rows):
+//   1. the row's logits, summed from their parts, into shared memory (the only HBM read of z: each lane loads 8
+//      consecutive columns of a part as one 16-byte word, so a warp reads 512 contiguous bytes per part and load), with
+//      the row max and the first argmax;
+//   2. e_j = exp(z_j - max) in place, S = sum e;
+//   3. sample: total clamped mass P (and probs_out = e/S); train: entropy, the clamp-masked sum of s (log p + 1) and,
+//      upstream, sum d_probs . s -- together they give G = sum g s of the epilogue without a pass per term;
+//   4. sample: inverse-CDF scan over 32-column chunks (warp inclusive scan, running total carried across chunks);
+//      train: d(logits) = s (g - G), written 8 columns (16 bytes) per lane and part.
+// The arithmetic is that of epilogue_head_sample / epilogue_head_train (mlp_tcgen05.cu) but for the order of the sums:
+// the sampler's running clamped mass is a chunked warp scan rather than one sequential sum, so a u within a few ulps of a
+// bucket edge may select the neighbouring action.  The narrow and the wide path never serve the same action count.
+// HBM bytes per row: train 2 * z_parts * A in, 2 * dz_parts * dz_cols out, 12 B of scalars; sample 2 * z_parts * A in
+// (+ 4 A of probs_out), 12-16 B out.
+constexpr int WD_WARPS = 4;          // rows in flight per block (shared memory: 4 * pad8(A) floats)
+constexpr int WD_MIN = 257, WD_MAX = 4096;
+
+__device__ __forceinline__ float clamp_p(float s) { return fminf(fmaxf(s, 1e-11f), 1.0f); }     // :54, :74
+
+template <bool TRAIN, bool UPSTREAM = false>
+__global__ void __launch_bounds__(WD_WARPS * 32)
+head_discrete_kernel(ZView z, int64_t M, int A, const float* __restrict__ actions, const float* __restrict__ old_logp,
+                     const float* __restrict__ adv, float inv_batch, float clip, float ent_coef, DzView dz, int dz_cols,
+                     float* __restrict__ logp_out, float* __restrict__ metrics, uint64_t seed, uint64_t offset,
+                     int deterministic, const float* __restrict__ u_inject, float* __restrict__ actions_out,
+                     int64_t* __restrict__ actions_i64_out, float* __restrict__ probs_out,
+                     const float* __restrict__ up_logp, const float* __restrict__ up_ent,
+                     const float* __restrict__ up_probs) {
+    extern __shared__ float4 s_dyn[];
+    __shared__ float s_red[WD_WARPS][5];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int A8 = (A + 7) & ~7;
+    float* e = reinterpret_cast<float*>(s_dyn) + (size_t)warp * A8;
+    float m_ent = 0.f, m_kl = 0.f, m_clip = 0.f, m_surr = 0.f, m_rows = 0.f;
+    for (int64_t row = (int64_t)blockIdx.x * WD_WARPS + warp; row < M; row += (int64_t)gridDim.x * WD_WARPS) {
+        // pass 1: logits -> shared memory, max and first argmax
+        float mx = -INFINITY;
+        int amax = 0;
+        const uint16_t* zr = z.p + row * z.ld;
+#pragma unroll 2
+        for (int c0 = lane * 8; c0 < A; c0 += 256) {
+            float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+            uint4 wq[3];                                   // every part's load in flight before the first add
+#pragma unroll
+            for (int q = 0; q < 3; ++q)
+                if (q < z.parts) wq[q] = __ldg(reinterpret_cast<const uint4*>(zr + q * z.pstride + c0));
+#pragma unroll
+            for (int q = 2; q >= 0; --q) {                 // the summation order of zload
+                if (q >= z.parts) continue;
+                const uint32_t ww[4] = {wq[q].x, wq[q].y, wq[q].z, wq[q].w};
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    v[2 * j] += __uint_as_float(ww[j] << 16);
+                    v[2 * j + 1] += __uint_as_float(ww[j] & 0xFFFF0000u);
+                }
+            }
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                if (c0 + j < A && v[j] > mx) {
+                    mx = v[j];
+                    amax = c0 + j;
+                }
+            }
+            reinterpret_cast<float4*>(e + c0)[0] = make_float4(v[0], v[1], v[2], v[3]);
+            reinterpret_cast<float4*>(e + c0)[1] = make_float4(v[4], v[5], v[6], v[7]);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const float omx = __shfl_xor_sync(0xffffffffu, mx, o);
+            const int oa = __shfl_xor_sync(0xffffffffu, amax, o);
+            if (omx > mx || (omx == mx && oa < amax)) {
+                mx = omx;
+                amax = oa;
+            }
+        }
+        __syncwarp();
+        // pass 2: e = exp(z - max), S
+        float S = 0.f;
+        for (int c = lane; c < A; c += 32) {
+            const float x = __expf(e[c] - mx);
+            e[c] = x;
+            S += x;
+        }
+        S = warp_sum(S);
+        __syncwarp();
+        const float invS = __frcp_rn(S);   // == 1.0f / S (both round the reciprocal to nearest), no division slow path
+
+        if (!TRAIN) {
+            // DiscreteFF.get_action / get_output (discrete_policy.py:35-62)
+            float P = 0.f;
+            if (probs_out != nullptr || !deterministic) {
+                for (int c = lane; c < A; c += 32) {
+                    const float s = e[c] * invS;
+                    if (probs_out != nullptr) probs_out[row * A + c] = s;                // unclamped softmax (:35-42)
+                    P += clamp_p(s);               // total clamped mass: torch.multinomial normalises what it is given
+                }
+                P = warp_sum(P);
+            }
+            int act;
+            float pa;
+            if (deterministic) {
+                act = amax;
+                pa = clamp_p(invS);                // exp(0) / S
+            } else {
+                float u;
+                if (u_inject != nullptr) {
+                    u = __ldg(u_inject + row);
+                } else {
+                    const uint64_t ctr = offset + (uint64_t)row;
+                    const uint4 r = philox4x32_10(make_uint4((uint32_t)ctr, (uint32_t)(ctr >> 32), 0u, 0u),
+                                                  make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+                    u = u01(r.x);
+                }
+                const float thr = u * P;
+                act = A - 1;                       // no running mass above thr (rounding): the last action
+                pa = 0.f;
+                float carry = 0.f;
+                for (int c0 = 0; c0 < A; c0 += 32) {
+                    const int col = c0 + lane;
+                    const float pj = col < A ? clamp_p(e[col] * invS) : 0.f;
+                    float run = pj;
+#pragma unroll
+                    for (int o = 1; o < 32; o <<= 1) {
+                        const float t = __shfl_up_sync(0xffffffffu, run, o);
+                        if (lane >= o) run += t;
+                    }
+                    run += carry;
+                    const unsigned hit = __ballot_sync(0xffffffffu, col < A && run > thr);
+                    if (hit != 0u) {
+                        const int l = __ffs(hit) - 1;
+                        act = c0 + l;
+                        pa = __shfl_sync(0xffffffffu, pj, l);
+                        break;
+                    }
+                    carry = __shfl_sync(0xffffffffu, run, 31);
+                    pa = __shfl_sync(0xffffffffu, pj, (A - 1) & 31);     // used only after the last chunk
+                }
+            }
+            if (lane == 0) {
+                if (actions_out != nullptr) actions_out[row] = (float)act;       // batched_agent_manager.py:204
+                if (actions_i64_out != nullptr) actions_i64_out[row] = (int64_t)act;
+                if (logp_out != nullptr) logp_out[row] = logf(pa);               // :60
+            }
+            __syncwarp();
+            continue;
+        }
+
+        // get_backprop_data (:64-80) + the PPO block (ppo_learner.py:153-177) or upstream gradients, backward into z
+        int a = 0;
+        float old_lp = 0.f, advv = 0.f, up_lp = 0.f;
+        if (UPSTREAM) {
+            if (up_logp != nullptr) {
+                a = min(max((int)__ldg(actions + row), 0), A - 1);
+                up_lp = __ldg(up_logp + row);
+            }
+        } else {
+            a = min(max((int)__ldg(actions + row), 0), A - 1);                   // acts.long(), :71
+            old_lp = __ldg(old_logp + row);
+            advv = __ldg(adv + row);
+        }
+        const float* dpr = (UPSTREAM && up_probs != nullptr) ? up_probs + row * A : nullptr;
+        // pass 3: entropy, T1 = sum_{mask} s (log p + 1), T2 = sum d_probs . s
+        float H = 0.f, T1 = 0.f, T2 = 0.f;
+        for (int c = lane; c < A; c += 32) {
+            const float s = e[c] * invS;
+            const float pj = clamp_p(s);
+            const float lg = __logf(pj);
+            if (!UPSTREAM) H -= pj * lg;                                          // :78
+            if (s >= 1e-11f && s <= 1.0f) T1 += s * (lg + 1.0f);                  // clamp mask
+            if (UPSTREAM && dpr != nullptr) T2 += __ldg(dpr + c) * s;
+        }
+        if (!UPSTREAM) H = warp_sum(H);
+        T1 = warp_sum(T1);
+        if (UPSTREAM) T2 = warp_sum(T2);
+        const float s_a = e[a] * invS;
+        const float p_a = clamp_p(s_a);
+        const float logp = logf(p_a);                                             // :76-77
+        float ga, cw;
+        PpoRow r = {0.f, 0.f, 0.f, 0.f};
+        if (UPSTREAM) {
+            ga = up_lp / p_a;                                                     // dL/dp_a = d_logp / p_a
+            cw = up_ent != nullptr ? -__ldg(up_ent) / (float)M : 0.f;            // dL/dp_j = -(d_ent/M)(log p_j + 1)
+        } else {
+            r = ppo_row(logp, old_lp, advv, clip, inv_batch);
+            ga = r.d_logp / p_a;
+            cw = ent_coef * inv_batch;
+        }
+        // G = sum_j g_j s_j with g_j = mask_j (cw (log p_j + 1) + [j == a] ga) + d_probs_j
+        const float G = cw * T1 + ((s_a >= 1e-11f && s_a <= 1.0f) ? ga * s_a : 0.f) + T2;
+        // pass 4: dz_j = s_j (g_j - G) -> dz parts (columns A..dz_cols zero)
+        uint16_t* dr = dz.p + row * dz.ld;
+        for (int c0 = lane * 8; c0 < dz_cols; c0 += 256) {
+            float o[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+            if (c0 < A) {
+                const float4 e0 = reinterpret_cast<const float4*>(e + c0)[0];
+                const float4 e1 = reinterpret_cast<const float4*>(e + c0)[1];
+                const float ev[8] = {e0.x, e0.y, e0.z, e0.w, e1.x, e1.y, e1.z, e1.w};
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const int col = c0 + j;
+                    if (col < A) {
+                        const float s = ev[j] * invS;
+                        const float pj = clamp_p(s);
+                        float g = cw * (__logf(pj) + 1.0f) + (col == a ? ga : 0.f);
+                        g = (s >= 1e-11f && s <= 1.0f) ? g : 0.f;
+                        if (UPSTREAM && dpr != nullptr) g += __ldg(dpr + col);
+                        o[j] = s * (g - G);
+                    }
+                }
+            }
+            for (int q = 0; q < dz.parts; ++q) {
+                uint4 w;
+                w.x = pack_bf16x2(o[0], o[1]);
+                w.y = pack_bf16x2(o[2], o[3]);
+                w.z = pack_bf16x2(o[4], o[5]);
+                w.w = pack_bf16x2(o[6], o[7]);
+                *reinterpret_cast<uint4*>(dr + q * dz.pstride + c0) = w;
+                const uint32_t ww[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    o[2 * j] -= __uint_as_float(ww[j] << 16);
+                    o[2 * j + 1] -= __uint_as_float(ww[j] & 0xFFFF0000u);
+                }
+            }
+        }
+        if (!UPSTREAM) {
+            if (lane == 0 && logp_out != nullptr) logp_out[row] = logp;
+            m_ent += H;
+            m_kl += r.kl;
+            m_clip += r.clipc;
+            m_surr += r.surr;
+            m_rows += 1.f;
+        }
+        __syncwarp();                      // every lane is done with e before the next row overwrites it
+    }
+    if (TRAIN && !UPSTREAM) {
+        // metrics as the other heads accumulate them, one atomic per block and quantity
+        if (lane == 0) {
+            s_red[warp][0] = m_ent;
+            s_red[warp][1] = m_kl;
+            s_red[warp][2] = m_clip;
+            s_red[warp][3] = m_surr;
+            s_red[warp][4] = m_rows;
+        }
+        __syncthreads();
+        if (threadIdx.x < 5 && metrics != nullptr) {
+            float t = 0.f, rows = 0.f;
+            for (int w = 0; w < WD_WARPS; ++w) {
+                t += s_red[w][threadIdx.x];
+                rows += s_red[w][4];
+            }
+            if (rows > 0.f) atomicAdd(metrics + threadIdx.x, t);
+        }
+    }
+}
+
+template <bool TRAIN, bool UPSTREAM>
+int launch_discrete(cudaStream_t s, const ZView& zv, int64_t M, int A, const float* actions, const float* old_logp,
+                    const float* adv, float inv_batch, float clip, float ent_coef, const DzView& dv, int dz_cols,
+                    float* logp_out, float* metrics, uint64_t seed, uint64_t offset, int deterministic,
+                    const float* u_inject, float* actions_out, int64_t* actions_i64_out, float* probs_out,
+                    const float* up_logp, const float* up_ent, const float* up_probs) {
+    auto kfn = head_discrete_kernel<TRAIN, UPSTREAM>;
+    static bool configured = false;
+    if (!configured) {
+        RLPPO_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)(WD_WARPS * WD_MAX * sizeof(float))));
+        configured = true;
+    }
+    const size_t smem = (size_t)WD_WARPS * ((A + 7) & ~7) * sizeof(float);
+    static size_t cached_smem = 0;      // resident blocks per SM for the last shared-memory size asked about
+    static int per_sm = 0;
+    if (smem != cached_smem) {
+        RLPPO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kfn, WD_WARPS * 32, smem));
+        if (per_sm < 1) per_sm = 1;
+        cached_smem = smem;
+    }
+    const int64_t need = (M + WD_WARPS - 1) / WD_WARPS;
+    const int64_t resident = (int64_t)per_sm * num_sms();
+    const unsigned grid = (unsigned)(need < resident ? need : resident);
+    kfn<<<grid, WD_WARPS * 32, smem, s>>>(zv, M, A, actions, old_logp, adv, inv_batch, clip, ent_coef, dv, dz_cols,
+                                           logp_out, metrics, seed, offset, deterministic, u_inject, actions_out,
+                                           actions_i64_out, probs_out, up_logp, up_ent, up_probs);
+    RLPPO_LAUNCH_CHECK();
+    return RLPPO_OK;
+}
+
+// z / dz views the 16-byte accesses of head_discrete_kernel can address: aligned base, ld and part stride in whole
+// 8-column groups, each part pad8(A) columns wide
+int check_discrete_views(const uint16_t* z, int64_t ldz, int z_parts, int64_t z_pstride, int64_t M, int A,
+                         const uint16_t* dz, int64_t lddz, int dz_parts, int64_t dz_pstride, int dz_cols) {
+    RLPPO_CHECK_ARG(A >= WD_MIN && A <= WD_MAX, "wide discrete head: n_actions must be in [%d,%d] (got %d)", WD_MIN,
+                    WD_MAX, A);
+    RLPPO_CHECK_ARG(M >= 1, "bad argument");
+    const int A8 = (A + 7) & ~7;
+    RLPPO_CHECK_ARG(z != nullptr && z_parts >= 1 && z_parts <= 3 && (reinterpret_cast<uintptr_t>(z) & 15) == 0 &&
+                        ldz % 8 == 0 && (z_parts == 1 || (z_pstride % 8 == 0 && z_pstride >= A8)) &&
+                        ldz >= (int64_t)(z_parts - 1) * z_pstride + A8,
+                    "bad logits view (16-byte aligned, ld and part stride multiples of 8 covering pad8(n_actions))");
+    if (dz != nullptr) {
+        RLPPO_CHECK_ARG(dz_parts >= 1 && dz_parts <= 3 && dz_cols >= A8 && dz_cols % 8 == 0 &&
+                            (reinterpret_cast<uintptr_t>(dz) & 15) == 0 && lddz % 8 == 0 &&
+                            (dz_parts == 1 || (dz_pstride % 8 == 0 && dz_pstride >= dz_cols)) &&
+                            lddz >= (int64_t)(dz_parts - 1) * dz_pstride + dz_cols,
+                        "bad d(logits) view (16-byte aligned, ld, part stride and columns multiples of 8)");
+    }
+    return RLPPO_OK;
+}
+
 int check_z(const uint16_t* z, int64_t ldz, int parts, int64_t pstride, int cols) {
     RLPPO_CHECK_ARG(z != nullptr && parts >= 1 && parts <= 3 && (parts == 1 || pstride >= cols) &&
                         ldz >= (int64_t)(parts - 1) * pstride + cols, "bad logits view");
@@ -419,5 +733,47 @@ int rlppo_head_continuous_sample(const uint16_t* z, int64_t ldz, int z_parts, in
         deterministic, n_inject, actions_out, ld_aout, nullptr, nullptr, nullptr, nullptr);
     RLPPO_LAUNCH_CHECK();
     return RLPPO_OK;
+}
+
+int rlppo_head_discrete_train(const uint16_t* z, int64_t ldz, int z_parts, int64_t z_pstride, int64_t M, int n_actions,
+                              const float* actions, const float* old_logp, const float* adv, float inv_batch, float clip,
+                              float ent_coef, uint16_t* dz, int64_t lddz, int dz_parts, int64_t dz_pstride, int dz_cols,
+                              float* logp_out, float* metrics, void* stream) {
+    RLPPO_REQUIRE_DEVICE();
+    RLPPO_CHECK_ARG(actions && old_logp && adv && dz, "null pointer");
+    int rc = check_discrete_views(z, ldz, z_parts, z_pstride, M, n_actions, dz, lddz, dz_parts, dz_pstride, dz_cols);
+    if (rc) return rc;
+    return launch_discrete<true, false>(static_cast<cudaStream_t>(stream), ZView{z, ldz, z_parts, z_pstride}, M,
+                                        n_actions, actions, old_logp, adv, inv_batch, clip, ent_coef,
+                                        DzView{dz, lddz, dz_parts, dz_pstride}, dz_cols, logp_out, metrics, 0, 0, 0,
+                                        nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
+}
+
+int rlppo_head_discrete_backward(const uint16_t* z, int64_t ldz, int z_parts, int64_t z_pstride, int64_t M,
+                                 int n_actions, const float* actions, const float* d_logp, const float* d_ent,
+                                 const float* d_probs, uint16_t* dz, int64_t lddz, int dz_parts, int64_t dz_pstride,
+                                 int dz_cols, void* stream) {
+    RLPPO_REQUIRE_DEVICE();
+    RLPPO_CHECK_ARG(dz && (d_logp == nullptr || actions != nullptr), "null pointer");
+    int rc = check_discrete_views(z, ldz, z_parts, z_pstride, M, n_actions, dz, lddz, dz_parts, dz_pstride, dz_cols);
+    if (rc) return rc;
+    return launch_discrete<true, true>(static_cast<cudaStream_t>(stream), ZView{z, ldz, z_parts, z_pstride}, M,
+                                       n_actions, actions, nullptr, nullptr, 0.f, 0.f, 0.f,
+                                       DzView{dz, lddz, dz_parts, dz_pstride}, dz_cols, nullptr, nullptr, 0, 0, 0,
+                                       nullptr, nullptr, nullptr, nullptr, d_logp, d_ent, d_probs);
+}
+
+int rlppo_head_discrete_sample(const uint16_t* z, int64_t ldz, int z_parts, int64_t z_pstride, int64_t M, int n_actions,
+                               const float* u_inject, uint64_t seed, uint64_t offset, int deterministic,
+                               float* actions_out, int64_t* actions_i64_out, float* logp_out, float* probs_out,
+                               void* stream) {
+    RLPPO_REQUIRE_DEVICE();
+    RLPPO_CHECK_ARG(actions_out || actions_i64_out || logp_out || probs_out, "no output");
+    int rc = check_discrete_views(z, ldz, z_parts, z_pstride, M, n_actions, nullptr, 0, 0, 0, 0);
+    if (rc) return rc;
+    return launch_discrete<false, false>(static_cast<cudaStream_t>(stream), ZView{z, ldz, z_parts, z_pstride}, M,
+                                         n_actions, nullptr, nullptr, nullptr, 0.f, 0.f, 0.f, DzView{nullptr, 0, 0, 0},
+                                         0, logp_out, nullptr, seed, offset, deterministic, u_inject, actions_out,
+                                         actions_i64_out, probs_out, nullptr, nullptr, nullptr);
 }
 }

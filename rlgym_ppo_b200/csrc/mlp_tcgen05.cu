@@ -1074,6 +1074,13 @@ wgrad_multi_kernel(const __grid_constant__ WMaps maps, const WMultiParams p) {
 // column sums of a bf16 matrix: db[n] += sum_m dY[m,n]   (bias gradients)
 __global__ void colsum_kernel(const uint16_t* __restrict__ dy, int64_t ld, int64_t M, int N, int n8,
                               float* __restrict__ db, int64_t rows_per_block) {
+    // blockIdx.y: a slice of the columns (a grid of more than one only for N > 2048: a wide policy head's logits)
+    const int slice = (n8 / 8 + gridDim.y - 1) / gridDim.y * 8;
+    const int c0 = blockIdx.y * slice;
+    dy += c0;
+    db += c0;
+    n8 = min(slice, n8 - c0);
+    N = min(n8, N - c0);
     extern __shared__ float s_acc[];  // n8 floats (N rounded up to 8; the padding columns of dY are zero)
     for (int i = threadIdx.x; i < n8; i += blockDim.x) s_acc[i] = 0.f;
     __syncthreads();
@@ -1366,7 +1373,9 @@ int rlppo_linear_wgrad_split(const uint16_t* dy, int64_t lddy, const uint16_t* x
     if (rc) return rc;
     if (db != nullptr) {
         const int n8 = (N + 7) / 8 * 8;
-        RLPPO_CHECK_ARG(n8 <= lddy && n8 / 8 <= 256, "bias-gradient pass needs N padded to 8 within lddy");
+        RLPPO_CHECK_ARG(n8 <= lddy, "bias-gradient pass needs N padded to 8 within lddy");
+        // at most 2048 columns (256 threads of 8) per block: wider dY is split over blockIdx.y
+        const unsigned col_slices = (unsigned)((n8 / 8 + 255) / 256);
         // padded columns of dY are zero by construction, so summing n8 columns is safe; only N are written
         // ~8 blocks per SM: with 512 rows per block a 50 000-row dY gave 98 blocks of 512 dependent 16-byte loads per
         // thread -- 2 TB/s, and at the wide nets (N = 2048) the pass cost 72 % of the weight-gradient GEMM it follows
@@ -1374,12 +1383,13 @@ int rlppo_linear_wgrad_split(const uint16_t* dy, int64_t lddy, const uint16_t* x
         rows_per_block = (rows_per_block + 7) / 8 * 8;
         if (rows_per_block < 32) rows_per_block = 32;
         const unsigned blocks = (unsigned)((M + rows_per_block - 1) / rows_per_block);
+        const int slice = (int)((n8 / 8 + col_slices - 1) / col_slices) * 8;     // as colsum_kernel computes it
         int threads = 256;
-        if (threads < n8 / 8) threads = n8 / 8;
+        if (threads < slice / 8) threads = slice / 8;
         const int dy_parts = sp ? sp->a_parts : 1;
         for (int q = 0; q < dy_parts; ++q) {     // every part of a split dY contributes to the column sums
-            colsum_kernel<<<blocks, threads, n8 * sizeof(float), s>>>(dy + (sp ? q * sp->a_pstride : 0), lddy, M, N, n8, db,
-                                                                      rows_per_block);
+            colsum_kernel<<<dim3(blocks, col_slices), threads, slice * sizeof(float), s>>>(
+                dy + (sp ? q * sp->a_pstride : 0), lddy, M, N, n8, db, rows_per_block);
             RLPPO_LAUNCH_CHECK();
         }
     }

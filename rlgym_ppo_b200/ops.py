@@ -346,6 +346,37 @@ def head_continuous_sample(z, z_parts, z_pstride, M, n_act, var_min, var_max, ac
          work=("byte", M * (4 * n_act * z_parts + 4 * (n_act + 1))))
 
 
+# ---- wide discrete head (257..4096 actions): per-row kernels over the split logits of the last Linear ----------------
+def _discrete_bytes(M, n_actions, z_parts, dz_cols=0, dz_parts=0):
+    """HBM bytes of one pass: the logits once, d(logits) once, the per-row scalars."""
+    return M * (2 * n_actions * z_parts + 2 * dz_cols * dz_parts + 12)
+
+
+def head_discrete_sample(z, z_parts, z_pstride, M, n_actions, u=None, seed=0, offset=0, deterministic=False,
+                         actions_out=None, actions_i64_out=None, logp_out=None, probs_out=None):
+    nbytes = _discrete_bytes(M, n_actions, z_parts) + (4 * M * n_actions if probs_out is not None else 0)
+    call("rlppo_head_discrete_sample", ptr(z), z.stride(0), int(z_parts), int(z_pstride), int(M), int(n_actions), ptr(u),
+         int(seed) & (2 ** 64 - 1), int(offset) & (2 ** 64 - 1), int(bool(deterministic)), ptr(actions_out),
+         ptr(actions_i64_out), ptr(logp_out), ptr(probs_out), stream_ptr(), work=("byte", nbytes))
+
+
+def head_discrete_train(z, z_parts, z_pstride, M, n_actions, actions, old_logp, adv, inv_batch, clip, ent_coef, dz,
+                        dz_parts, dz_pstride, dz_cols, metrics, logp_out=None):
+    call("rlppo_head_discrete_train", ptr(z), z.stride(0), int(z_parts), int(z_pstride), int(M), int(n_actions),
+         ptr(actions), ptr(old_logp), ptr(adv), float(inv_batch), float(clip), float(ent_coef), ptr(dz), dz.stride(0),
+         int(dz_parts), int(dz_pstride), int(dz_cols), ptr(logp_out), ptr(metrics), stream_ptr(),
+         work=("byte", _discrete_bytes(M, n_actions, z_parts, dz_cols, dz_parts)))
+
+
+def head_discrete_backward(z, z_parts, z_pstride, M, n_actions, actions, d_logp, d_ent, d_probs, dz, dz_parts, dz_pstride,
+                           dz_cols):
+    """d_logp f32[M], d_ent f32[1], d_probs f32[M, n_actions]: device tensors or None."""
+    nbytes = _discrete_bytes(M, n_actions, z_parts, dz_cols, dz_parts) + (4 * M * n_actions if d_probs is not None else 0)
+    call("rlppo_head_discrete_backward", ptr(z), z.stride(0), int(z_parts), int(z_pstride), int(M), int(n_actions),
+         ptr(actions), ptr(d_logp), ptr(d_ent), ptr(d_probs), ptr(dz), dz.stride(0), int(dz_parts), int(dz_pstride),
+         int(dz_cols), stream_ptr(), work=("byte", nbytes))
+
+
 # ---- backward of the heads for arbitrary upstream gradients (torch autograd through the modules) ---------------------
 def policy_head_backward(h, wq, bias, n_actions, K, actions, d_logp, d_ent, d_probs, dz, M=None, split=None):
     """d_logp f32[M], d_ent f32[1], d_probs f32[M, n_actions]: device tensors or None."""

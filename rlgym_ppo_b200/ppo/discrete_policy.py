@@ -4,6 +4,10 @@ Same constructor, attributes (`.model`, `.n_actions`, `.device`) and state-dict 
 runs in hand-written sm_100a kernels: bf16 tcgen05 GEMMs with fp32 TMEM accumulation for the Linear/ReLU stack,
 and the softmax -> clamp(1e-11, 1) -> {multinomial sample | log-prob gather + entropy} tail fused into the
 epilogue of the last GEMM (rlppo_policy_head_sample / rlppo_policy_head_train).
+
+Up to 256 actions a row's logits fit the epilogue's tile.  Wider action spaces (257..4096, `wide`) run the last Linear
+on its own (Stack.logits, fp32-exact split logits) followed by the per-row kernels rlppo_head_discrete_{sample,train,
+backward}, with the same arithmetic.
 """
 import numpy as np
 import torch
@@ -12,15 +16,21 @@ import torch.nn as nn
 from .. import ops
 from ._mlp import BF16, Stack, StackFunction, autograd_wanted, build_sequential, grad_f32
 
+EPILOGUE_MAX_ACTIONS = 256     # widest head the fused epilogue of the head GEMM serves
+MAX_ACTIONS = 4096             # widest head the per-row kernels serve
+
 
 class DiscreteFF(nn.Module):
     autograd = False    # True: differentiable get_output / forward / get_backprop_data (_mlp.autograd_wanted)
 
     def __init__(self, input_shape, n_actions, layer_sizes, device, precision=None):
         super().__init__()
+        if int(n_actions) > MAX_ACTIONS:
+            raise ValueError(f"DiscreteFF supports at most {MAX_ACTIONS} actions (got {int(n_actions)})")
         self.device = device
         self.model = build_sequential(input_shape, layer_sizes, n_actions, softmax=True)   # :22-31
         self.n_actions = int(n_actions)
+        self.wide = self.n_actions > EPILOGUE_MAX_ACTIONS
         self._stack = Stack(self.model, device, precision)
         dev = self._stack.device
         # standalone arenas; PPOLearner re-binds both nets into one shared arena
@@ -82,11 +92,41 @@ class DiscreteFF(nn.Module):
             return acts, logp, None
         h = st.forward_hidden(x, n, ws)
         probs = torch.empty((n, self.n_actions), dtype=torch.float32, device=dev) if want_probs else None
-        if n:
+        if n and self.wide:
+            z, parts, ps = st.logits(h, n, ws)
+            ops.head_discrete_sample(z, parts, ps, n, self.n_actions, seed=self._seed, offset=self._offset,
+                                     deterministic=deterministic, actions_i64_out=acts, logp_out=logp, probs_out=probs)
+            self._offset += n
+        elif n:
             st.policy_head_sample(h, n, self.n_actions, seed=self._seed, offset=self._offset,
                                   deterministic=deterministic, actions_i64_out=acts, logp_out=logp, probs_out=probs)
             self._offset += n
         return acts, logp, probs
+
+    # ---- wide heads: last Linear -> per-row kernel -> the head's weight / data gradients ----------------------------
+    def _wide_head_backward(self, h, M, ws, actions, d_logp, d_ent, d_probs, gw, gb):
+        st = self._stack
+        z, parts, ps = st.logits(h, M, ws)
+        dz, dparts, dps, dcols = st.dz_view(ws)
+        ops.head_discrete_backward(z, parts, ps, M, self.n_actions, actions, d_logp, d_ent, d_probs, dz, dparts, dps,
+                                   dcols)
+        return st.head_backward(h, M, ws, gw, gb)
+
+    def _head_backward(self, h, M, ws, actions, d_logp, d_ent, d_probs, gw, gb):
+        """Head backward for upstream gradients of (log-prob, mean entropy, probabilities).  Returns dL/dH_last."""
+        if self.wide:
+            return self._wide_head_backward(h, M, ws, actions, d_logp, d_ent, d_probs, gw, gb)
+        return self._stack.policy_head_backward(h, M, ws, self.n_actions, actions, d_logp, d_ent, d_probs, gw, gb)
+
+    def train_head(self, h, M, ws, actions, old_logp, adv, inv_b, clip, ent_coef, metrics, logp_out=None):
+        """PPOLearner._train_chunk for wide heads: logits, the PPO block and its backward into d(logits), then the head's
+        weight / bias gradients.  Returns dL/dH_last."""
+        st = self._stack
+        z, parts, ps = st.logits(h, M, ws)
+        dz, dparts, dps, dcols = st.dz_view(ws)
+        ops.head_discrete_train(z, parts, ps, M, self.n_actions, actions, old_logp, adv, inv_b, clip, ent_coef, dz, dparts,
+                                dps, dcols, metrics, logp_out=logp_out)
+        return st.head_backward(h, M, ws)
 
     # ---- reference surface -------------------------------------------------------------------------------------
     def get_output(self, obs):
@@ -99,8 +139,7 @@ class DiscreteFF(nn.Module):
                 return probs, probs.shape[0], None
 
             def head_backward(h, M, ws, grads, gw, gb, saved):
-                return self._stack.policy_head_backward(h, M, ws, self.n_actions, None, None, None,
-                                                        grad_f32(grads[0], M, self.n_actions), gw, gb)
+                return self._head_backward(h, M, ws, None, None, None, grad_f32(grads[0], M, self.n_actions), gw, gb)
             probs = StackFunction.apply(self._stack, run, head_backward, *self.parameters())
         else:
             _, _, probs = self._head_sample(obs, True, True)
@@ -140,8 +179,7 @@ class DiscreteFF(nn.Module):
                 return (logp, ent), logp.shape[0], acts_f.clone()
 
             def head_backward(h, M, ws, grads, gw, gb, acts_f):
-                return self._stack.policy_head_backward(h, M, ws, self.n_actions, acts_f, grad_f32(grads[0], M),
-                                                        grad_f32(grads[1], 1), None, gw, gb)
+                return self._head_backward(h, M, ws, acts_f, grad_f32(grads[0], M), grad_f32(grads[1], 1), None, gw, gb)
             return StackFunction.apply(self._stack, run, head_backward, *self.parameters())
         logp, ent, _ = self._backprop_forward(obs, acts)
         return logp, ent
@@ -157,6 +195,12 @@ class DiscreteFF(nn.Module):
         zeros = torch.zeros(n, dtype=torch.float32, device=dev)
         logp = torch.empty(n, dtype=torch.float32, device=dev)
         metrics = torch.zeros(8, dtype=torch.float32, device=dev)
+        if self.wide:
+            z, parts, ps = st.logits(h, n, ws)
+            dz, dparts, dps, dcols = st.dz_view(ws)
+            ops.head_discrete_train(z, parts, ps, n, self.n_actions, acts_f, zeros, zeros, 0.0, 0.2, 0.0, dz, dparts, dps,
+                                    dcols, metrics, logp_out=logp)
+            return logp.view(-1, 1), metrics[0] / metrics[4], acts_f
         hl = st.hidden[-1]
         sp = ops.make_split(3, 3, 3, 2, ops.pad64(hl), ops.pad64(hl), ops.pad64(st.out_dim)) if st.exact else None
         ops.policy_head_train(h, st.wq[-1], st.b[-1], self.n_actions, hl, acts_f, zeros, zeros, 0.0, 0.2,

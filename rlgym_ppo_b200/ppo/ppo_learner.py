@@ -332,8 +332,9 @@ class PPOLearner(object):
                 n += 1
                 continue
             h = st.forward_hidden(x, M, ws)
-            if is_policy and self.policy_type != 0:
-                # MultiDiscrete / Continuous: last Linear -> per-row head kernel -> head wgrad / dgrad
+            if is_policy and (self.policy_type != 0 or net.wide):
+                # MultiDiscrete / Continuous / Discrete above 256 actions: last Linear -> per-row head kernel -> head
+                # wgrad, colsum (per dz part), dgrad
                 dh = net.train_head(h, M, ws, mb["actions"], mb["old_logp"], mb["adv"], inv_b, float(self.clip_range),
                                     float(self.ent_coef), metrics)
                 n += 5 + (1 if st.exact else 0)
