@@ -33,6 +33,10 @@ extern "C" {
 #define RLPPO_ERR_WORKSPACE (-4)
 
 /* ---- library ------------------------------------------------------------------------------------ */
+/* 101: the layer-wise GEMM, policy-head and value-head entry points and rlppo_rows_to_bf16 have one form each, under the
+ * plain name and with the argument list of the split-operand / standardising form it absorbed (those names are gone).
+ * A binding written against 100 would pass the old, shorter argument lists to the same names without any error: check
+ * this number before binding. */
 int rlppo_version(void);
 const char* rlppo_last_error(void);
 /* 0 if the current CUDA device can run the sm_100a kernels; RLPPO_ERR_DEVICE otherwise. */
@@ -123,41 +127,75 @@ int rlppo_host_permutation(uint32_t* h_key, int32_t* h_pos, int64_t n, int64_t* 
 
 /* ---- operand preparation ------------------------------------------------------------------------- */
 /* f32 [n_rows, width] (ld src_ld) -> bf16 [n_rows, dst_ld], zero padded; used for the value-net input
- * [states ; next_states[-1]] (learner.py:347-349) and policy inference obs. */
-int rlppo_rows_to_bf16(const float* src, int64_t src_ld, int64_t n_rows, int width, uint16_t* dst,
-                       int64_t dst_ld, void* stream);
-/* Same with obs standardisation fused: clip((x-mean)/std, -5, 5) (batched_agent_manager.py:303-315).
- * dst_f32 (optional, ld dst_f32_ld): the standardised rows in f32 as well -- what the trajectory stores. */
-int rlppo_rows_standardize_to_bf16(const float* src, int64_t src_ld, int64_t n_rows, int width,
-                                   const float* mean, const float* std, float clip, uint16_t* dst,
-                                   int64_t dst_ld, float* dst_f32, int64_t dst_f32_ld, void* stream);
+ * [states ; next_states[-1]] (learner.py:347-349) and policy inference obs.
+ *   mean, std f32[width] (both or neither): standardise first, clip((x-mean)/std, -clip, clip)
+ *     (batched_agent_manager.py:303-315, clip = 5); NULL: the rows as they are.
+ *   dst_f32 (optional, ld dst_f32_ld; needs mean): the standardised rows in f32 as well -- what the trajectory stores.
+ *   Exactly one of mean / std NULL, or dst_f32 without mean: RLPPO_ERR_ARG. */
+int rlppo_rows_to_bf16(const float* src, int64_t src_ld, int64_t n_rows, int width, const float* mean,
+                       const float* std, float clip, uint16_t* dst, int64_t dst_ld, float* dst_f32,
+                       int64_t dst_f32_ld, void* stream);
 /* fp32 master weight W [out,in] (torch nn.Linear layout) -> bf16 W [out_pad, in_pad] (K-major operand of
  * the forward GEMM) and, if wt != NULL, bf16 W^T [in_pad, out_pad] (operand of the dgrad GEMM). */
 int rlppo_weight_to_bf16(const float* w, int out_f, int in_f, uint16_t* wq, int64_t wq_ld, int out_pad,
                          uint16_t* wt, int64_t wt_ld, int in_pad, void* stream);
+
+/* ---- precision mode "fp32": split bf16 operands on the same tcgen05 kernels ------------------------------
+ * The reference computes its Linear layers in fp32 (torch CPU/GPU SGEMM, discrete_policy.py:22-31,
+ * value_estimator.py:19-28).  With plain bf16 operands the forward pre-activations carry ~1e-3 relative error, which
+ * flips ReLU masks of near-zero units and moves per-tensor gradients by several per cent -- outside the 1e-3 parity bar
+ * (profiles/r02_precision_study.md).  In this mode every f32 matrix is stored as `parts` bf16 matrices side by side
+ * in one buffer (value = part0 + part1 + part2; part q in columns [q*pstride, q*pstride + cols), pstride a multiple of
+ * 64 columns, padding zero) and a GEMM accumulates the products part_i(A) x part_j(B) for i + j < order into the same
+ * fp32 TMEM accumulator, smallest terms first:
+ *   forward / heads: 3 x 3 parts, order 3 -> 6 products, ~2^-24 per product (fp32-equivalent pre-activations);
+ *   dgrad / wgrad:   2 x 2 parts, order 2 -> 3 products, ~2^-16 (no branch points in the backward: linear errors only).
+ * The GEMM and policy-head entry points below take the split descriptor `sp`: they run a longer k loop (a "k schedule"
+ * of part pairs) and epilogues that write their f32 result as out_parts bf16 parts.  a = the row operand (x, dy, h),
+ * b = the weight operand (w, wt; for wgrad: a = dy, b = x).  sp == NULL means plain bf16 operands. */
+typedef struct rlppo_split {
+    int32_t a_parts;        /* parts of the first (row) operand, 1..3 */
+    int32_t b_parts;        /* parts of the second (weight) operand, 1..3 */
+    int32_t order;          /* products kept: i + j < order */
+    int32_t out_parts;      /* parts the result is written as, 1..3 */
+    int64_t a_pstride;      /* column offset between parts of the first operand (elements) */
+    int64_t b_pstride;      /* ... of the second operand */
+    int64_t out_pstride;    /* ... of the output */
+} rlppo_split;
+/* f32 rows -> parts (optionally standardised first, as rlppo_rows_to_bf16; mean/std NULL: plain). */
+int rlppo_rows_split_bf16(const float* src, int64_t src_ld, int64_t n_rows, int width, const float* mean,
+                          const float* std, float clip, uint16_t* dst, int64_t dst_ld, int parts, int64_t pstride,
+                          void* stream);
+/* fp32 master weight W [out,in] -> split W [out_rows, q_parts*q_pstride] (forward operand) and/or split
+ * W^T [in_rows, t_parts*t_pstride] (dgrad operand); either output may be NULL.  Padding rows/columns are zeroed. */
+int rlppo_weight_split_bf16(const float* w, int out_f, int in_f, uint16_t* wq, int64_t wq_ld, int q_parts,
+                            int64_t q_pstride, int out_rows, uint16_t* wt, int64_t wt_ld, int t_parts,
+                            int64_t t_pstride, int in_rows, void* stream);
 
 /* ---- (a-3, d-2) MLP on tcgen05 tensor cores: discrete_policy.py:22-42, value_estimator.py:19-36 ----
  * All GEMMs: bf16 operands staged by TMA (128B swizzle), fp32 accumulation in TMEM, one elected thread
  * issuing tcgen05.mma, epilogue warps reading TMEM with tcgen05.ld.  M = rows (timesteps).
  *
  * rlppo_linear_fwd:  Y[M,N] = act(X[M,K] * W[N,K]^T + bias)   (nn.Linear + ReLU), Y bf16.
- *   x ld = ldx (>= K, multiple of 8), w bf16 [>=N rows, ldw], bias f32[N] or NULL, relu 0/1. */
-int rlppo_linear_fwd(const uint16_t* x, int64_t ldx, const uint16_t* w, int64_t ldw, const float* bias,
-                     uint16_t* y, int64_t ldy, int64_t M, int N, int K, int relu, void* stream);
+ *   x ld = ldx (>= K, multiple of 8), w bf16 [>=N rows, ldw], bias f32[N] or NULL, relu 0/1.
+ *   bias_n: entries of `bias` (0 = N): lets a Linear whose width is not a multiple of 8 (21 logits, 2n outputs) run with
+ *   N padded to 8 without reading past its bias vector. */
+int rlppo_linear_fwd(const uint16_t* x, int64_t ldx, const uint16_t* w, int64_t ldw, const float* bias, int bias_n,
+                     uint16_t* y, int64_t ldy, int64_t M, int N, int K, int relu, const rlppo_split* sp, void* stream);
 /* rlppo_linear_dgrad: dX[M,K] = (dY[M,N] * W[N,K]) (.) (Hprev > 0); wt = bf16 W^T [K, ldwt>=N].
- *   hprev = the ReLU output that was this layer's input (bf16 [M,ldh]) or NULL (no mask). */
-int rlppo_linear_dgrad(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt,
-                       const uint16_t* hprev, int64_t ldh, uint16_t* dx, int64_t lddx, int64_t M, int N,
-                       int K, void* stream);
-/* The same, and db_below f32[K] += column sums of the stored dX (= the bias gradient of the layer that produced
- * Hprev, ppo_learner.py:179-180 autograd): saves that layer's separate column-sum pass over dX. */
-int rlppo_linear_dgrad_db(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt,
-                          const uint16_t* hprev, int64_t ldh, uint16_t* dx, int64_t lddx, float* db_below,
-                          int64_t M, int N, int K, void* stream);
+ *   hprev = the ReLU output that was this layer's input (bf16 [M,ldh]) or NULL (no mask).
+ *   db_below (optional f32[K]) += column sums of the stored dX (= the bias gradient of the layer that produced Hprev,
+ *   ppo_learner.py:179-180 autograd): saves that layer's separate column-sum pass over dX.
+ *   Split operands: the ReLU mask is read from part 0 of hprev (x > 0 <=> bf16(x) > 0); db_below sums the un-split f32
+ *   values. */
+int rlppo_linear_dgrad(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt, const uint16_t* hprev,
+                       int64_t ldh, uint16_t* dx, int64_t lddx, float* db_below, int64_t M, int N, int K,
+                       const rlppo_split* sp, void* stream);
 /* rlppo_linear_wgrad: dW[N,K] += dY[M,N]^T * X[M,K]  (fp32, torch [out,in] layout with ld = lddw) and
- *   db[N] += column sums of dY (if db != NULL).  Split over M across the SMs; fp32 atomics. */
-int rlppo_linear_wgrad(const uint16_t* dy, int64_t lddy, const uint16_t* x, int64_t ldx, float* dw,
-                       int64_t lddw, float* db, int64_t M, int N, int K, void* stream);
+ *   db[N] += column sums of dY (if db != NULL; over all parts of a split dY).  Split over M across the SMs; fp32
+ *   atomics. */
+int rlppo_linear_wgrad(const uint16_t* dy, int64_t lddy, const uint16_t* x, int64_t ldx, float* dw, int64_t lddw,
+                       float* db, int64_t M, int N, int K, const rlppo_split* sp, void* stream);
 
 /* All weight gradients of an optimiser step in ONE persistent launch (<= 8 layers): for every item
  * dW[N,K] += dY[M,N]^T * X[M,K] as rlppo_linear_wgrad, but dY is read once per 256 k (not once per 128), row
@@ -181,11 +219,13 @@ int rlppo_wgrad_multi(const rlppo_wgrad_item* h_items, int n_items, void* stream
  *   actions_out f32[M] (the manager casts actions to f32, batched_agent_manager.py:204) and/or
  *   actions_i64_out int64[M]; logp_out f32[M]; probs_out optional f32[M, n_actions] (get_output).
  *   deterministic != 0: per-row argmax, logp of it (the reference's deterministic branch returns one
- *   global argmax, discrete_policy.py:56-57; the per-row form is what its batch-of-1 use means). */
+ *   global argmax, discrete_policy.py:56-57; the per-row form is what its batch-of-1 use means).
+ *   sp: split operands of the head GEMM, or NULL. */
 int rlppo_policy_head_sample(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw,
                              const float* bias, int64_t M, int n_actions, int K, const float* u_inject,
                              uint64_t seed, uint64_t offset, int deterministic, float* actions_out,
-                             int64_t* actions_i64_out, float* logp_out, float* probs_out, void* stream);
+                             int64_t* actions_i64_out, float* logp_out, float* probs_out, const rlppo_split* sp,
+                             void* stream);
 
 /* Policy head, training (DiscreteFF.get_backprop_data discrete_policy.py:64-80 + ppo_learner.py:153-177
  * + the analytic backward of SURVEY.md A.3), fused into the head GEMM's epilogue:
@@ -193,84 +233,29 @@ int rlppo_policy_head_sample(const uint16_t* h, int64_t ldh, const uint16_t* w, 
  *   loss terms; dz[M, lddz] (bf16) = d(ppo_loss)/dz with weight inv_batch = 1/batch_size;
  *   metrics f32[8] accumulated with atomics: [0] sum entropy, [1] sum kl, [2] sum clipped-count,
  *   [3] sum min(ratio*A, clip(ratio)*A), [4] rows processed; [5..7] reserved.
- *   logp_out optional f32[M]. */
+ *   logp_out optional f32[M].
+ *   sp: split operands, or NULL; d(logits) is then written as sp->out_parts parts of out_pstride columns each
+ *   (lddz >= out_parts * out_pstride). */
 int rlppo_policy_head_train(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw,
                             const float* bias, int64_t M, int n_actions, int K, const float* actions,
                             const float* old_logp, const float* adv, float inv_batch, float clip,
                             float ent_coef, uint16_t* dz, int64_t lddz, float* logp_out, float* metrics,
-                            void* stream);
+                            const rlppo_split* sp, void* stream);
 
 /* Value head (ValueEstimator last Linear(.,1), value_estimator.py:27; MSELoss ppo_learner.py:176),
  * fused SIMT pass over the last hidden activation H[M,K] (bf16):
  *   v = H*w + b  -> values_out f32[M] (if non-NULL).
  *   if targets != NULL: dv = 2*inv_batch*(v - target); dH[M,lddh] (bf16) = dv * w (.) (H > 0);
- *   dw[K] += sum_m dv*H;  db[1] += sum dv;  metrics[5] += sum (v-target)^2, metrics[6] += rows. */
+ *   dw[K] += sum_m dv*H;  db[1] += sum dv;  metrics[5] += sum (v-target)^2, metrics[6] += rows.
+ *   H is given as h_parts split parts h_pstride columns apart and dH written as dh_parts parts dh_pstride apart
+ *   (1..3 parts each, strides multiples of 8 covering K; plain bf16: 1, 0, 1, 0). */
 int rlppo_value_head(const uint16_t* h, int64_t ldh, const float* w, const float* bias, int64_t M, int K,
                      float* values_out, const float* targets, float inv_batch, uint16_t* dh, int64_t lddh,
-                     float* dw, float* db, float* metrics, void* stream);
-
-/* ---- precision mode "fp32": split bf16 operands on the same tcgen05 kernels ------------------------------
- * The reference computes its Linear layers in fp32 (torch CPU/GPU SGEMM, discrete_policy.py:22-31,
- * value_estimator.py:19-28).  With plain bf16 operands the forward pre-activations carry ~1e-3 relative error, which
- * flips ReLU masks of near-zero units and moves per-tensor gradients by several per cent -- outside the 1e-3 parity bar
- * (profiles/r02_precision_study.md).  In this mode every f32 matrix is stored as `parts` bf16 matrices side by side
- * in one buffer (value = part0 + part1 + part2; part q in columns [q*pstride, q*pstride + cols), pstride a multiple of
- * 64 columns, padding zero) and a GEMM accumulates the products part_i(A) x part_j(B) for i + j < order into the same
- * fp32 TMEM accumulator, smallest terms first:
- *   forward / heads: 3 x 3 parts, order 3 -> 6 products, ~2^-24 per product (fp32-equivalent pre-activations);
- *   dgrad / wgrad:   2 x 2 parts, order 2 -> 3 products, ~2^-16 (no branch points in the backward: linear errors only).
- * The kernels are the ones above with a longer k loop (a "k schedule" of part pairs) and epilogues that write their
- * f32 result as out_parts bf16 parts.  sp == NULL is the plain bf16 entry point. */
-typedef struct rlppo_split {
-    int32_t a_parts;        /* parts of the first (row) operand, 1..3 */
-    int32_t b_parts;        /* parts of the second (weight) operand, 1..3 */
-    int32_t order;          /* products kept: i + j < order */
-    int32_t out_parts;      /* parts the result is written as, 1..3 */
-    int64_t a_pstride;      /* column offset between parts of the first operand (elements) */
-    int64_t b_pstride;      /* ... of the second operand */
-    int64_t out_pstride;    /* ... of the output */
-} rlppo_split;
-/* f32 rows -> parts (optionally standardised first, as rlppo_rows_standardize_to_bf16; mean/std NULL: plain). */
-int rlppo_rows_split_bf16(const float* src, int64_t src_ld, int64_t n_rows, int width, const float* mean,
-                          const float* std, float clip, uint16_t* dst, int64_t dst_ld, int parts, int64_t pstride,
-                          void* stream);
-/* fp32 master weight W [out,in] -> split W [out_rows, q_parts*q_pstride] (forward operand) and/or split
- * W^T [in_rows, t_parts*t_pstride] (dgrad operand); either output may be NULL.  Padding rows/columns are zeroed. */
-int rlppo_weight_split_bf16(const float* w, int out_f, int in_f, uint16_t* wq, int64_t wq_ld, int q_parts,
-                            int64_t q_pstride, int out_rows, uint16_t* wt, int64_t wt_ld, int t_parts,
-                            int64_t t_pstride, int in_rows, void* stream);
-/* rlppo_linear_fwd / _dgrad(_db) / _wgrad / heads over split operands.  a = the row operand (x, dy, h), b = the weight
- * operand (w, wt; for wgrad: a = dy, b = x).  The dgrad ReLU mask is read from part 0 of hprev (x > 0 <=> bf16(x) > 0);
- * db_below / db sums take the un-split f32 values / all parts. */
-/* bias_n: entries of `bias` (0 = N): lets a Linear whose width is not a multiple of 8 (21 logits, 2n outputs) run with N
- * padded to 8 without reading past its bias vector. */
-int rlppo_linear_fwd_split(const uint16_t* x, int64_t ldx, const uint16_t* w, int64_t ldw, const float* bias,
-                           int bias_n, uint16_t* y, int64_t ldy, int64_t M, int N, int K, int relu,
-                           const rlppo_split* sp, void* stream);
-int rlppo_linear_dgrad_split(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt,
-                             const uint16_t* hprev, int64_t ldh, uint16_t* dx, int64_t lddx, float* db_below,
-                             int64_t M, int N, int K, const rlppo_split* sp, void* stream);
-int rlppo_linear_wgrad_split(const uint16_t* dy, int64_t lddy, const uint16_t* x, int64_t ldx, float* dw,
-                             int64_t lddw, float* db, int64_t M, int N, int K, const rlppo_split* sp, void* stream);
-int rlppo_policy_head_sample_split(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw,
-                                   const float* bias, int64_t M, int n_actions, int K, const float* u_inject,
-                                   uint64_t seed, uint64_t offset, int deterministic, float* actions_out,
-                                   int64_t* actions_i64_out, float* logp_out, float* probs_out,
-                                   const rlppo_split* sp, void* stream);
-/* d(logits) is written as sp->out_parts parts of out_pstride columns each (lddz >= out_parts * out_pstride). */
-int rlppo_policy_head_train_split(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw,
-                                  const float* bias, int64_t M, int n_actions, int K, const float* actions,
-                                  const float* old_logp, const float* adv, float inv_batch, float clip,
-                                  float ent_coef, uint16_t* dz, int64_t lddz, float* logp_out, float* metrics,
-                                  const rlppo_split* sp, void* stream);
-/* rlppo_value_head with H given as h_parts parts and dH written as dh_parts parts. */
-int rlppo_value_head_split(const uint16_t* h, int64_t ldh, const float* w, const float* bias, int64_t M, int K,
-                           float* values_out, const float* targets, float inv_batch, uint16_t* dh, int64_t lddh,
-                           float* dw, float* db, float* metrics, int h_parts, int64_t h_pstride, int dh_parts,
-                           int64_t dh_pstride, void* stream);
+                     float* dw, float* db, float* metrics, int h_parts, int64_t h_pstride, int dh_parts,
+                     int64_t dh_pstride, void* stream);
 
 /* ---- (f-4) the other two action heads: multi_discrete_policy.py:16-89, continuous_policy.py:23-120 ------------
- * Per-row tails over the output of the policy's last Linear (run it with rlppo_linear_fwd_split, relu = 0, out_parts = 3:
+ * Per-row tails over the output of the policy's last Linear (run it with rlppo_linear_fwd, relu = 0, out_parts = 3:
  * z = the logits as split bf16 parts, fp32-exact).  z view: z [M, ldz], z_parts parts z_pstride columns apart.
  *
  * MultiDiscrete (21 logits = 8 categoricals with bins 3,3,3,3,3,2,2,2; torch_functions.py:81-122): log-prob and entropy
@@ -306,7 +291,8 @@ int rlppo_head_continuous_sample(const uint16_t* z, int64_t ldz, int z_parts, in
  * The training heads above differentiate the PPO loss only.  These take the gradient of each forward output as a
  * DEVICE pointer (every one optional, NULL = zero; the entropy gradient is f32[1], nothing is read on the host) and
  * write d(logits) in the layout the head's weight / data gradient GEMMs consume, as the _train forms do.
- *   rlppo_policy_head_backward[_split]: head GEMM + epilogue as rlppo_policy_head_train[_split], minus the loss block.
+ *   rlppo_policy_head_backward: head GEMM + epilogue as rlppo_policy_head_train (sp and dz as there), minus the loss
+ *     block.
  *     d_logp f32[M] (gathered log-prob of `actions`), d_ent f32[1] (mean entropy: each row gets d_ent / M),
  *     d_probs f32[M, n_actions] (get_output's unclamped softmax, added outside the clamp mask):
  *     g_j = [1e-11 <= s_j <= 1] (d_logp/p_a [j == a] - (d_ent/M)(log p_j + 1)) + d_probs_j;  dz = s (.) (g - sum g s)
@@ -315,16 +301,13 @@ int rlppo_head_continuous_sample(const uint16_t* z, int64_t ldz, int z_parts, in
  *     (ref_oracle.py:441-449).  get_output's gradient IS d(logits): stage it with rlppo_rows_to_bf16 / _split_bf16.
  *   rlppo_head_continuous_backward: d_logp, d_ent (mean over M*n elements, ref_oracle.py:473-478) and get_output's
  *     d_mean / d_std f32[M, n], back through the affine map of the std half and the Tanh.
- *   rlppo_value_head_backward[_split]: rlppo_value_head's training pass with dv = d_values[row] loaded:
+ *   rlppo_value_head_backward: rlppo_value_head's training pass (split parts as there) with dv = d_values[row] loaded:
  *     dH = dv * w (.) (H > 0);  dw[K] += sum_m dv*H;  db[1] += sum dv.  d_values is the head's only upstream gradient
  *     and is required (NULL: RLPPO_ERR_ARG); db may be NULL. */
 int rlppo_policy_head_backward(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
                                int64_t M, int n_actions, int K, const float* actions, const float* d_logp,
-                               const float* d_ent, const float* d_probs, uint16_t* dz, int64_t lddz, void* stream);
-int rlppo_policy_head_backward_split(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
-                                     int64_t M, int n_actions, int K, const float* actions, const float* d_logp,
-                                     const float* d_ent, const float* d_probs, uint16_t* dz, int64_t lddz,
-                                     const rlppo_split* sp, void* stream);
+                               const float* d_ent, const float* d_probs, uint16_t* dz, int64_t lddz,
+                               const rlppo_split* sp, void* stream);
 int rlppo_head_multi_discrete_backward(const uint16_t* z, int64_t ldz, int z_parts, int64_t z_pstride, int64_t M,
                                        const float* actions, int64_t ld_act, const float* d_logp, const float* d_ent,
                                        uint16_t* dz, int64_t lddz, int dz_parts, int64_t dz_pstride, int dz_cols,
@@ -335,10 +318,8 @@ int rlppo_head_continuous_backward(const uint16_t* z, int64_t ldz, int z_parts, 
                                    uint16_t* dz, int64_t lddz, int dz_parts, int64_t dz_pstride, int dz_cols,
                                    void* stream);
 int rlppo_value_head_backward(const uint16_t* h, int64_t ldh, const float* w, int64_t M, int K,
-                              const float* d_values, uint16_t* dh, int64_t lddh, float* dw, float* db, void* stream);
-int rlppo_value_head_backward_split(const uint16_t* h, int64_t ldh, const float* w, int64_t M, int K,
-                                    const float* d_values, uint16_t* dh, int64_t lddh, float* dw, float* db,
-                                    int h_parts, int64_t h_pstride, int dh_parts, int64_t dh_pstride, void* stream);
+                              const float* d_values, uint16_t* dh, int64_t lddh, float* dw, float* db,
+                              int h_parts, int64_t h_pstride, int dh_parts, int64_t dh_pstride, void* stream);
 
 /* ---- whole-network fused kernels (hidden widths 64/128/192/256, <= 4 hidden layers, obs <= 256, <= 128 actions) ----
  * One persistent tcgen05 kernel runs a 128-row tile of samples through the WHOLE Linear/ReLU stack, the head and
@@ -469,7 +450,7 @@ int rlppo_sqdiff(const float* a, const float* b, const int64_t* h_seg_off, int n
 
 /* ---- wide discrete head: DiscreteFF with 257 <= n_actions <= 4096 -------------------------------------------------
  * The fused epilogue of rlppo_policy_head_* holds a row's logits in one TMEM tile (<= 256 actions).  Wider softmax
- * policies run their last Linear as rlppo_linear_fwd_split (relu = 0, out_parts = 3: fp32-exact logits as split bf16
+ * policies run their last Linear as rlppo_linear_fwd (relu = 0, out_parts = 3: fp32-exact logits as split bf16
  * parts, as the (f-4) heads above) and these per-row kernels over it, one warp per row.  The z view is as for the (f-4)
  * heads and must allow 16-byte accesses: z 16-byte aligned, ldz and z_pstride multiples of 8, every part pad8(n_actions)
  * columns wide.  The arithmetic is that of the epilogue forms (p = clamp(softmax(z), 1e-11, 1)); only the order of the

@@ -42,37 +42,27 @@ _SIGS = {
     "rlppo_ring_append_fields_dev": ([_P, _I, _L, _P, _L, _P], _I),
     "rlppo_gather_batch": ([_P, _P, _P, _P, _P, _L, _P, _L, _I, _L, _L, _P, _P, _L, _P, _P, _P, _P, _P, _P, _P], _I),
     "rlppo_host_permutation": ([_P, _P, _L, _P], _I),
-    "rlppo_rows_to_bf16": ([_P, _L, _L, _I, _P, _L, _P], _I),
-    "rlppo_rows_standardize_to_bf16": ([_P, _L, _L, _I, _P, _P, _F, _P, _L, _P, _L, _P], _I),
+    "rlppo_rows_to_bf16": ([_P, _L, _L, _I, _P, _P, _F, _P, _L, _P, _L, _P], _I),
     "rlppo_weight_to_bf16": ([_P, _I, _I, _P, _L, _I, _P, _L, _I, _P], _I),
-    "rlppo_linear_fwd": ([_P, _L, _P, _L, _P, _P, _L, _L, _I, _I, _I, _P], _I),
-    "rlppo_linear_dgrad": ([_P, _L, _P, _L, _P, _L, _P, _L, _L, _I, _I, _P], _I),
-    "rlppo_linear_dgrad_db": ([_P, _L, _P, _L, _P, _L, _P, _L, _P, _L, _I, _I, _P], _I),
-    "rlppo_linear_wgrad": ([_P, _L, _P, _L, _P, _L, _P, _L, _I, _I, _P], _I),
+    "rlppo_linear_fwd": ([_P, _L, _P, _L, _P, _I, _P, _L, _L, _I, _I, _I, _P, _P], _I),
+    "rlppo_linear_dgrad": ([_P, _L, _P, _L, _P, _L, _P, _L, _P, _L, _I, _I, _P, _P], _I),
+    "rlppo_linear_wgrad": ([_P, _L, _P, _L, _P, _L, _P, _L, _I, _I, _P, _P], _I),
     "rlppo_wgrad_multi": ([_P, _I, _P], _I),
-    "rlppo_policy_head_sample": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _U64, _U64, _I, _P, _P, _P, _P, _P], _I),
-    "rlppo_policy_head_train": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _P, _P, _F, _F, _F, _P, _L, _P, _P, _P], _I),
-    "rlppo_value_head": ([_P, _L, _P, _P, _L, _I, _P, _P, _F, _P, _L, _P, _P, _P, _P], _I),
+    "rlppo_policy_head_sample": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _U64, _U64, _I, _P, _P, _P, _P, _P, _P], _I),
+    "rlppo_policy_head_train": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _P, _P, _F, _F, _F, _P, _L, _P, _P, _P, _P], _I),
+    "rlppo_value_head": ([_P, _L, _P, _P, _L, _I, _P, _P, _F, _P, _L, _P, _P, _P, _I, _L, _I, _L, _P], _I),
     "rlppo_rows_split_bf16": ([_P, _L, _L, _I, _P, _P, _F, _P, _L, _I, _L, _P], _I),
     "rlppo_weight_split_bf16": ([_P, _I, _I, _P, _L, _I, _L, _I, _P, _L, _I, _L, _I, _P], _I),
-    "rlppo_linear_fwd_split": ([_P, _L, _P, _L, _P, _I, _P, _L, _L, _I, _I, _I, _P, _P], _I),
-    "rlppo_linear_dgrad_split": ([_P, _L, _P, _L, _P, _L, _P, _L, _P, _L, _I, _I, _P, _P], _I),
-    "rlppo_linear_wgrad_split": ([_P, _L, _P, _L, _P, _L, _P, _L, _I, _I, _P, _P], _I),
-    "rlppo_policy_head_sample_split": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _U64, _U64, _I, _P, _P, _P, _P, _P, _P], _I),
-    "rlppo_policy_head_train_split": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _P, _P, _F, _F, _F, _P, _L, _P, _P, _P, _P], _I),
-    "rlppo_value_head_split": ([_P, _L, _P, _P, _L, _I, _P, _P, _F, _P, _L, _P, _P, _P, _I, _L, _I, _L, _P], _I),
     "rlppo_head_multi_discrete_train": ([_P, _L, _I, _L, _L, _P, _L, _P, _P, _F, _F, _F, _P, _L, _I, _L, _I, _P, _P, _P], _I),
     "rlppo_head_multi_discrete_sample": ([_P, _L, _I, _L, _L, _P, _U64, _U64, _I, _P, _L, _P, _P], _I),
     "rlppo_head_continuous_train": ([_P, _L, _I, _L, _L, _I, _F, _F, _P, _L, _P, _P, _F, _F, _F, _P, _L, _I, _L, _I, _P,
                                      _P, _P], _I),
     "rlppo_head_continuous_sample": ([_P, _L, _I, _L, _L, _I, _F, _F, _P, _U64, _U64, _I, _P, _L, _P, _P], _I),
-    "rlppo_policy_head_backward": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _P, _P, _P, _P, _L, _P], _I),
-    "rlppo_policy_head_backward_split": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _P, _P, _P, _P, _L, _P, _P], _I),
+    "rlppo_policy_head_backward": ([_P, _L, _P, _L, _P, _L, _I, _I, _P, _P, _P, _P, _P, _L, _P, _P], _I),
     "rlppo_head_multi_discrete_backward": ([_P, _L, _I, _L, _L, _P, _L, _P, _P, _P, _L, _I, _L, _I, _P], _I),
     "rlppo_head_continuous_backward": ([_P, _L, _I, _L, _L, _I, _F, _F, _P, _L, _P, _P, _P, _P, _P, _L, _I, _L, _I, _P],
                                        _I),
-    "rlppo_value_head_backward": ([_P, _L, _P, _L, _I, _P, _P, _L, _P, _P, _P], _I),
-    "rlppo_value_head_backward_split": ([_P, _L, _P, _L, _I, _P, _P, _L, _P, _P, _I, _L, _I, _L, _P], _I),
+    "rlppo_value_head_backward": ([_P, _L, _P, _L, _I, _P, _P, _L, _P, _P, _I, _L, _I, _L, _P], _I),
     "rlppo_policy_train_fused": ([_P, _P, _L, _I, _P, _P, _P, _F, _F, _F, _P, _P, _P], _I),
     "rlppo_policy_infer_fused": ([_P, _P, _L, _I, _P, _U64, _U64, _P, _I, _P, _P, _P, _P], _I),
     "rlppo_u64_add": ([_P, _U64, _P], _I),

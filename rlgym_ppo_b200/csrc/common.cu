@@ -63,7 +63,7 @@ int num_sms() {
 }  // namespace rlppo
 
 extern "C" {
-int rlppo_version(void) { return 100; }
+int rlppo_version(void) { return 101; }
 const char* rlppo_last_error(void) { return rlppo::g_err; }
 int rlppo_device_check(void) { return rlppo::check_device(); }
 }

@@ -3,7 +3,7 @@
 //                     categoricals (bins 3,3,3,3,3,2,2,2); log-prob and entropy summed over the eight.
 //   ContinuousPolicy  continuous_policy.py:23-120 + MapContinuousToAction (torch_functions.py:15-33): Tanh over 2n outputs,
 //                     mean = first half, std = second half mapped onto [var_min, var_max], diagonal Gaussian.
-// Their last Linear runs on the tensor-core GEMM (rlppo_linear_fwd[_split], output written as three bf16 parts so the
+// Their last Linear runs on the tensor-core GEMM (rlppo_linear_fwd, output written as three bf16 parts so the
 // logits keep fp32 precision); these kernels are the per-row tails -- sampling (get_action), and for training
 // get_backprop_data + the PPO loss block (ppo_learner.py:146-185) + its analytic backward into the logits.  At most 21 /
 // 2n <= 64 columns per row: one thread per row, HBM-bound, ~100-200 B per row.
@@ -299,7 +299,7 @@ __global__ void head_ct_kernel(ZView z, int64_t M, int n_act, float var_m, float
 
 // ---- Discrete, wide (257..4096 actions) ---------------------------------------------------------------------------
 // DiscreteFF (discrete_policy.py:22-80) for action spaces too wide for the head GEMM's fused epilogue, where a row's
-// logits must fit one TMEM tile (<= 256 columns).  The last Linear writes its logits as split parts (rlppo_linear_fwd_split)
+// logits must fit one TMEM tile (<= 256 columns).  The last Linear writes its logits as split parts (rlppo_linear_fwd)
 // and this kernel is the per-row tail, one warp per row (grid-stride over the rows):
 //   1. the row's logits, summed from their parts, into shared memory (the only HBM read of z: each lane loads 8
 //      consecutive columns of a part as one 16-byte word, so a warp reads 512 contiguous bytes per part and load), with

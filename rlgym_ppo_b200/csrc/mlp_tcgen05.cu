@@ -1204,9 +1204,8 @@ int launch_wgrad_t(const CUtensorMap& tmX, const CUtensorMap& tmDY, const WgradP
 
 extern "C" {
 
-int rlppo_linear_fwd_split(const uint16_t* x, int64_t ldx, const uint16_t* w, int64_t ldw, const float* bias,
-                           int bias_n, uint16_t* y, int64_t ldy, int64_t M, int N, int K, int relu,
-                           const rlppo_split* sp, void* stream) {
+int rlppo_linear_fwd(const uint16_t* x, int64_t ldx, const uint16_t* w, int64_t ldw, const float* bias, int bias_n,
+                     uint16_t* y, int64_t ldy, int64_t M, int N, int K, int relu, const rlppo_split* sp, void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(x && w && y, "null pointer");
     RLPPO_CHECK_ARG(N % 8 == 0 && ldy >= N && ldy % 8 == 0, "N and ldy must be multiples of 8");
@@ -1217,14 +1216,9 @@ int rlppo_linear_fwd_split(const uint16_t* x, int64_t ldx, const uint16_t* w, in
     return launch_rowgemm<EPI_BIAS_ACT>(x, ldx, w, ldw, N, p, 0, sp, static_cast<cudaStream_t>(stream));
 }
 
-int rlppo_linear_fwd(const uint16_t* x, int64_t ldx, const uint16_t* w, int64_t ldw, const float* bias, uint16_t* y,
-                     int64_t ldy, int64_t M, int N, int K, int relu, void* stream) {
-    return rlppo_linear_fwd_split(x, ldx, w, ldw, bias, 0, y, ldy, M, N, K, relu, nullptr, stream);
-}
-
-int rlppo_linear_dgrad_split(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt, const uint16_t* hprev,
-                             int64_t ldh, uint16_t* dx, int64_t lddx, float* db_below, int64_t M, int N, int K,
-                             const rlppo_split* sp, void* stream) {
+int rlppo_linear_dgrad(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt, const uint16_t* hprev,
+                       int64_t ldh, uint16_t* dx, int64_t lddx, float* db_below, int64_t M, int N, int K,
+                       const rlppo_split* sp, void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(dy && wt && dx, "null pointer");
     RLPPO_CHECK_ARG(K % 8 == 0 && lddx >= K && lddx % 8 == 0, "K and lddx must be multiples of 8");
@@ -1236,21 +1230,10 @@ int rlppo_linear_dgrad_split(const uint16_t* dy, int64_t lddy, const uint16_t* w
     return launch_rowgemm<EPI_RELU_MASK>(dy, lddy, wt, ldwt, K, p, 0, sp, static_cast<cudaStream_t>(stream));
 }
 
-int rlppo_linear_dgrad(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt, const uint16_t* hprev,
-                       int64_t ldh, uint16_t* dx, int64_t lddx, int64_t M, int N, int K, void* stream) {
-    return rlppo_linear_dgrad_split(dy, lddy, wt, ldwt, hprev, ldh, dx, lddx, nullptr, M, N, K, nullptr, stream);
-}
-
-int rlppo_linear_dgrad_db(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt, const uint16_t* hprev,
-                          int64_t ldh, uint16_t* dx, int64_t lddx, float* db_below, int64_t M, int N, int K,
-                          void* stream) {
-    return rlppo_linear_dgrad_split(dy, lddy, wt, ldwt, hprev, ldh, dx, lddx, db_below, M, N, K, nullptr, stream);
-}
-
-int rlppo_policy_head_sample_split(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
-                                   int64_t M, int n_actions, int K, const float* u_inject, uint64_t seed,
-                                   uint64_t offset, int deterministic, float* actions_out, int64_t* actions_i64_out,
-                                   float* logp_out, float* probs_out, const rlppo_split* sp, void* stream) {
+int rlppo_policy_head_sample(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
+                             int64_t M, int n_actions, int K, const float* u_inject, uint64_t seed, uint64_t offset,
+                             int deterministic, float* actions_out, int64_t* actions_i64_out, float* logp_out,
+                             float* probs_out, const rlppo_split* sp, void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(h && w, "null pointer");
     RLPPO_CHECK_ARG(n_actions >= 1 && n_actions <= 256, "n_actions must be in [1,256]");
@@ -1262,18 +1245,10 @@ int rlppo_policy_head_sample_split(const uint16_t* h, int64_t ldh, const uint16_
     return launch_rowgemm<EPI_HEAD_SAMPLE>(h, ldh, w, ldw, n_actions, p, 128, sp, static_cast<cudaStream_t>(stream));
 }
 
-int rlppo_policy_head_sample(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
-                             int64_t M, int n_actions, int K, const float* u_inject, uint64_t seed, uint64_t offset,
-                             int deterministic, float* actions_out, int64_t* actions_i64_out, float* logp_out,
-                             float* probs_out, void* stream) {
-    return rlppo_policy_head_sample_split(h, ldh, w, ldw, bias, M, n_actions, K, u_inject, seed, offset, deterministic,
-                                          actions_out, actions_i64_out, logp_out, probs_out, nullptr, stream);
-}
-
-int rlppo_policy_head_train_split(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
-                                  int64_t M, int n_actions, int K, const float* actions, const float* old_logp,
-                                  const float* adv, float inv_batch, float clip, float ent_coef, uint16_t* dz,
-                                  int64_t lddz, float* logp_out, float* metrics, const rlppo_split* sp, void* stream) {
+int rlppo_policy_head_train(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
+                            int64_t M, int n_actions, int K, const float* actions, const float* old_logp,
+                            const float* adv, float inv_batch, float clip, float ent_coef, uint16_t* dz, int64_t lddz,
+                            float* logp_out, float* metrics, const rlppo_split* sp, void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(h && w && actions && old_logp && adv && dz, "null pointer");
     RLPPO_CHECK_ARG(n_actions >= 1 && n_actions <= 256, "n_actions must be in [1,256]");
@@ -1291,22 +1266,14 @@ int rlppo_policy_head_train_split(const uint16_t* h, int64_t ldh, const uint16_t
     return launch_rowgemm<EPI_HEAD_TRAIN>(h, ldh, w, ldw, n_actions, p, min_bn, sp, static_cast<cudaStream_t>(stream));
 }
 
-int rlppo_policy_head_train(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
-                            int64_t M, int n_actions, int K, const float* actions, const float* old_logp,
-                            const float* adv, float inv_batch, float clip, float ent_coef, uint16_t* dz, int64_t lddz,
-                            float* logp_out, float* metrics, void* stream) {
-    return rlppo_policy_head_train_split(h, ldh, w, ldw, bias, M, n_actions, K, actions, old_logp, adv, inv_batch, clip,
-                                         ent_coef, dz, lddz, logp_out, metrics, nullptr, stream);
-}
-
 // Backward of get_backprop_data (discrete_policy.py:64-80: clamp(softmax(z), 1e-11, 1) -> log -> gather / entropy mean)
 // and of get_output (:35-42, the unclamped softmax) for arbitrary upstream gradients; the clamp passes gradient where
 // 1e-11 <= s_j <= 1 (torch.clamp's backward):
 //   g_j = mask_j * (d_logp/p_a [j == a] - (d_ent/M)(log p_j + 1)) + d_probs_j,  dz = s (.) (g - sum g.s).
-int rlppo_policy_head_backward_split(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
-                                     int64_t M, int n_actions, int K, const float* actions, const float* d_logp,
-                                     const float* d_ent, const float* d_probs, uint16_t* dz, int64_t lddz,
-                                     const rlppo_split* sp, void* stream) {
+int rlppo_policy_head_backward(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
+                               int64_t M, int n_actions, int K, const float* actions, const float* d_logp,
+                               const float* d_ent, const float* d_probs, uint16_t* dz, int64_t lddz,
+                               const rlppo_split* sp, void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(h && w && dz && (d_logp == nullptr || actions != nullptr), "null pointer");
     RLPPO_CHECK_ARG(n_actions >= 1 && n_actions <= 256, "n_actions must be in [1,256]");
@@ -1322,15 +1289,8 @@ int rlppo_policy_head_backward_split(const uint16_t* h, int64_t ldh, const uint1
     return launch_rowgemm<EPI_HEAD_BWD>(h, ldh, w, ldw, n_actions, p, min_bn, sp, static_cast<cudaStream_t>(stream));
 }
 
-int rlppo_policy_head_backward(const uint16_t* h, int64_t ldh, const uint16_t* w, int64_t ldw, const float* bias,
-                               int64_t M, int n_actions, int K, const float* actions, const float* d_logp,
-                               const float* d_ent, const float* d_probs, uint16_t* dz, int64_t lddz, void* stream) {
-    return rlppo_policy_head_backward_split(h, ldh, w, ldw, bias, M, n_actions, K, actions, d_logp, d_ent, d_probs, dz,
-                                            lddz, nullptr, stream);
-}
-
-int rlppo_linear_wgrad_split(const uint16_t* dy, int64_t lddy, const uint16_t* x, int64_t ldx, float* dw, int64_t lddw,
-                             float* db, int64_t M, int N, int K, const rlppo_split* sp, void* stream) {
+int rlppo_linear_wgrad(const uint16_t* dy, int64_t lddy, const uint16_t* x, int64_t ldx, float* dw, int64_t lddw,
+                       float* db, int64_t M, int N, int K, const rlppo_split* sp, void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(dy && x && dw && M >= 1 && N >= 1 && K >= 1, "bad argument");
     RLPPO_CHECK_ARG(M < (1ll << 31), "M too large for TMA coordinates");
@@ -1394,11 +1354,6 @@ int rlppo_linear_wgrad_split(const uint16_t* dy, int64_t lddy, const uint16_t* x
         }
     }
     return RLPPO_OK;
-}
-
-int rlppo_linear_wgrad(const uint16_t* dy, int64_t lddy, const uint16_t* x, int64_t ldx, float* dw, int64_t lddw,
-                       float* db, int64_t M, int N, int K, void* stream) {
-    return rlppo_linear_wgrad_split(dy, lddy, x, ldx, dw, lddw, db, M, N, K, nullptr, stream);
 }
 
 int rlppo_wgrad_multi(const rlppo_wgrad_item* h_items, int n_items, void* stream) {

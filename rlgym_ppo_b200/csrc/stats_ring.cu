@@ -431,35 +431,26 @@ int rlppo_gather_batch(const float* actions, const float* logp, const float* val
     return RLPPO_OK;
 }
 
-int rlppo_rows_to_bf16(const float* src, int64_t src_ld, int64_t n_rows, int width, uint16_t* dst, int64_t dst_ld,
+int rlppo_rows_to_bf16(const float* src, int64_t src_ld, int64_t n_rows, int width, const float* mean,
+                       const float* stdv, float clip, uint16_t* dst, int64_t dst_ld, float* dst_f32, int64_t dst_f32_ld,
                        void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(src && dst && dst_ld >= width && n_rows >= 0, "bad argument");
-    RLPPO_CHECK_ARG(dst_ld % 8 == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0,
-                    "bf16 rows: dst_ld must be a multiple of 8 and dst 16-byte aligned");
-    if (n_rows == 0) return RLPPO_OK;
-    const int64_t total = n_rows * (dst_ld / 8);
-    const unsigned blocks = (unsigned)min((int64_t)rlppo::num_sms() * 16, (total + 255) / 256);
-    rows_to_bf16_kernel<false><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(src, src_ld, n_rows, width, nullptr,
-                                                                                       nullptr, 0.f, dst, dst_ld, nullptr, 0);
-    RLPPO_LAUNCH_CHECK();
-    return RLPPO_OK;
-}
-
-int rlppo_rows_standardize_to_bf16(const float* src, int64_t src_ld, int64_t n_rows, int width, const float* mean,
-                                   const float* stdv, float clip, uint16_t* dst, int64_t dst_ld, float* dst_f32,
-                                   int64_t dst_f32_ld, void* stream) {
-    RLPPO_REQUIRE_DEVICE();
-    RLPPO_CHECK_ARG(src && dst && mean && stdv && dst_ld >= width && n_rows >= 0, "bad argument");
+    RLPPO_CHECK_ARG((mean == nullptr) == (stdv == nullptr), "mean and std go together");
+    RLPPO_CHECK_ARG(mean || !dst_f32, "dst_f32 holds standardised rows: it needs mean and std");
     RLPPO_CHECK_ARG(dst_ld % 8 == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0,
                     "bf16 rows: dst_ld must be a multiple of 8 and dst 16-byte aligned");
     if (n_rows == 0) return RLPPO_OK;
     const int64_t total = n_rows * (dst_ld / 8);
     const unsigned blocks = (unsigned)min((int64_t)rlppo::num_sms() * 16, (total + 255) / 256);
     RLPPO_CHECK_ARG(!dst_f32 || dst_f32_ld >= width, "dst_f32_ld must be >= width");
-    rows_to_bf16_kernel<true><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(src, src_ld, n_rows, width, mean,
-                                                                                      stdv, clip, dst, dst_ld, dst_f32,
-                                                                                      dst_f32_ld);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (mean == nullptr)
+        rows_to_bf16_kernel<false><<<blocks, 256, 0, s>>>(src, src_ld, n_rows, width, nullptr, nullptr, 0.f, dst, dst_ld,
+                                                          nullptr, 0);
+    else
+        rows_to_bf16_kernel<true><<<blocks, 256, 0, s>>>(src, src_ld, n_rows, width, mean, stdv, clip, dst, dst_ld, dst_f32,
+                                                         dst_f32_ld);
     RLPPO_LAUNCH_CHECK();
     return RLPPO_OK;
 }

@@ -157,10 +157,10 @@ int launch(const uint16_t* h, int64_t ldh, const float* w, const float* bias, in
 
 }  // namespace
 
-extern "C" int rlppo_value_head_split(const uint16_t* h, int64_t ldh, const float* w, const float* bias, int64_t M,
-                                      int K, float* values_out, const float* targets, float inv_batch, uint16_t* dh,
-                                      int64_t lddh, float* dw, float* db, float* metrics, int h_parts, int64_t h_pstride,
-                                      int dh_parts, int64_t dh_pstride, void* stream) {
+extern "C" int rlppo_value_head(const uint16_t* h, int64_t ldh, const float* w, const float* bias, int64_t M, int K,
+                                float* values_out, const float* targets, float inv_batch, uint16_t* dh, int64_t lddh,
+                                float* dw, float* db, float* metrics, int h_parts, int64_t h_pstride, int dh_parts,
+                                int64_t dh_pstride, void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(h && w && M >= 1, "bad argument");
     RLPPO_CHECK_ARG(K % 8 == 0 && K >= 8 && K <= 2048 && ldh % 8 == 0, "K must be a multiple of 8 in [8,2048]");
@@ -182,19 +182,11 @@ extern "C" int rlppo_value_head_split(const uint16_t* h, int64_t ldh, const floa
 #undef RLPPO_VH
 }
 
-extern "C" int rlppo_value_head(const uint16_t* h, int64_t ldh, const float* w, const float* bias, int64_t M, int K,
-                                float* values_out, const float* targets, float inv_batch, uint16_t* dh, int64_t lddh,
-                                float* dw, float* db, float* metrics, void* stream) {
-    return rlppo_value_head_split(h, ldh, w, bias, M, K, values_out, targets, inv_batch, dh, lddh, dw, db, metrics, 1, 0, 1,
-                                  0, stream);
-}
-
 // Backward of ValueEstimator.forward (value_estimator.py:27, the last Linear(K,1) over ReLU activations H) for an
 // arbitrary upstream gradient d_values f32[M] (device): dH = dv * w (.) (H > 0), dw[K] += sum_m dv*H, db[1] += sum dv.
-extern "C" int rlppo_value_head_backward_split(const uint16_t* h, int64_t ldh, const float* w, int64_t M, int K,
-                                               const float* d_values, uint16_t* dh, int64_t lddh, float* dw, float* db,
-                                               int h_parts, int64_t h_pstride, int dh_parts, int64_t dh_pstride,
-                                               void* stream) {
+extern "C" int rlppo_value_head_backward(const uint16_t* h, int64_t ldh, const float* w, int64_t M, int K,
+                                         const float* d_values, uint16_t* dh, int64_t lddh, float* dw, float* db,
+                                         int h_parts, int64_t h_pstride, int dh_parts, int64_t dh_pstride, void* stream) {
     RLPPO_REQUIRE_DEVICE();
     RLPPO_CHECK_ARG(h && w && d_values && dh && dw && M >= 1, "bad argument");
     RLPPO_CHECK_ARG(K % 8 == 0 && K >= 8 && K <= 2048 && ldh % 8 == 0, "K must be a multiple of 8 in [8,2048]");
@@ -212,10 +204,4 @@ extern "C" int rlppo_value_head_backward_split(const uint16_t* h, int64_t ldh, c
     if (K <= 1024) return RLPPO_VHB(4);
     return RLPPO_VHB(8);
 #undef RLPPO_VHB
-}
-
-extern "C" int rlppo_value_head_backward(const uint16_t* h, int64_t ldh, const float* w, int64_t M, int K,
-                                         const float* d_values, uint16_t* dh, int64_t lddh, float* dw, float* db,
-                                         void* stream) {
-    return rlppo_value_head_backward_split(h, ldh, w, M, K, d_values, dh, lddh, dw, db, 1, 0, 1, 0, stream);
 }

@@ -153,13 +153,9 @@ def gather_batch(buf, idx, out_actions=None, out_logp=None, out_values=None, out
 def rows_to_bf16(src, dst, mean=None, std=None, clip=5.0, dst_f32=None):
     n_rows, width = src.shape
     assert dst.dtype == BF16 and dst.shape[0] >= n_rows
-    if mean is None:
-        call("rlppo_rows_to_bf16", ptr(src), src.stride(0), n_rows, width, ptr(dst), dst.stride(0), stream_ptr(),
-             work=("byte", n_rows * (4 * width + 2 * dst.stride(0))))
-    else:
-        call("rlppo_rows_standardize_to_bf16", ptr(src), src.stride(0), n_rows, width, ptr(mean), ptr(std),
-             float(clip), ptr(dst), dst.stride(0), ptr(dst_f32), 0 if dst_f32 is None else dst_f32.stride(0),
-             stream_ptr(), work=("byte", n_rows * (4 * width + 2 * dst.stride(0))))
+    call("rlppo_rows_to_bf16", ptr(src), src.stride(0), n_rows, width, ptr(mean), ptr(std), float(clip), ptr(dst),
+         dst.stride(0), ptr(dst_f32), 0 if dst_f32 is None else dst_f32.stride(0), stream_ptr(),
+         work=("byte", n_rows * (4 * width + 2 * dst.stride(0))))
 
 
 def weight_to_bf16(w, wq, wt=None):
@@ -212,44 +208,29 @@ def weight_split(w, wq, q_parts, q_pstride, wt=None, t_parts=0, t_pstride=0):
 def linear_fwd(x, wq, bias, y, N, K, relu, M=None, split=None, bias_n=0):
     M = x.shape[0] if M is None else M
     if split is not None:
-        call("rlppo_linear_fwd_split", ptr(x), x.stride(0), ptr(wq), wq.stride(0), ptr(bias), int(bias_n), ptr(y),
-             y.stride(0), int(M), int(N), int(K), int(bool(relu)), _sp(split), stream_ptr(),
-             work=("flop", 2.0 * M * N * K, "mma_flop", 2.0 * M * N * K * _n_products(split),
-                   "byte", 2.0 * (M * K * split.a_parts + N * K * split.b_parts + M * N * split.out_parts)))
-        return
-    call("rlppo_linear_fwd", ptr(x), x.stride(0), ptr(wq), wq.stride(0), ptr(bias), ptr(y), y.stride(0), int(M),
-         int(N), int(K), int(bool(relu)), stream_ptr(),
-         work=("flop", 2.0 * M * N * K, "byte", 2.0 * (M * K + N * K + M * N)))
+        work = ("flop", 2.0 * M * N * K, "mma_flop", 2.0 * M * N * K * _n_products(split),
+                "byte", 2.0 * (M * K * split.a_parts + N * K * split.b_parts + M * N * split.out_parts))
+    else:
+        work = ("flop", 2.0 * M * N * K, "byte", 2.0 * (M * K + N * K + M * N))
+    call("rlppo_linear_fwd", ptr(x), x.stride(0), ptr(wq), wq.stride(0), ptr(bias), int(bias_n), ptr(y), y.stride(0),
+         int(M), int(N), int(K), int(bool(relu)), _sp(split), stream_ptr(), work=work)
 
 
 def linear_dgrad(dy, wt, hprev, dx, N, K, M=None, db_below=None, split=None):
     """db_below (optional f32[K]): += column sums of dx, the bias gradient of the layer below (fused into the epilogue)."""
     M = dy.shape[0] if M is None else M
-    work = ("flop", 2.0 * M * N * K, "byte", 2.0 * (M * N + N * K + M * K * (2 if hprev is not None else 1)))
-    if split is not None:
-        call("rlppo_linear_dgrad_split", ptr(dy), dy.stride(0), ptr(wt), wt.stride(0), ptr(hprev),
-             0 if hprev is None else hprev.stride(0), ptr(dx), dx.stride(0), ptr(db_below), int(M), int(N), int(K),
-             _sp(split), stream_ptr(), work=work)
-        return
-    if db_below is None:
-        call("rlppo_linear_dgrad", ptr(dy), dy.stride(0), ptr(wt), wt.stride(0), ptr(hprev),
-             0 if hprev is None else hprev.stride(0), ptr(dx), dx.stride(0), int(M), int(N), int(K), stream_ptr(),
-             work=work)
-    else:
-        call("rlppo_linear_dgrad_db", ptr(dy), dy.stride(0), ptr(wt), wt.stride(0), ptr(hprev),
-             0 if hprev is None else hprev.stride(0), ptr(dx), dx.stride(0), ptr(db_below), int(M), int(N), int(K),
-             stream_ptr(), work=work)
+    call("rlppo_linear_dgrad", ptr(dy), dy.stride(0), ptr(wt), wt.stride(0), ptr(hprev),
+         0 if hprev is None else hprev.stride(0), ptr(dx), dx.stride(0), ptr(db_below), int(M), int(N), int(K),
+         _sp(split), stream_ptr(),
+         work=("flop", 2.0 * M * N * K, "byte", 2.0 * (M * N + N * K + M * K * (2 if hprev is not None else 1))))
 
 
 def linear_wgrad(dy, x, dw, db, N, K, M=None, split=None):
     M = dy.shape[0] if M is None else M
-    if split is not None:
-        call("rlppo_linear_wgrad_split", ptr(dy), dy.stride(0), ptr(x), x.stride(0), ptr(dw), dw.stride(0), ptr(db),
-             int(M), int(N), int(K), _sp(split), stream_ptr(),
-             work=("flop", 2.0 * M * N * K, "byte", 2.0 * M * (N * split.a_parts + K * split.b_parts) + 4.0 * N * K))
-        return
+    a_parts, b_parts = (1, 1) if split is None else (split.a_parts, split.b_parts)
     call("rlppo_linear_wgrad", ptr(dy), dy.stride(0), ptr(x), x.stride(0), ptr(dw), dw.stride(0), ptr(db), int(M),
-         int(N), int(K), stream_ptr(), work=("flop", 2.0 * M * N * K, "byte", 2.0 * M * (N + K) + 4.0 * N * K))
+         int(N), int(K), _sp(split), stream_ptr(),
+         work=("flop", 2.0 * M * N * K, "byte", 2.0 * M * (N * a_parts + K * b_parts) + 4.0 * N * K))
 
 
 def wgrad_multi(items, M):
@@ -274,44 +255,30 @@ def wgrad_multi(items, M):
 def policy_head_sample(h, wq, bias, n_actions, K, M=None, u=None, seed=0, offset=0, deterministic=False,
                        actions_out=None, actions_i64_out=None, logp_out=None, probs_out=None, split=None):
     M = h.shape[0] if M is None else M
-    if split is not None:
-        call("rlppo_policy_head_sample_split", ptr(h), h.stride(0), ptr(wq), wq.stride(0), ptr(bias), int(M),
-             int(n_actions), int(K), ptr(u), int(seed) & (2 ** 64 - 1), int(offset) & (2 ** 64 - 1),
-             int(bool(deterministic)), ptr(actions_out), ptr(actions_i64_out), ptr(logp_out), ptr(probs_out),
-             _sp(split), stream_ptr(), work=("flop", 2.0 * M * n_actions * K))
-        return
     call("rlppo_policy_head_sample", ptr(h), h.stride(0), ptr(wq), wq.stride(0), ptr(bias), int(M), int(n_actions),
          int(K), ptr(u), int(seed) & (2 ** 64 - 1), int(offset) & (2 ** 64 - 1), int(bool(deterministic)),
-         ptr(actions_out), ptr(actions_i64_out), ptr(logp_out), ptr(probs_out), stream_ptr(),
+         ptr(actions_out), ptr(actions_i64_out), ptr(logp_out), ptr(probs_out), _sp(split), stream_ptr(),
          work=("flop", 2.0 * M * n_actions * K))
 
 
 def policy_head_train(h, wq, bias, n_actions, K, actions, old_logp, adv, inv_batch, clip, ent_coef, dz, metrics,
                       logp_out=None, M=None, split=None):
     M = h.shape[0] if M is None else M
-    if split is not None:
-        call("rlppo_policy_head_train_split", ptr(h), h.stride(0), ptr(wq), wq.stride(0), ptr(bias), int(M),
-             int(n_actions), int(K), ptr(actions), ptr(old_logp), ptr(adv), float(inv_batch), float(clip),
-             float(ent_coef), ptr(dz), dz.stride(0), ptr(logp_out), ptr(metrics), _sp(split), stream_ptr(),
-             work=("flop", 2.0 * M * n_actions * K))
-        return
     call("rlppo_policy_head_train", ptr(h), h.stride(0), ptr(wq), wq.stride(0), ptr(bias), int(M), int(n_actions),
          int(K), ptr(actions), ptr(old_logp), ptr(adv), float(inv_batch), float(clip), float(ent_coef), ptr(dz),
-         dz.stride(0), ptr(logp_out), ptr(metrics), stream_ptr(), work=("flop", 2.0 * M * n_actions * K))
+         dz.stride(0), ptr(logp_out), ptr(metrics), _sp(split), stream_ptr(), work=("flop", 2.0 * M * n_actions * K))
 
 
 def value_head(h, w, bias, K, values_out=None, targets=None, inv_batch=0.0, dh=None, dw=None, db=None, metrics=None,
                M=None, h_parts=1, h_pstride=0, dh_parts=1, dh_pstride=0):
     M = h.shape[0] if M is None else M
     if h_parts > 1 or dh_parts > 1:
-        call("rlppo_value_head_split", ptr(h), h.stride(0), ptr(w), ptr(bias), int(M), int(K), ptr(values_out),
-             ptr(targets), float(inv_batch), ptr(dh), 0 if dh is None else dh.stride(0), ptr(dw), ptr(db), ptr(metrics),
-             int(h_parts), int(h_pstride), int(dh_parts), int(dh_pstride), stream_ptr(),
-             work=("byte", M * K * 2 * (h_parts + (dh_parts if targets is not None else 0)) + 8 * M))
-        return
+        nbytes = M * K * 2 * (h_parts + (dh_parts if targets is not None else 0)) + 8 * M
+    else:
+        nbytes = M * K * 2 * (2 if targets is not None else 1) + 4 * M * (2 if targets is not None else 1)
     call("rlppo_value_head", ptr(h), h.stride(0), ptr(w), ptr(bias), int(M), int(K), ptr(values_out), ptr(targets),
-         float(inv_batch), ptr(dh), 0 if dh is None else dh.stride(0), ptr(dw), ptr(db), ptr(metrics), stream_ptr(),
-         work=("byte", M * K * 2 * (2 if targets is not None else 1) + 4 * M * (2 if targets is not None else 1)))
+         float(inv_batch), ptr(dh), 0 if dh is None else dh.stride(0), ptr(dw), ptr(db), ptr(metrics), int(h_parts),
+         int(h_pstride), int(dh_parts), int(dh_pstride), stream_ptr(), work=("byte", nbytes))
 
 
 # ---- the other two action heads (rlppo_head_*: per-row tails over the split logits of the last Linear) ----------------
@@ -381,12 +348,9 @@ def head_discrete_backward(z, z_parts, z_pstride, M, n_actions, actions, d_logp,
 def policy_head_backward(h, wq, bias, n_actions, K, actions, d_logp, d_ent, d_probs, dz, M=None, split=None):
     """d_logp f32[M], d_ent f32[1], d_probs f32[M, n_actions]: device tensors or None."""
     M = h.shape[0] if M is None else M
-    args = (ptr(h), h.stride(0), ptr(wq), wq.stride(0), ptr(bias), int(M), int(n_actions), int(K), ptr(actions),
-            ptr(d_logp), ptr(d_ent), ptr(d_probs), ptr(dz), dz.stride(0))
-    if split is not None:
-        call("rlppo_policy_head_backward_split", *args, _sp(split), stream_ptr(), work=("flop", 2.0 * M * n_actions * K))
-        return
-    call("rlppo_policy_head_backward", *args, stream_ptr(), work=("flop", 2.0 * M * n_actions * K))
+    call("rlppo_policy_head_backward", ptr(h), h.stride(0), ptr(wq), wq.stride(0), ptr(bias), int(M), int(n_actions),
+         int(K), ptr(actions), ptr(d_logp), ptr(d_ent), ptr(d_probs), ptr(dz), dz.stride(0), _sp(split), stream_ptr(),
+         work=("flop", 2.0 * M * n_actions * K))
 
 
 def head_multi_discrete_backward(z, z_parts, z_pstride, M, actions, d_logp, d_ent, dz, dz_parts, dz_pstride, dz_cols):
@@ -405,14 +369,9 @@ def head_continuous_backward(z, z_parts, z_pstride, M, n_act, var_min, var_max, 
 
 def value_head_backward(h, w, K, d_values, dh, dw, db, M=None, h_parts=1, h_pstride=0, dh_parts=1, dh_pstride=0):
     M = h.shape[0] if M is None else M
-    work = ("byte", M * K * 2 * (h_parts + dh_parts) + 4 * M)
-    if h_parts > 1 or dh_parts > 1:
-        call("rlppo_value_head_backward_split", ptr(h), h.stride(0), ptr(w), int(M), int(K), ptr(d_values), ptr(dh),
-             dh.stride(0), ptr(dw), ptr(db), int(h_parts), int(h_pstride), int(dh_parts), int(dh_pstride), stream_ptr(),
-             work=work)
-        return
     call("rlppo_value_head_backward", ptr(h), h.stride(0), ptr(w), int(M), int(K), ptr(d_values), ptr(dh), dh.stride(0),
-         ptr(dw), ptr(db), stream_ptr(), work=work)
+         ptr(dw), ptr(db), int(h_parts), int(h_pstride), int(dh_parts), int(dh_pstride), stream_ptr(),
+         work=("byte", M * K * 2 * (h_parts + dh_parts) + 4 * M))
 
 
 # ---- whole-network fused kernels --------------------------------------------------------------------------------

@@ -364,18 +364,17 @@ class Stack:
         gw = self.gw if gw is None else gw
         gb = self.gb if gb is None else gb
         d = d_last
-        # fuse_db: the bias gradient of layer i-1 comes out of the dgrad epilogue that produces dL/dH_{i-1}
-        # (rlppo_linear_dgrad_db) instead of a separate column-sum pass over that tensor.  Measured on c3 in one box:
-        # 47.3 -> 46.4 ms per step (with the first, unpipelined epilogue it was a wash).  RLPPO_FUSE_DB=0 turns it off.
-        fuse_db = getattr(self, "fuse_bias_grad_into_dgrad", os.environ.get("RLPPO_FUSE_DB", "1") == "1")
-        db_done = False
+        # The bias gradient of layer i-1 comes out of the dgrad epilogue that produces dL/dH_{i-1} (db_below) instead of
+        # a separate column-sum pass over that tensor: only the top hidden layer's wgrad sums its own.  Measured on c3 in
+        # one box: 47.3 -> 46.4 ms per step (with the first, unpipelined epilogue it was a wash).
+        top = len(self.hidden) - 1
         d_ps = ops.pad64(max(self.hidden))        # "fp32" mode: part stride of the gradient ping-pong buffers
-        for i in range(len(self.hidden) - 1, -1, -1):
+        for i in range(top, -1, -1):
             inp = ws["h"][i - 1] if i > 0 else x
             K = self.hidden[i - 1] if i > 0 else self.in_dim
             N = self.hidden[i]
             sp_w = ops.make_split(2, 2, 2, 1, d_ps, ops.pad64(K)) if self.exact else None
-            ops.linear_wgrad(d, inp, gw[i], None if db_done else gb[i], N, K, M=M, split=sp_w)
+            ops.linear_wgrad(d, inp, gw[i], gb[i] if i == top else None, N, K, M=M, split=sp_w)
             if i > 0:
                 nxt = ws["d"][0] if d.data_ptr() != ws["d"][0].data_ptr() else ws["d"][1]
                 if self.exact:
@@ -384,9 +383,7 @@ class Stack:
                 else:
                     dx = nxt[:, :K] if nxt.shape[1] != K else nxt
                     sp_d = None
-                ops.linear_dgrad(d, self.wt[i], inp, dx, N, K, M=M, db_below=gb[i - 1] if fuse_db else None,
-                                 split=sp_d)
-                db_done = fuse_db
+                ops.linear_dgrad(d, self.wt[i], inp, dx, N, K, M=M, db_below=gb[i - 1], split=sp_d)
                 d = dx
 
     # ---- torch autograd ---------------------------------------------------------------------------------------------

@@ -3,6 +3,7 @@ declares, refuses to compute without a B200, and its host-side permutation is Nu
 import ctypes
 import os
 import re
+import subprocess
 
 import numpy as np
 import pytest
@@ -16,6 +17,12 @@ def _declared():
     return sorted(set(re.findall(r"\b(rlppo_[a-z0-9_]+)\s*\(", src)))
 
 
+def _exported(path):
+    """The rlppo_* functions the shared library defines (its dynamic symbol table)."""
+    out = subprocess.run(["nm", "-D", "--defined-only", path], check=True, capture_output=True, text=True).stdout
+    return sorted({f[2] for f in (line.split() for line in out.splitlines()) if len(f) == 3 and f[2].startswith("rlppo_")})
+
+
 def test_header_symbols_exported_and_bound():
     from rlgym_ppo_b200 import _lib
     lib = ctypes.CDLL(_lib.LIB_PATH)
@@ -25,6 +32,9 @@ def test_header_symbols_exported_and_bound():
         assert hasattr(lib, n), f"{n} declared in include/rlppo.h but not exported"
         assert n in _lib.EXPORTED, f"{n} not bound in rlgym_ppo_b200/_lib.py"
     assert sorted(_lib.EXPORTED) == names
+    # and nothing beyond the header: an entry point whose declaration is gone must not linger in a .cu file
+    undeclared = sorted(set(_exported(_lib.LIB_PATH)) - set(names))
+    assert not undeclared, f"exported by the library but not declared in include/rlppo.h: {undeclared}"
     assert _lib.version() >= 100
 
 
@@ -37,7 +47,7 @@ def test_no_cpu_fallback():
         _lib.require_device()
     # a compute entry point called without a device must fail, not compute on the host
     x = np.zeros(8, np.float32)
-    rc = _lib._lib.rlppo_rows_to_bf16(x.ctypes.data, 8, 1, 8, x.ctypes.data, 8, None)
+    rc = _lib._lib.rlppo_rows_to_bf16(x.ctypes.data, 8, 1, 8, None, None, 5.0, x.ctypes.data, 8, None, 0, None)
     assert rc == -3 and "no CPU fallback" in _lib.last_error()
 
 

@@ -264,7 +264,7 @@ FWD_SHAPES = [(256, 89, 0), (256, 256, 0), (1024, 2048, 0), (2048, 1024, 0), (24
 @pytest.mark.parametrize("M", [1, 127, 129, 50000])
 @pytest.mark.parametrize("N,K,bias_n", FWD_SHAPES, ids=[f"{n}x{k}" for n, k, _ in FWD_SHAPES])
 def test_linear_fwd_split(ops, M, N, K, bias_n):
-    """rlppo_linear_fwd_split with make_split(3,3,3,out_parts) (forward_hidden / logits in "fp32" mode) for relu 0/1 and
+    """rlppo_linear_fwd with make_split(3,3,3,out_parts) (forward_hidden / logits in "fp32" mode) for relu 0/1 and
     out_parts 1..3; make_split(3,3,2,3) must fail the bound; make_split(1,1,1,3) (the bf16 mode's logits: single-part
     operands, output as 3 parts) against fp64 of the bf16 operands, bound sqrt(K) * u.  The output starts as a sentinel:
     rows >= M and the columns between N and the part stride stay untouched; with relu every part of a negative
@@ -355,7 +355,7 @@ def _hprev(M, K, seed):
 @pytest.mark.parametrize("M", [129, 5000])
 @pytest.mark.parametrize("N,K", [(96, 256), (89, 256), (256, 1024), (1024, 256)])
 def test_linear_dgrad_split(ops, M, N, K):
-    """rlppo_linear_dgrad_split, make_split(2,2,2,2, d_ps, pad64(N), d_ps) as backward_hidden / head_backward pass it:
+    """rlppo_linear_dgrad, make_split(2,2,2,2, d_ps, pad64(N), d_ps) as backward_hidden / head_backward pass it:
     dX = (dY W) (.) (hprev > 0), hprev a 3-part ReLU output whose mask is read from part 0; db_below += fp64 column sums of
     the reconstructed f32 dX.  N = 96 is the head's out_pad; N = 89 a contraction that is not a multiple of 8 (its
     padding columns in dY and W^T must be zero).  Masked entries are +0 in both parts."""
@@ -406,7 +406,7 @@ def test_linear_dgrad_split(ops, M, N, K):
 @pytest.mark.parametrize("M", [129, 5000])
 @pytest.mark.parametrize("N,K,a_ps", [(1024, 89, 1024), (256, 89, 1024), (90, 256, 128)])
 def test_linear_wgrad_split(ops, M, N, K, a_ps):
-    """rlppo_linear_wgrad_split, make_split(2,2,2,1, a_pstride, b_pstride) with a_pstride != b_pstride, as
+    """rlppo_linear_wgrad, make_split(2,2,2,1, a_pstride, b_pstride) with a_pstride != b_pstride, as
     backward_hidden passes it for hidden widths (1024, 256) and K = 89 (d_ps = pad64(max(hidden)) = 1024 against
     pad64(K)), and as head_backward passes it for 90 logits (pad64(90) against pad64(256)).  dW and db start nonzero and
     are accumulated into; db is the column sum of ALL parts of dY."""
@@ -470,7 +470,7 @@ def _prob_bound(z64, zabs, A):
 
 @pytest.mark.parametrize("A", [1, 2, 21, 90, 128, 256])
 def test_policy_head_sample_split(ops, A):
-    """rlppo_policy_head_sample_split, schedule (3,3,3,1) (Stack.policy_head_sample in "fp32" mode): probs against the
+    """rlppo_policy_head_sample, schedule (3,3,3,1) (Stack.policy_head_sample in "fp32" mode): probs against the
     fp64 softmax of the fp64 logits within _prob_bound (measured on a B200: at most 0.15 of it), log-prob of the drawn
     action against log(clamp(p64[a])), actions against O.sample_inverse_cdf on the fp64 probabilities -- a differing row
     must have u * P within the fp32 CDF's error of a CDF boundary -- and the deterministic per-row argmax."""
@@ -567,7 +567,7 @@ def _check_train(ops, M, K, A, scale, split):
 
 @pytest.mark.parametrize("A", [21, 90, 256])
 def test_policy_head_train_split(ops, A):
-    """rlppo_policy_head_train_split, schedule (3,3,3,2): dz (2 parts) against fp64 autograd of the PPO loss block.
+    """rlppo_policy_head_train, schedule (3,3,3,2): dz (2 parts) against fp64 autograd of the PPO loss block.
     Bound rel-L2 <= 3e-5: the 2-part output keeps 16 bits (2^-16 per element), and __expf / __logf (a few ulp, 2^-21.4
     absolute for __logf near 1) move s and log p by ~1e-6 relative.  Measured on a B200: 2.5e-6.  logp_out within
     _prob_bound's eps plus logf's rounding; metrics [0..4] against the fp64 means."""
@@ -605,7 +605,7 @@ def test_policy_head_train_saturated_logits(ops, split):
 
 @pytest.mark.parametrize("M,K", [(129, 256), (1000, 1024)])
 def test_value_head_split(ops, M, K):
-    """rlppo_value_head_split: H in 3 parts (fp32-exact), dH written as 2 parts, targets given.  Bounds (rigorous, from
+    """rlppo_value_head: H in 3 parts (fp32-exact), dH written as 2 parts, targets given.  Bounds (rigorous, from
     the kernel's summation order: K/256 chunks of 8 fused multiply-adds per lane, a 5-level warp tree, + b):
       |v - v64| <= (8 K/256 + 6) u (sum_k |h w| + |b|);
       dv = 2 inv (v - t): |dv - dv64| <= 2 inv (|v - v64| + u |v - t|) + 2 u |dv| (inv is passed as f32);
@@ -671,7 +671,7 @@ DISC = _subsets(("d_logp", "d_ent", "d_probs"))
 @pytest.mark.parametrize("split", [False, True], ids=["bf16", "split"])
 @pytest.mark.parametrize("given", DISC, ids=[_sid(s) for s in DISC])
 def test_policy_head_backward_subsets(ops, given, split, M, saturated):
-    """rlppo_policy_head_backward[_split] with every subset of (d_logp, d_ent, d_probs), the rest NULL (actions NULL too
+    """rlppo_policy_head_backward with every subset of (d_logp, d_ent, d_probs), the rest NULL (actions NULL too
     when d_logp is): dz against fp64 autograd of [log p[a], mean entropy, softmax] (clamp then log) with zeros for the
     missing gradients.  dz is written over more columns than the head has (128 for 90 logits); those come out zero.
 
@@ -825,7 +825,7 @@ def test_head_continuous_backward_subsets(ops, given, dz_parts, M, saturated):
 @pytest.mark.parametrize("M", [1, 129])
 @pytest.mark.parametrize("split", [False, True], ids=["bf16", "split"])
 def test_value_head_backward(ops, split, M, with_db):
-    """rlppo_value_head_backward[_split]: dH = dv w (.) (H > 0), dw += sum dv H, db += sum dv (db optional).  d_values
+    """rlppo_value_head_backward: dH = dv w (.) (H > 0), dw += sum dv H, db += sum dv (db optional).  d_values
     is the head's only upstream gradient and is required (NULL is an argument error).  Bounds: dH is one f32 product
     rounded to the output's parts (2^-9 bf16 / 2^-16 + u for 2 parts); dw and db are sums of M exact-input terms:
     M u (rigorous).  H carries tiny positives and -0.0; the split dH's columns between K and its part stride stay
