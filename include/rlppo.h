@@ -79,6 +79,16 @@ int rlppo_gae_compose_carry(const double* summaries, int rank, int world, double
 int rlppo_welford_update(float* mean, float* m2, int64_t* count, const void* samples, int samples_are_f64,
                          int64_t n, int dim, float* std_out, float* mean_out, void* stream);
 
+/* Merge of Welford states (running_stats.py:71-98, increment_from_serialized_other): folds n_others states into
+ * (mean, m2, count) in order, bit for bit the host formula applied other after other: f32 round-to-nearest, no
+ * contraction, counts converted to f32 as NumPy 2 converts a Python int (via double), mean (c*mu + c'*mu')/C and
+ * m2 + m2' + ((delta^2*c)*c')/C; an other with count 0 is skipped.  Other i is the block at
+ * others + i*other_stride_bytes laid out as [count i64 | mean f32[dim] | m2 f32[dim] | ...] (the device state of
+ * WelfordRunningStat), so blocks all-gathered from data-parallel ranks merge in place; stride % 8 == 0.  Writes
+ * std_out / mean_out as rlppo_welford_update does.  Any dim >= 1; one block, no host synchronisation, graph-capturable. */
+int rlppo_welford_merge(float* mean, float* m2, int64_t* count, const void* others, int64_t other_stride_bytes,
+                        int n_others, int dim, float* std_out, float* mean_out, void* stream);
+
 /* ---- (c-1) ExperienceBuffer store: rlgym_ppo/ppo/experience_buffer.py:17-37,54-80 -----------------
  * The FIFO `_cat` as a ring: logical row i lives at physical row (start+i) % capacity.  The host keeps
  * (start,size); these kernels move rows.  rlppo_ring_append copies n_rows rows of `src` (row-major,

@@ -37,6 +37,7 @@ _SIGS = {
     "rlppo_gae_chunk_summary": ([_P, _P, _P, _I, _P, _L, _D, _D, _P, _P, _P, _SZ, _P], _I),
     "rlppo_gae_compose_carry": ([_P, _I, _I, _P, _P], _I),
     "rlppo_welford_update": ([_P, _P, _P, _P, _I, _L, _I, _P, _P, _P], _I),
+    "rlppo_welford_merge": ([_P, _P, _P, _P, _L, _I, _I, _P, _P, _P], _I),
     "rlppo_ring_append": ([_P, _L, _P, _L, _L, _L, _P, _I, _L, _L, _I, _P], _I),
     "rlppo_ring_append_fields": ([_P, _I, _L, _L, _L, _P], _I),
     "rlppo_ring_append_fields_dev": ([_P, _I, _L, _P, _L, _P], _I),

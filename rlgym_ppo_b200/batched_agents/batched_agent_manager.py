@@ -38,7 +38,7 @@ from .wire import WireConn
 
 class BatchedAgentManager(object):
     def __init__(self, policy, min_inference_size=8, seed=123, standardize_obs=True, steps_per_obs_stats_increment=5,
-                 device=None):
+                 device=None, keep_obs_delta=False):
         self.policy = policy
         self.seed = seed
         self.processes = []
@@ -49,6 +49,10 @@ class BatchedAgentManager(object):
         self.steps_per_obs_stats_increment = steps_per_obs_stats_increment
         self.steps_since_obs_stats_update = 0
         self.obs_stats = None
+        # data-parallel Learner: obs_delta is a second Welford state fed the same samples as obs_stats, holding the
+        # increments since the ranks last merged their statistics (Learner resets it after every merge)
+        self.keep_obs_delta = keep_obs_delta
+        self.obs_delta = None
         self.ep_rews = []
         self.n_procs = 0
         self.device = device
@@ -110,11 +114,18 @@ class BatchedAgentManager(object):
         if self.standardize_obs:
             # NB the reference builds WelfordRunningStat(shape=obs) and seeds it with the reset observations (:377-380)
             self.obs_stats = WelfordRunningStat(self.obs_dim, device=self.device)
+            if self.keep_obs_delta:
+                self.obs_delta = WelfordRunningStat(self.obs_dim, device=self.device)
             for o in first:
-                self.obs_stats.increment(o, o.shape[0])
+                self._increment_obs_stats(o)
         self.processes[0][1].send(("shapes",))
         _, obs_size, n_acts, space_type = self._recv(self.processes[0][1], "shapes")
         return obs_size, n_acts, space_type
+
+    def _increment_obs_stats(self, o):
+        self.obs_stats.increment(o, o.shape[0])
+        if self.obs_delta is not None:
+            self.obs_delta.increment(o, o.shape[0])
 
     @staticmethod
     def _recv(conn, expect):
@@ -216,7 +227,7 @@ class BatchedAgentManager(object):
             if self.standardize_obs:                      # :303-315 (per response)
                 self.steps_since_obs_stats_update += 1
                 if self.steps_since_obs_stats_update > self.steps_per_obs_stats_increment:
-                    self.obs_stats.increment(o, o.shape[0])
+                    self._increment_obs_stats(o)
                     self.steps_since_obs_stats_update = 0
                     self._stats_dirty = True
             in_flight.discard(pid)

@@ -52,6 +52,56 @@ __global__ void welford_kernel(float* mean, float* m2, int64_t* count, const voi
     if (j == 0) *count = c;  // single block when dim <= 1024 (checked on the host)
 }
 
+// A count next to an f32 array, as NumPy 2 converts a Python int there: to double, then to float.
+__device__ __forceinline__ float count_to_f32(int64_t c) { return __double2float_rn(__ll2double_rn(c)); }
+
+// Chan's parallel merge of n_others Welford states into (mean, m2, count), others applied in order: the reference's
+// increment_from_serialized_other (running_stats.py:71-98) with its evaluation order, f32 round-to-nearest throughout.
+// Other i is the block at others + i * stride: [count i64 | mean f32[dim] | m2 f32[dim] | ...].  One block; threads
+// stride over dim.
+__global__ void welford_merge_kernel(float* mean, float* m2, int64_t* count, const unsigned char* __restrict__ others,
+                                     int64_t stride, int n_others, int dim, float* std_out, float* mean_out) {
+    const int64_t c0 = *count;
+    int64_t c = c0;
+    for (int j = threadIdx.x; j < dim; j += blockDim.x) {
+        float mu = mean[j], s2 = m2[j];
+        c = c0;
+        for (int i = 0; i < n_others; ++i) {
+            const unsigned char* blk = others + (int64_t)i * stride;
+            const int64_t oc = *reinterpret_cast<const int64_t*>(blk);
+            if (oc == 0) continue;
+            const float omu = reinterpret_cast<const float*>(blk + 8)[j];
+            const float os2 = reinterpret_cast<const float*>(blk + 8)[dim + j];
+            const int64_t cn = c + oc;
+            const float fc = count_to_f32(c), fo = count_to_f32(oc), fn = count_to_f32(cn);
+            const float delta = __fsub_rn(omu, mu);
+            const float d2 = __fmul_rn(delta, delta);
+            const float mu_n = __fdiv_rn(__fadd_rn(__fmul_rn(fc, mu), __fmul_rn(fo, omu)), fn);
+            s2 = __fadd_rn(__fadd_rn(s2, os2), __fdiv_rn(__fmul_rn(__fmul_rn(d2, fc), fo), fn));
+            mu = mu_n;
+            c = cn;
+        }
+        mean[j] = mu;
+        m2[j] = s2;
+        if (std_out) {  // as welford_kernel
+            float sd = 1.f;
+            if (c >= 2) {
+                float var = __fdiv_rn(s2, (float)(c - 1));
+                if (var == 0.f) var = 1.f;
+                sd = __fsqrt_rn(var);
+            }
+            std_out[j] = sd;
+        }
+        if (mean_out) mean_out[j] = (c >= 2) ? mu : 0.f;
+    }
+    __syncthreads();  // every thread has read *count
+    if (threadIdx.x == 0) {
+        c = c0;
+        for (int i = 0; i < n_others; ++i) c += *reinterpret_cast<const int64_t*>(others + (int64_t)i * stride);
+        *count = c;
+    }
+}
+
 // ---- ring append ----------------------------------------------------------------------------------------
 template <bool F64>
 __global__ void ring_append_kernel(float* ring, int64_t ring_ld, uint16_t* ring_bf16, int64_t bf16_ld,
@@ -338,6 +388,21 @@ int rlppo_welford_update(float* mean, float* m2, int64_t* count, const void* sam
         welford_kernel<true><<<1, threads, 0, s>>>(mean, m2, count, samples, n, dim, std_out, mean_out);
     else
         welford_kernel<false><<<1, threads, 0, s>>>(mean, m2, count, samples, n, dim, std_out, mean_out);
+    RLPPO_LAUNCH_CHECK();
+    return RLPPO_OK;
+}
+
+int rlppo_welford_merge(float* mean, float* m2, int64_t* count, const void* others, int64_t other_stride_bytes,
+                        int n_others, int dim, float* std_out, float* mean_out, void* stream) {
+    RLPPO_REQUIRE_DEVICE();
+    RLPPO_CHECK_ARG(mean && m2 && count && (others || n_others == 0), "null pointer");
+    RLPPO_CHECK_ARG(dim >= 1 && n_others >= 0, "dim must be >= 1 and n_others >= 0");
+    RLPPO_CHECK_ARG(n_others == 0 || (other_stride_bytes >= 8 + 8 * (int64_t)dim && other_stride_bytes % 8 == 0 &&
+                                      (reinterpret_cast<uintptr_t>(others) & 7) == 0),
+                    "other blocks: stride must hold [count | mean | m2] and keep the i64 counts 8-byte aligned");
+    const int threads = (int)min((int64_t)1024, ((int64_t)dim + 31) / 32 * 32);
+    welford_merge_kernel<<<1, threads, 0, static_cast<cudaStream_t>(stream)>>>(
+        mean, m2, count, static_cast<const unsigned char*>(others), other_stride_bytes, n_others, dim, std_out, mean_out);
     RLPPO_LAUNCH_CHECK();
     return RLPPO_OK;
 }

@@ -23,7 +23,7 @@ from typing import Tuple, Union
 import numpy as np
 import torch
 
-from . import _lib, ops
+from . import _lib, ops, parallel
 from ._graphs import GraphCache
 from ._staging import Stager
 from .ppo import ExperienceBuffer, PPOLearner
@@ -88,11 +88,17 @@ class Learner(object):
             random_seed: int = 123,
             n_checkpoints_to_keep: int = 5,
             shm_buffer_size: int = 8192,
-            device: str = "auto"):
+            device: str = "auto",
+            data_parallel: bool = False):
         assert (
                 env_create_function is not None
         ), "MUST PROVIDE A FUNCTION TO CREATE RLGYM FUNCTIONS TO INITIALIZE RLGYM-PPO"
 
+        # data_parallel: one Learner per GPU under torchrun, trained as one (weak scaling, see INTEGRATION.md).  At world
+        # size 1 nothing below differs from data_parallel=False.
+        self._owns_group, local_rank = parallel.init_torchrun() if data_parallel else (False, None)
+        self.world_size, self.rank = parallel.world() if data_parallel else (1, 0)
+        self.data_parallel = self.world_size > 1
         if checkpoints_save_folder is None:
             checkpoints_save_folder = os.path.join("data", "checkpoints", "rlgym-ppo-run")
         self.add_unix_timestamp = add_unix_timestamp
@@ -110,6 +116,10 @@ class Learner(object):
         self.standardize_returns = standardize_returns
         self.save_every_ts = save_every_ts
         self.ts_since_last_save = 0
+        if self.data_parallel:
+            # one run: rank 0's save folder, and the checkpoint rank 0 resolves "latest" to, on every rank
+            self.checkpoints_save_folder, checkpoint_load_folder = parallel.agree_on_folders(
+                checkpoints_save_folder, checkpoint_load_folder, self._latest_checkpoint)
 
         # There is no CPU learner here: "auto"/"gpu" pick the current CUDA device, anything else must name one.
         _lib.require_device()
@@ -119,6 +129,8 @@ class Learner(object):
             self.device = device
         else:
             raise _lib.RlppoError(f"device {device!r}: rlgym_ppo_b200 runs on a B200 only (no CPU fallback)")
+        if local_rank is not None and torch.device(self.device).index not in (None, local_rank):
+            raise _lib.RlppoError(f"device {device!r}: a data-parallel rank runs on its torchrun GPU, cuda:{local_rank}")
         print(f"Using device {self.device}")
 
         self.exp_buffer_size = exp_buffer_size
@@ -129,17 +141,20 @@ class Learner(object):
         self.return_stats = WelfordRunningStat(1, device=self.device)
         self.epoch = 0
 
-        self.experience_buffer = ExperienceBuffer(self.exp_buffer_size, seed=random_seed, device=self.device)
+        env_seed, buffer_seed = (parallel.rank_seeds(random_seed, self.rank, n_proc) if self.data_parallel
+                                 else (random_seed, random_seed))
+        self.experience_buffer = ExperienceBuffer(self.exp_buffer_size, seed=buffer_seed, device=self.device)
 
         print("Initializing processes...")
         from .batched_agents import BatchedAgentManager
         collect_metrics_fn = None if metrics_logger is None else self.metrics_logger.collect_metrics
         self.agent = BatchedAgentManager(
             None, min_inference_size=min_inference_size,
-            seed=random_seed,
+            seed=env_seed,
             standardize_obs=standardize_obs,
             steps_per_obs_stats_increment=steps_per_obs_stats_increment,
             device=self.device,
+            keep_obs_delta=self.data_parallel,
         )
         obs_space_size, act_space_size, action_space_type = self.agent.init_processes(
             n_processes=n_proc,
@@ -170,7 +185,12 @@ class Learner(object):
             critic_lr=critic_lr,
             clip_range=ppo_clip_range,
             ent_coef=ppo_ent_coef,
+            **(dict(process_group=torch.distributed.group.WORLD, dp_mode="sharded") if self.data_parallel else {}),
         )
+        if self.data_parallel:
+            # after the nets are built, so that the initial weights do not depend on the rank
+            policy = self.ppo_learner.policy
+            policy._seed = parallel.sampler_seed(policy._seed, self.rank)
 
         self.agent.policy = self.ppo_learner.policy
 
@@ -182,11 +202,15 @@ class Learner(object):
             "ppo_batch_size", "ppo_minibatch_size", "ppo_ent_coef", "ppo_clip_range", "gae_lambda", "gae_gamma",
             "policy_lr", "critic_lr", "shm_buffer_size")}
 
-        self.wandb_run = wandb_run
-        wandb_loaded = checkpoint_load_folder is not None and self.load(checkpoint_load_folder, load_wandb, policy_lr,
+        self.wandb_run = wandb_run if self.rank == 0 else None
+        self._obs_loaded = False
+        wandb_loaded = checkpoint_load_folder is not None and self.load(checkpoint_load_folder,
+                                                                        load_wandb and self.rank == 0, policy_lr,
                                                                         critic_lr)
+        if self.data_parallel:
+            self._start_replicas()
 
-        if log_to_wandb and self.wandb_run is None and not wandb_loaded:
+        if log_to_wandb and self.rank == 0 and self.wandb_run is None and not wandb_loaded:
             import wandb
             print("Attempting to create new wandb run...")
             self.wandb_run = wandb.init(project=wandb_project_name or "rlgym-ppo",
@@ -208,6 +232,24 @@ class Learner(object):
                 group["lr"] = lr
             print(f"New {label} learning rate: {lr}")
 
+    def _start_replicas(self):
+        """Data parallel: every rank starts from rank 0's parameter arena, Adam moments and step counters (after any
+        checkpoint load), and from the same observation statistics: the loaded ones, else none (the increments each rank
+        made so far, its reset observations, are in its delta and enter the first merge)."""
+        import torch.distributed as dist
+        ppo = self.ppo_learner
+        for t in (ppo._params, ppo._m, ppo._v, ppo._steps):
+            dist.broadcast(t, src=0)
+        ppo.policy._stack.refresh_operands(force=True)
+        ppo.value_net._stack.refresh_operands(force=True)
+        self._obs_base = None
+        if self.agent.standardize_obs:
+            self._obs_base = WelfordRunningStat(self.agent.obs_stats.shape, device=self.device)
+            if self._obs_loaded:
+                self._obs_base.copy_device_(self.agent.obs_stats)
+                self.agent.obs_delta.reset()
+        self._t_exchange = None
+
     def learn(self):
         """Run iterations until the timestep limit; on an exception print it, try to checkpoint, and always release the
         workers (the contract of learner.py:218-238)."""
@@ -227,6 +269,8 @@ class Learner(object):
     def _iteration(self):
         """collect -> add_new_experience -> PPOLearner.learn -> report.  Returns the number of steps collected."""
         from .util import reporting
+        if self.data_parallel:
+            return self._iteration_dp()
         t_start = time.perf_counter()
         experience, env_metrics, n_steps, t_collect = self.agent.collect_timesteps(self.ts_per_epoch)
         if self.metrics_logger is not None:
@@ -250,6 +294,56 @@ class Learner(object):
         reporting.report_metrics(loggable_metrics=report, debug_metrics=None, wandb_run=self.wandb_run)
         return n_steps
 
+    def _iteration_dp(self):
+        """collect -> exchange -> merge of the observation statistics -> add_new_experience -> learn -> report (rank 0).
+        Returns the number of steps collected by all ranks.
+
+        The exchange is one all-gather of every rank's observation-statistics delta and collection tail.  It comes before
+        add_new_experience, whose first call holds a collective of its own, and a rank whose collection raised still takes
+        part (with its error flag set): every rank issues the same collectives in the same order, and all of them leave
+        the loop together when any rank failed."""
+        from .util import reporting
+        t_start = time.perf_counter()
+        cum0 = self.agent.cumulative_timesteps
+        error, experience, env_metrics, n_steps, t_collect = None, None, [], 0, 0.0
+        try:
+            experience, env_metrics, n_steps, t_collect = self.agent.collect_timesteps(self.ts_per_epoch)
+        except Exception as e:  # noqa: BLE001  (re-raised below, after the exchange)
+            error, t_collect = e, time.perf_counter() - t_start
+        t_x = time.perf_counter()
+        delta = self.agent.obs_delta
+        block = delta.device_block() if delta is not None else torch.empty(0, dtype=torch.uint8, device=self.device)
+        blocks, stride, tails = parallel.exchange(
+            block, parallel.pack_tail(n_steps, t_collect, self.agent.average_reward, error is not None))
+        agg = parallel.combine_tails(tails)
+        if agg["failed"]:
+            self.agent.cumulative_timesteps = cum0
+            if error is not None:
+                raise error
+            raise RuntimeError(f"environment collection failed on data-parallel rank(s) {agg['failed']}")
+        if delta is not None:
+            # base <- base + every rank's increments, in rank order; the base becomes every rank's working statistics
+            self._obs_base.merge_device(blocks, self.world_size, stride)
+            self.agent.obs_stats.copy_device_(self._obs_base)
+            delta.reset()
+        torch.cuda.current_stream().synchronize()
+        self._t_exchange = time.perf_counter() - t_x
+        self.agent.cumulative_timesteps = cum0 + agg["steps"]
+        if self.metrics_logger is not None:
+            metrics = parallel.gather_metrics(env_metrics)
+            if self.rank == 0:
+                self.metrics_logger.report_metrics(metrics, self.wandb_run, self.agent.cumulative_timesteps)
+        self.add_new_experience(experience)
+        report = dict(self.ppo_learner.learn(self.experience_buffer))
+        if self.rank == 0:
+            if self.epoch < 1:
+                report["Value Function Loss"] = np.nan
+            report["Cumulative Timesteps"] = self.agent.cumulative_timesteps
+            report["Total Iteration Time"] = t_total = time.perf_counter() - t_start
+            report.update(parallel.collection_report(agg, t_total))
+            reporting.report_metrics(loggable_metrics=report, debug_metrics=None, wandb_run=self.wandb_run)
+        return agg["steps"]
+
     def _poll_keys(self, kb):
         """p = pause until a key, c = checkpoint, q = checkpoint and stop.  Returns True when the loop should end."""
         if not kb.kbhit():
@@ -269,11 +363,14 @@ class Learner(object):
 
     def _learn(self):
         from .util.kbhit import KBHit
-        kb = KBHit()   # guarded: no-op without a TTY (gpurun / CI)
-        print("Press (p) to pause (c) to checkpoint, (q) to checkpoint and quit (after next iteration)\n")
+        kb = None
+        if not self.data_parallel:     # data parallel: the ranks take every loop decision together, so no keys
+            kb = KBHit()   # guarded: no-op without a TTY (gpurun / CI)
+            print("Press (p) to pause (c) to checkpoint, (q) to checkpoint and quit (after next iteration)\n")
+        # data parallel: cumulative_timesteps, timestep_limit and save_every_ts count the steps of all ranks
         while self.agent.cumulative_timesteps < self.timestep_limit:
             self.ts_since_last_save += self._iteration()
-            if self._poll_keys(kb):
+            if kb is not None and self._poll_keys(kb):
                 return
             if self.ts_since_last_save >= self.save_every_ts:
                 self.save(self.agent.cumulative_timesteps)
@@ -497,7 +594,9 @@ class Learner(object):
             "reward_running_stats": self.return_stats.to_json(),
         }
         if self.agent.standardize_obs:
-            bk["obs_running_stats"] = self.agent.obs_stats.to_json()
+            # data parallel: the merged statistics of all ranks
+            obs_stats = self._obs_base if self.data_parallel else self.agent.obs_stats
+            bk["obs_running_stats"] = obs_stats.to_json()
         run = self.wandb_run
         if run is not None:
             bk.update(wandb_run_id=run.id, wandb_project=run.project, wandb_entity=run.entity, wandb_group=run.group,
@@ -505,6 +604,8 @@ class Learner(object):
         return bk
 
     def save(self, cumulative_timesteps):
+        if self.rank != 0:       # data parallel: rank 0 writes the run's checkpoints
+            return
         root = self.checkpoints_save_folder
         target = os.path.join(root, str(cumulative_timesteps))
         os.makedirs(target, exist_ok=True)
@@ -567,6 +668,7 @@ class Learner(object):
         if self.agent.standardize_obs and "obs_running_stats" in bk:
             self.agent.obs_stats = WelfordRunningStat(1, device=self.device)
             self.agent.obs_stats.from_json(bk["obs_running_stats"])
+            self._obs_loaded = True
         if new_policy_lr is not None or new_critic_lr is not None:
             self.update_learning_rate(new_policy_lr, new_critic_lr)
         resumed = False
@@ -586,3 +688,7 @@ class Learner(object):
         if agent is not None and hasattr(agent, "cleanup"):
             agent.cleanup()
         self.experience_buffer.clear()
+        if self._owns_group:
+            import torch.distributed as dist
+            dist.destroy_process_group()
+            self._owns_group = False

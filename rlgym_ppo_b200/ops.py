@@ -98,6 +98,15 @@ def welford_update(mean, m2, count, samples, n, std_out=None, mean_out=None):
          int(n), dim, ptr(std_out), ptr(mean_out), stream_ptr())
 
 
+def welford_merge(mean, m2, count, others, n_others, stride_bytes, std_out=None, mean_out=None):
+    """Fold n_others Welford states (blocks [count i64 | mean f32[dim] | m2 f32[dim] | ...], stride_bytes apart, starting
+    at the device tensor `others`) into (mean, m2, count), in order (rlppo_welford_merge)."""
+    assert count.dtype == torch.int64 and others.is_cuda and others.is_contiguous()
+    assert others.numel() * others.element_size() >= int(n_others) * int(stride_bytes), "others too small"
+    call("rlppo_welford_merge", ptr(mean), ptr(m2), ptr(count), ptr(others), int(stride_bytes), int(n_others),
+         mean.numel(), ptr(std_out), ptr(mean_out), stream_ptr())
+
+
 # ---- ring / gather --------------------------------------------------------------------------------------
 def ring_append(ring, phys_first, src, n_rows, ring_bf16=None):
     cap = ring.shape[0]

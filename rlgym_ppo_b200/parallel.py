@@ -4,6 +4,9 @@ GPUs, gloo in the CPU tests).  No tensor math here beyond the collectives themse
 The reference has no distributed mode (SURVEY.md 2.2); the seam is its gradient accumulation over minibatch slices
 (ppo_learner.py:134-193), which sums (mb/B)-scaled minibatch gradients before ONE clip + Adam step.
 """
+import os
+
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -87,3 +90,102 @@ def report_from_sums(sums):
     rows_v = s[6] if s[6] > 0 else 1.0
     return {"Policy Entropy": s[0] / rows_p, "Mean KL Divergence": s[1] / rows_p, "SB3 Clip Fraction": s[2] / rows_p,
             "Value Function Loss": s[5] / rows_v}
+
+
+# ---- Learner(data_parallel=True): one learner on every GPU of a box, one process per GPU under torchrun -----------------
+# Each rank collects its own rollouts (weak scaling, dp_mode="sharded").  Once per iteration the ranks exchange, in ONE
+# all-gather, their observation-statistics increments (a Welford device block) and a small f64 tail:
+TAIL = ("steps", "collect_time", "average_reward", "has_reward", "error")
+
+
+def init_torchrun():
+    """(created, local_rank): joins the process group of a torchrun launch.  An initialised group is used as it is
+    (created = False); without one, NCCL is initialised from the torchrun environment.  Without a torchrun environment
+    there is one process: (False, None).  The current CUDA device becomes cuda:LOCAL_RANK whenever LOCAL_RANK is set."""
+    local = os.environ.get("LOCAL_RANK")
+    local = None if local is None else int(local)
+    if local is not None:
+        torch.cuda.set_device(local)
+    if dist.is_available() and dist.is_initialized():
+        return False, local
+    if local is None or "WORLD_SIZE" not in os.environ:
+        return False, None
+    dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    return True, local
+
+
+def rank_seeds(random_seed, rank, n_proc):
+    """(environment seed base, experience-buffer seed) of `rank`: its workers are seeded base + proc_id, i.e.
+    random_seed + rank * n_proc + proc_id, and its buffer random_seed + rank.  Rank 0 keeps the single-process seeds."""
+    return random_seed + rank * n_proc, random_seed + rank
+
+
+def sampler_seed(seed, rank):
+    """Key of `rank`'s policy sampler (Philox) from the key every rank drew: rank 0 keeps it, the others mix in their
+    rank so that no two ranks sample the same action stream."""
+    if rank == 0:
+        return seed
+    return (seed ^ (rank * 0x9E3779B97F4A7C15)) % (1 << 62)
+
+
+def pack_tail(steps, collect_time, average_reward, error):
+    """This rank's f64 tail (TAIL order); average_reward None (no episode finished yet) is sent as has_reward = 0."""
+    has = average_reward is not None
+    return np.array([steps, collect_time, average_reward if has else 0.0, float(has), float(bool(error))], np.float64)
+
+
+def combine_tails(tails):
+    """tails f64 [world, len(TAIL)] in rank order -> what every rank acts on: the global step count, the slowest
+    collection, the mean of the ranks' average rewards (None when no rank has one), the ranks that failed."""
+    t = np.asarray(tails, np.float64).reshape(-1, len(TAIL))
+    rew = t[t[:, 3] != 0, 2]
+    return {"steps": int(round(t[:, 0].sum())), "collect_time": float(t[:, 1].max()),
+            "average_reward": float(rew.mean()) if len(rew) else None,
+            "failed": [int(r) for r in np.flatnonzero(t[:, 4] != 0)]}
+
+
+def collection_report(agg, total_time):
+    """The collection entries of the iteration report (learner.py:275-296) over all ranks: global steps over the slowest
+    rank's collection time, and over this rank's iteration time."""
+    steps, t_collect = agg["steps"], agg["collect_time"]
+    return {"Timesteps Collected": steps, "Timestep Collection Time": t_collect,
+            "Timestep Consumption Time": total_time - t_collect,
+            "Collected Steps per Second": steps / t_collect if t_collect > 0 else float("nan"),
+            "Overall Steps per Second": steps / total_time if total_time > 0 else float("nan"),
+            "Policy Reward": np.nan if agg["average_reward"] is None else agg["average_reward"]}
+
+
+def exchange(block, tail, group=None):
+    """ONE all-gather of [block bytes | tail f64] from every rank.  block: uint8 tensor (8-byte multiple; may be empty) on
+    the collective's device; tail: f64 array.  Returns (gathered uint8 [world * stride], stride in bytes, tails f64
+    [world, len(tail)] on the host)."""
+    nb = int(block.numel())
+    assert block.dtype == torch.uint8 and nb % 8 == 0
+    tail = torch.from_numpy(np.ascontiguousarray(tail, np.float64))
+    stride = nb + 8 * int(tail.numel())
+    world = dist.get_world_size(group)
+    send = torch.empty(stride, dtype=torch.uint8, device=block.device)
+    send[:nb].copy_(block)
+    send[nb:].view(torch.float64).copy_(tail)
+    out = torch.empty(world * stride, dtype=torch.uint8, device=block.device)
+    dist.all_gather_into_tensor(out, send, group=group)
+    tails = out.view(world, stride)[:, nb:].contiguous().view(torch.float64).cpu().numpy()
+    return out, stride, tails
+
+
+def agree_on_folders(save_folder, load_folder, resolve_latest, group=None):
+    """Rank 0's checkpoint folders on every rank: its (time-stamped) save folder, and the folder to load, with "latest"
+    resolved by rank 0 (resolve_latest(); None when there is nothing to load)."""
+    if dist.get_rank(group) == 0 and load_folder == "latest":
+        load_folder = resolve_latest()
+    obj = [save_folder, load_folder]
+    dist.broadcast_object_list(obj, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
+    return obj[0], obj[1]
+
+
+def gather_metrics(metrics, group=None):
+    """Every rank's collected metrics, concatenated in rank order, on rank 0 (None on the others)."""
+    rank = dist.get_rank(group)
+    out = [None] * dist.get_world_size(group) if rank == 0 else None
+    dist.gather_object(metrics, out, dst=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
+    return [m for ms in out for m in ms] if rank == 0 else None

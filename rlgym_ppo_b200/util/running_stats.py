@@ -71,6 +71,23 @@ class WelfordRunningStat(object):
         dist.broadcast(d["raw"], src=src, group=group)
         self._dev_is_newer = True
 
+    def device_block(self):
+        """The device state as one uint8 block [count i64 | mean f32[dim] | m2 f32[dim] | std | mean_out], the layout
+        merge_device reads."""
+        return self._push()["raw"]
+
+    def merge_device(self, blocks, n, stride_bytes):
+        """Fold n device blocks (device_block layouts, stride_bytes apart in the tensor `blocks`) into these statistics in
+        order: increment_from_serialized_other applied to each, bit for bit, without leaving the device."""
+        d = self._push()
+        ops.welford_merge(d["mean"], d["m2"], d["count"], blocks, n, stride_bytes, d["std"], d["mean_out"])
+        self._dev_is_newer = True
+
+    def copy_device_(self, other):
+        """Make these statistics a copy of `other`'s (same dim), device to device."""
+        self._push()["raw"].copy_(other.device_block())
+        self._dev_is_newer = True
+
     def device_std(self):
         """f32[dim] device tensor holding `std` (running_stats.py:60-69); no host synchronisation."""
         return self._push()["std"]
