@@ -11,12 +11,17 @@ from .. import ops
 from ._head_policy import HeadPolicy
 from ._mlp import build_sequential, grad_f32
 
+MAX_ACTIONS = 32     # widest action space rlppo_head_continuous_* serve (2 * 32 network outputs)
+
 
 class ContinuousPolicy(HeadPolicy):
     def __init__(self, input_shape, output_shape, layer_sizes, device, var_min=0.1, var_max=1.0, precision=None):
         super().__init__()
         self.device = device
         assert int(output_shape) % 2 == 0, "ContinuousPolicy outputs a mean and a std per action"
+        if not 1 <= int(output_shape) // 2 <= MAX_ACTIONS:
+            raise ValueError(f"ContinuousPolicy supports 1 to {MAX_ACTIONS} actions, i.e. output_shape 2 to "
+                             f"{2 * MAX_ACTIONS} (got {int(output_shape)})")
         self.n_act = int(output_shape) // 2
         self.act_width = self.n_act
         self.var_min, self.var_max = float(var_min), float(var_max)

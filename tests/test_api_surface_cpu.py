@@ -40,3 +40,12 @@ def test_surface_matches_reference(path):
         assert got[:len(want)] == want, f"{path}.{name}: {got[:len(want)]} != {want}"
         for extra in got[len(want):]:
             assert extra[1] is not None, f"{path}.{name}: extra parameter {extra[0]} must be optional"
+
+
+@pytest.mark.parametrize("output_shape", [0, 66, 128])
+def test_continuous_policy_rejects_unsupported_widths(output_shape):
+    """ContinuousPolicy serves 1 to 32 actions (2 to 64 outputs): anything else is refused at construction, before any
+    device work, rather than by the kernel at the first call."""
+    from rlgym_ppo_b200.ppo import ContinuousPolicy
+    with pytest.raises(ValueError, match="1 to 32 actions"):
+        ContinuousPolicy(8, output_shape, (64,), "cuda:0")

@@ -48,6 +48,7 @@ import pytest
 import torch
 
 from oracle import ref_oracle as O
+from parity_helpers import philox_rows, philox_uniform
 from test_split_kernels_gpu import _prob_bound
 
 pytestmark = pytest.mark.gpu
@@ -705,6 +706,8 @@ def test_policy_infer_fused(ops, hidden, obs, A, M):
       deterministic: the argmax wherever the top-2 gap exceeds 2 zerr, log-prob of the row maximum.
       d_offset: a launch with offset o and a device counter advanced by rlppo_u64_add(c) draws exactly what a launch
         with offset o + c draws, and not what offset o alone draws.
+      Philox stream: with seed 0x0123456789ABCDEF and offset + device counter = 2^32 - M/2, the actions and log-probs
+        equal those drawn from the host restatement's uniforms (tests/parity_helpers.py), bit for bit.
     Nothing is written at row M.
     Measured on a B200: logp_out at most 0.287 of lp_tol; logit intervals up to 0.094 wide on the bench shape at
     M = 3000, where 16 of 1788 boundary rows sample differently from the fp64 reference (1 of 257 for (64, 64), 4 of 387
@@ -766,6 +769,17 @@ def test_policy_infer_fused(ops, hidden, obs, A, M):
     assert torch.equal(out[0][0], out[1][0]) and torch.equal(bits(out[0][1]), bits(out[1][1]))
     if A > 1 and M > 1:
         assert not torch.equal(out[0][0], out[2][0])
+    # the Philox stream (counter (offset + device offset + row, high word, 0, 0), key (seed lo, seed hi)): a launch whose
+    # rows cross the carry into the counter's high word draws exactly what the host restatement's uniforms draw
+    seed, first = 0x0123456789ABCDEF, 2 ** 32 - M // 2
+    u_host = torch.from_numpy(philox_uniform(philox_rows(seed, first, M)[:, 0])).float().to(DEV)
+    draws = []
+    for kw in (dict(seed=seed, offset=first - 12345, offset_dev=ctr), dict(u=u_host)):
+        a_, l_ = torch.empty(M, dtype=torch.int64, device=DEV), torch.empty(M, device=DEV)
+        ops.policy_infer_fused(s, x, M, A, actions_i64_out=a_, logp_out=l_, **kw)
+        draws.append((a_, l_))
+    torch.cuda.synchronize()
+    assert torch.equal(draws[0][0], draws[1][0]) and torch.equal(bits(draws[0][1]), bits(draws[1][1]))
 
 
 VINFER_CASES = [((256, 256, 256), 89, M) for M in (1, 129, 3000)] + [((128,), 20, 3000), ((64, 64), 89, 3000),

@@ -107,6 +107,28 @@ def test_mt19937_permutation_restatement(golden):
     assert np.array_equal(p1[:64], g["perm150000.head"]) and np.array_equal(p2[:64], g["perm150000.second_head"])
 
 
+def test_philox4x32_10_known_answers():
+    """The host Philox that the samplers' stream tests draw from, pinned to the Random123 known-answer vectors
+    (kat_vectors, philox4x32_10), all three evaluated in one vectorised call; the uniform is the top 24 bits."""
+    from parity_helpers import philox4x32_10, philox_rows, philox_uniform
+    ctr = np.array([[0, 0, 0, 0], [0xFFFFFFFF] * 4, [0x243F6A88, 0x85A308D3, 0x13198A2E, 0x03707344]], np.uint32)
+    key = np.array([[0, 0], [0xFFFFFFFF] * 2, [0xA4093822, 0x299F31D0]], np.uint32)
+    want = np.array([[0x6627E8D5, 0xE169C58D, 0xBC57AC4C, 0x9B00DBD8],
+                     [0x408F276D, 0x41C83B0E, 0xA20BC7C6, 0x6D5451FD],
+                     [0xD16CFE09, 0x94FDCCEB, 0x5001E420, 0x24126EA1]], np.uint32)
+    assert np.array_equal(philox4x32_10(ctr, key), want)
+    assert np.array_equal(philox_uniform(np.array([0, 0xFF, 0x100, 0xFFFFFFFF], np.uint32)),
+                          [0.0, 0.0, 2.0 ** -24, 1.0 - 2.0 ** -24])
+    # the launch layout: ctr = offset + row carries into the counter's second word; the key is (seed lo, seed hi)
+    r = philox_rows(0xA4093822299F31D0, (0x85A308D3 << 32) + 0x243F6A88 - 1, 2, word2=0x13198A2E)
+    assert r.shape == (2, 4)
+    r1 = philox4x32_10(np.array([0x243F6A88, 0x85A308D3, 0x13198A2E, 0], np.uint32),
+                       np.array([0x299F31D0, 0xA4093822], np.uint32))
+    assert np.array_equal(r[1], r1)
+    r = philox_rows(1, 0xFFFFFFFF, 2)
+    assert np.array_equal(r[1], philox4x32_10(np.array([0, 1, 0, 0], np.uint32), np.array([1, 0], np.uint32)))
+
+
 def test_policy_and_value_forward(golden):
     g = golden("policy")
     pol, val = _params(g, "pol"), _params(g, "val")

@@ -28,12 +28,11 @@ import pytest
 import torch
 
 from oracle import ref_oracle as O
+from parity_helpers import DEV, SENTINEL, bits, philox_rows, philox_uniform, recon, sentinel, split_rows
 
 pytestmark = pytest.mark.gpu
 
-DEV = "cuda:0"
 U = 2.0 ** -24
-SENTINEL = 0x7FC1          # a bf16 NaN: a stray write, or a read of unwritten padding, cannot go unnoticed
 
 
 @pytest.fixture(scope="module")
@@ -46,21 +45,6 @@ def ops():
 # ------------------------------------------------------------------------------------------------------------
 # helpers
 # ------------------------------------------------------------------------------------------------------------
-def sentinel(rows, cols):
-    return torch.full((rows, cols), SENTINEL, dtype=torch.int16, device=DEV).view(torch.bfloat16)
-
-
-def bits(t):
-    return t.view(torch.int16)
-
-
-def recon(buf, parts, pstride, cols, rows=None):
-    """fp64 sum of the parts of a split buffer (CPU), columns [0, cols)."""
-    b = buf if rows is None else buf[rows]
-    b = b.cpu()
-    return sum(b[:, q * pstride:q * pstride + cols].double() for q in range(parts))
-
-
 TAIL = 127 * 2.0 ** -15 + 63 * 2.0 ** -23
 
 
@@ -75,15 +59,6 @@ def tailed(shape, seed, positive, device="cpu"):
 
 def gemm_err(y, ref, absum):
     return float(((y - ref).abs() / absum).max())
-
-
-def split_rows(ops, x, parts, pstride, ld=None, rows=None):
-    """f32 CPU rows -> split bf16 device buffer [rows, ld]."""
-    n, w = x.shape
-    rows = n if rows is None else rows
-    buf = torch.zeros((rows, ld or parts * pstride), dtype=torch.bfloat16, device=DEV)
-    ops.rows_split(x.to(DEV).contiguous(), buf, parts, pstride)
-    return buf
 
 
 def split_weight(ops, w, q_parts, q_pstride, out_rows, t_parts=0, t_pstride=0, in_rows=0):
@@ -504,6 +479,17 @@ def test_policy_head_sample_split(ops, A):
     lp_ref = torch.log(pc.gather(-1, a.view(-1, 1))).flatten()
     lp_tol = float(eps.max()) + 2 * 2.0 ** -23 * max(1.0, float(lp_ref.abs().max()))     # + logf's rounding
     assert float((logp.cpu().double() - lp_ref).abs().max()) <= lp_tol
+    # the Philox stream (counter (offset + row, high word, 0, 0), key (seed lo, seed hi)): a launch whose rows cross the
+    # carry into the counter's high word draws exactly what the host restatement's uniforms draw when injected
+    seed, off = 0x0123456789ABCDEF, 2 ** 32 - M // 2
+    u_host = torch.from_numpy(philox_uniform(philox_rows(seed, off, M)[:, 0])).float().to(DEV)
+    draws = []
+    for kw in (dict(seed=seed, offset=off), dict(u=u_host)):
+        a_, l_ = torch.empty(M, dtype=torch.int64, device=DEV), torch.empty(M, device=DEV)
+        ops.policy_head_sample(hs, wq, b.to(DEV), A, K, actions_i64_out=a_, logp_out=l_, split=sp, **kw)
+        draws.append((a_, l_))
+    torch.cuda.synchronize()
+    assert torch.equal(draws[0][0], draws[1][0]) and torch.equal(draws[0][1].view(torch.int32), draws[1][1].view(torch.int32))
     ops.policy_head_sample(hs, wq, b.to(DEV), A, K, deterministic=True, actions_i64_out=acts, logp_out=logp, split=sp)
     torch.cuda.synchronize()
     top2 = z64.topk(min(2, A), -1).values

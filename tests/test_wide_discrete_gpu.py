@@ -8,7 +8,7 @@ import pytest
 import torch
 
 from oracle import ref_oracle as O
-from parity_helpers import capture_steps, close, rel_l2, unflatten
+from parity_helpers import capture_steps, close, philox_rows, philox_uniform, rel_l2, unflatten
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -110,6 +110,17 @@ def test_sample_probs_argmax_and_inverse_cdf(ops, A):
     got_lp = logp.double().cpu()[keep]
     want_lp = torch.log(p.gather(-1, want[:, None]).flatten())[keep]
     assert torch.allclose(got_lp, want_lp, rtol=0, atol=2e-5 * max(1.0, float(want_lp.abs().max())))
+    # the Philox stream (counter (offset + row, high word, 0, 0), key (seed lo, seed hi)): a launch whose rows cross the
+    # carry into the counter's high word draws exactly what the host restatement's uniforms draw when injected
+    seed, off = 0x0123456789ABCDEF, 2 ** 32 - M // 2
+    u_host = torch.from_numpy(philox_uniform(philox_rows(seed, off, M)[:, 0])).float().to(DEV)
+    draws = []
+    for kw in (dict(seed=seed, offset=off), dict(u=u_host)):
+        a_, l_ = torch.empty(M, dtype=torch.int64, device=DEV), torch.empty(M, device=DEV)
+        ops.head_discrete_sample(zbuf, 3, P, M, A, actions_i64_out=a_, logp_out=l_, **kw)
+        draws.append((a_, l_))
+    torch.cuda.synchronize()
+    assert torch.equal(draws[0][0], draws[1][0]) and torch.equal(draws[0][1].view(torch.int32), draws[1][1].view(torch.int32))
 
 
 def _ppo_reference(z, a, old, adv, inv_b, clip, ent_coef):
