@@ -193,9 +193,11 @@ int rlppo_weight_split_bf16(const float* w, int out_f, int in_f, uint16_t* wq, i
 int rlppo_linear_fwd(const uint16_t* x, int64_t ldx, const uint16_t* w, int64_t ldw, const float* bias, int bias_n,
                      uint16_t* y, int64_t ldy, int64_t M, int N, int K, int relu, const rlppo_split* sp, void* stream);
 /* rlppo_linear_dgrad: dX[M,K] = (dY[M,N] * W[N,K]) (.) (Hprev > 0); wt = bf16 W^T [K, ldwt>=N].
+ *   K >= 1 need not be a multiple of 8: dX is written over pad8(K) columns (lddx, ldh multiples of 8 covering
+ *   pad8(K)); wt rows past K are read as zeros, so dX's padding columns come out zero.
  *   hprev = the ReLU output that was this layer's input (bf16 [M,ldh]) or NULL (no mask).
- *   db_below (optional f32[K]) += column sums of the stored dX (= the bias gradient of the layer that produced Hprev,
- *   ppo_learner.py:179-180 autograd): saves that layer's separate column-sum pass over dX.
+ *   db_below (optional f32[K]) += column sums of the stored dX over its K true columns (= the bias gradient of the
+ *   layer that produced Hprev, ppo_learner.py:179-180 autograd): saves that layer's separate column-sum pass over dX.
  *   Split operands: the ReLU mask is read from part 0 of hprev (x > 0 <=> bf16(x) > 0); db_below sums the un-split f32
  *   values. */
 int rlppo_linear_dgrad(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int64_t ldwt, const uint16_t* hprev,
@@ -253,12 +255,14 @@ int rlppo_policy_head_train(const uint16_t* h, int64_t ldh, const uint16_t* w, i
                             const rlppo_split* sp, void* stream);
 
 /* Value head (ValueEstimator last Linear(.,1), value_estimator.py:27; MSELoss ppo_learner.py:176),
- * fused SIMT pass over the last hidden activation H[M,K] (bf16):
+ * fused SIMT pass over the last hidden activation H[M,K] (bf16), 1 <= K <= 28672:
  *   v = H*w + b  -> values_out f32[M] (if non-NULL).
  *   if targets != NULL: dv = 2*inv_batch*(v - target); dH[M,lddh] (bf16) = dv * w (.) (H > 0);
  *   dw[K] += sum_m dv*H;  db[1] += sum dv;  metrics[5] += sum (v-target)^2, metrics[6] += rows.
  *   H is given as h_parts split parts h_pstride columns apart and dH written as dh_parts parts dh_pstride apart
- *   (1..3 parts each, strides multiples of 8 covering K; plain bf16: 1, 0, 1, 0). */
+ *   (1..3 parts each, strides multiples of 8 covering pad8(K); plain bf16: 1, 0, 1, 0).  H and dH rows span pad8(K)
+ *   columns (ldh, lddh multiples of 8 covering it): H's columns K..pad8(K)-1 must be zero, dH's are written as zeros;
+ *   w and dw hold exactly K floats.  K > 2048 runs a second kernel form (w and the dw partials in shared memory). */
 int rlppo_value_head(const uint16_t* h, int64_t ldh, const float* w, const float* bias, int64_t M, int K,
                      float* values_out, const float* targets, float inv_batch, uint16_t* dh, int64_t lddh,
                      float* dw, float* db, float* metrics, int h_parts, int64_t h_pstride, int dh_parts,

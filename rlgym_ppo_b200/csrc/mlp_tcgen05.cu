@@ -148,7 +148,9 @@ struct RowGemmParams {
     int relu;
     const uint16_t* mask;
     int64_t ldmask;
-    float* colsum;   // EPI_RELU_MASK: optional f32[N], += column sums of the bf16 output (= bias gradient of the layer below)
+    float* colsum;   // EPI_RELU_MASK: optional f32[colsum_n], += column sums of the bf16 output (= bias gradient of the
+                     // layer below)
+    int colsum_n;    // entries of `colsum` (<= N: the output's padding columns past it have no bias entry)
     // heads
     int n_actions;
     const float* actions;
@@ -708,7 +710,7 @@ rowgemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     for (int j = et; j < BLOCK_N; j += 128) {
                         const float cs = s_bias[j];
                         s_bias[j] = 0.f;
-                        if (n0 + j < p.N && cs != 0.f) atomicAdd(p.colsum + n0 + j, cs);
+                        if (n0 + j < p.colsum_n && cs != 0.f) atomicAdd(p.colsum + n0 + j, cs);
                     }
                     asm volatile("bar.sync 2, 128;" ::: "memory");
                 }
@@ -1220,13 +1222,16 @@ int rlppo_linear_dgrad(const uint16_t* dy, int64_t lddy, const uint16_t* wt, int
                        int64_t ldh, uint16_t* dx, int64_t lddx, float* db_below, int64_t M, int N, int K,
                        const rlppo_split* sp, void* stream) {
     RLPPO_REQUIRE_DEVICE();
-    RLPPO_CHECK_ARG(dy && wt && dx, "null pointer");
-    RLPPO_CHECK_ARG(K % 8 == 0 && lddx >= K && lddx % 8 == 0, "K and lddx must be multiples of 8");
-    RLPPO_CHECK_ARG(!hprev || ldh % 8 == 0, "ldh must be a multiple of 8");
-    // dX[M,K] = dY[M,N] * (W^T)[K,N]^T : the GEMM's "N" is K (in features), its contraction runs over N
+    RLPPO_CHECK_ARG(dy && wt && dx && K >= 1, "bad argument");
+    const int K8 = (K + 7) / 8 * 8;
+    RLPPO_CHECK_ARG(lddx >= K8 && lddx % 8 == 0, "lddx must be a multiple of 8 covering pad8(K)");
+    RLPPO_CHECK_ARG(!hprev || (ldh % 8 == 0 && ldh >= K8), "ldh must be a multiple of 8 covering pad8(K)");
+    // dX[M,K] = dY[M,N] * (W^T)[K,N]^T : the GEMM's "N" is K (in features), its contraction runs over N.  dX is
+    // written over pad8(K) columns (rows K.. of W^T read as zeros, so its padding columns get zeros); db_below
+    // takes only the K true columns.
     RowGemmParams p{};
-    p.M = M; p.N = K; p.K = N;
-    p.out = dx; p.ldo = lddx; p.mask = hprev; p.ldmask = ldh; p.colsum = db_below;
+    p.M = M; p.N = K8; p.K = N;
+    p.out = dx; p.ldo = lddx; p.mask = hprev; p.ldmask = ldh; p.colsum = db_below; p.colsum_n = K;
     return launch_rowgemm<EPI_RELU_MASK>(dy, lddy, wt, ldwt, K, p, 0, sp, static_cast<cudaStream_t>(stream));
 }
 

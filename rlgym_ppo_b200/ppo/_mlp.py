@@ -63,11 +63,11 @@ class Stack:
         self.linears = [m for m in model if isinstance(m, nn.Linear)]
         self.in_dim = self.linears[0].in_features
         self.hidden = [l.out_features for l in self.linears[:-1]]
+        # A hidden layer of width h runs on the device as pad8(h) units (16-byte rows for TMA): the extra units have zero
+        # weight rows and bias in wq, zero columns in the next layer's wq, hence zero activations and zero gradients.
+        # Only the bf16 operands and the workspaces are padded; parameters, gradients and state_dict keep true shapes.
+        self.hidden_pad = [ops.pad8(h) for h in self.hidden]
         self.out_dim = self.linears[-1].out_features
-        for h in self.hidden:
-            if h % 8 != 0:
-                raise ValueError(f"hidden layer width {h} is not a multiple of 8 (16-byte rows are required by the "
-                                 "TMA-staged tensor-core kernels)")
         self.in_pad = ops.pad8(self.in_dim)
         self.out_pad = ops.pad8(self.out_dim)
         self.n_params = sum(p.numel() for l in self.linears for p in (l.weight, l.bias))
@@ -208,11 +208,11 @@ class Stack:
 
     # ---- workspaces -------------------------------------------------------------------------------------
     def workspace(self, rows):
-        """Activation buffers for `rows` rows (grow-only): h[i] bf16 [rows, hidden_i]; two gradient ping-pong
+        """Activation buffers for `rows` rows (grow-only): h[i] bf16 [rows, pad8(hidden_i)]; two gradient ping-pong
         buffers as wide as the widest hidden layer; dz [rows, out_pad]."""
         if rows > self._ws_rows:
             cap = max(rows, 1)
-            wmax = max(self.hidden)
+            wmax = max(self.hidden_pad)
             if self.exact:
                 # split activations: forward tensors 3 parts, gradients 2 parts, each part pad64(width) columns (zero padded)
                 z = lambda parts, w: torch.zeros((cap, parts * ops.pad64(w)), dtype=BF16, device=self.device)  # noqa: E731
@@ -226,9 +226,9 @@ class Stack:
                 }
             else:
                 self._ws = {
-                    "h": [torch.empty((cap, h), dtype=BF16, device=self.device) for h in self.hidden],
+                    "h": [torch.empty((cap, h), dtype=BF16, device=self.device) for h in self.hidden_pad],
                     "d": [torch.empty((cap, wmax), dtype=BF16, device=self.device) for _ in range(2)],
-                    "dh": [torch.empty((cap, h), dtype=BF16, device=self.device) for h in self.hidden],
+                    "dh": [torch.empty((cap, h), dtype=BF16, device=self.device) for h in self.hidden_pad],
                     "dz": torch.zeros((cap, self.out_pad), dtype=BF16, device=self.device),
                     "z": torch.zeros((cap, 3 * ops.pad64(self.out_dim)), dtype=BF16, device=self.device),
                     "x": torch.zeros((cap, self.in_pad), dtype=BF16, device=self.device),
@@ -256,13 +256,15 @@ class Stack:
         prev, K, a_ps = x, self.in_dim, self.in_ps
         for i, h in enumerate(self.hidden):
             sp = ops.make_split(3, 3, 3, 3, a_ps, ops.pad64(K), ops.pad64(h)) if self.exact else None
-            ops.linear_fwd(prev, self.wq[i], self.b[i], ws["h"][i], h, K, True, M=M, split=sp)
+            n8 = self.hidden_pad[i]
+            ops.linear_fwd(prev, self.wq[i], self.b[i], ws["h"][i], n8, K, True, M=M, split=sp,
+                           bias_n=h if n8 != h else 0)
             prev, K, a_ps = ws["h"][i], h, ops.pad64(h)
         return prev
 
     def _d_buffers(self, ws):
-        """(dL/dH_last buffer, its part stride): ping-pong buffer 0, viewed at the last hidden width."""
-        hl = self.hidden[-1]
+        """(dL/dH_last buffer, its part stride): ping-pong buffer 0, viewed at the last (padded) hidden width."""
+        hl = self.hidden_pad[-1]
         d0 = ws["d"][0]
         if self.exact:
             return d0, ops.pad64(max(self.hidden))
@@ -359,8 +361,9 @@ class Stack:
         ops.policy_head_sample(h, self.wq[-1], self.b[-1], n_actions, hl, M=M, split=sp, **kw)
 
     def backward_hidden(self, x, M, ws, d_last, gw=None, gb=None):
-        """d_last = dL/dH_last (bf16 [>=M, hidden[-1]], already ReLU-masked).  Accumulates dW/db of every hidden
-        layer into gw / gb (default: the gradient arena; wgrad kernels add) and propagates through the stack."""
+        """d_last = dL/dH_last (bf16 [>=M, pad8(hidden[-1])], already ReLU-masked, padding columns zero).  Accumulates
+        dW/db of every hidden layer into gw / gb (default: the gradient arena; wgrad kernels add) and propagates through
+        the stack."""
         gw = self.gw if gw is None else gw
         gb = self.gb if gb is None else gb
         d = d_last
@@ -381,7 +384,8 @@ class Stack:
                     dx = nxt
                     sp_d = ops.make_split(2, 2, 2, 2, d_ps, ops.pad64(N), d_ps)
                 else:
-                    dx = nxt[:, :K] if nxt.shape[1] != K else nxt
+                    k8 = self.hidden_pad[i - 1]
+                    dx = nxt[:, :k8] if nxt.shape[1] != k8 else nxt
                     sp_d = None
                 ops.linear_dgrad(d, self.wt[i], inp, dx, N, K, M=M, db_below=gb[i - 1], split=sp_d)
                 d = dx
