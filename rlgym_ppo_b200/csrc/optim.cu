@@ -51,6 +51,13 @@ __global__ void seg_sumsq_kernel(const float* __restrict__ a, const float* __res
     if (threadIdx.x < segs.n) atomicAdd(out + threadIdx.x, s_part[threadIdx.x]);
 }
 
+// torch.nn.utils.clip_grad_norm_'s coefficient, clamp(max_norm / (total_norm + 1e-6), max=1).  torch.clamp keeps a NaN
+// (a NaN anywhere in the segment's gradient turns the whole segment's update into NaN); fminf would return 1 instead.
+__device__ __forceinline__ float clip_coef(float max_norm, float total_norm) {
+    const float c = max_norm / (total_norm + 1e-6f);
+    return c > 1.0f ? 1.0f : c;
+}
+
 // step counters are bumped by a one-thread prologue kernel so every Adam thread sees the same value
 __global__ void bump_steps_kernel(int64_t* step_count, int n_seg) {
     if (threadIdx.x < n_seg) step_count[threadIdx.x] += 1;
@@ -73,7 +80,7 @@ __global__ void clip_adam_kernel(float* __restrict__ p, const float* __restrict_
         const int k = threadIdx.x;
         // torch.nn.utils.clip_grad_norm_: coef = max_norm / (total_norm + 1e-6), clamped to 1
         const float total_norm = sqrtf(sqnorm[k]);
-        s_coef[k] = fminf(max_norm / (total_norm + 1e-6f), 1.0f);
+        s_coef[k] = clip_coef(max_norm, total_norm);
         const double t = (double)step_count[k];
         const double bc1 = 1.0 - pow(beta1d, t);
         const double bc2 = 1.0 - pow(beta2d, t);
@@ -388,7 +395,7 @@ norm_clip_adam_kernel(float* __restrict__ p, const float* __restrict__ g, float*
             t = rlppo::warp_sum(t);
             if (lane == 0) {
                 // torch.nn.utils.clip_grad_norm_: coef = max_norm / (total_norm + 1e-6), clamped to 1
-                s_coef[k] = fminf(max_norm / (sqrtf(t) + 1e-6f), 1.0f);
+                s_coef[k] = clip_coef(max_norm, sqrtf(t));
                 if (blockIdx.x == 0) {
                     if (sqnorm_out != nullptr) sqnorm_out[k] = t;
                     step_count[k] = (int64_t)s_t[k];
