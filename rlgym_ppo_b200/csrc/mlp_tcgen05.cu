@@ -1083,7 +1083,9 @@ __global__ void colsum_kernel(const uint16_t* __restrict__ dy, int64_t ld, int64
     db += c0;
     n8 = min(slice, n8 - c0);
     N = min(n8, N - c0);
-    extern __shared__ float s_acc[];  // n8 floats (N rounded up to 8; the padding columns of dY are zero)
+    // n8 floats (N rounded up to 8): 16-byte loads also sum dY's padding columns, whatever they hold; only the N true
+    // columns are stored
+    extern __shared__ float s_acc[];
     for (int i = threadIdx.x; i < n8; i += blockDim.x) s_acc[i] = 0.f;
     __syncthreads();
     const int groups = n8 >> 3;                      // 8 columns (16 B) per thread
@@ -1341,7 +1343,7 @@ int rlppo_linear_wgrad(const uint16_t* dy, int64_t lddy, const uint16_t* x, int6
         RLPPO_CHECK_ARG(n8 <= lddy, "bias-gradient pass needs N padded to 8 within lddy");
         // at most 2048 columns (256 threads of 8) per block: wider dY is split over blockIdx.y
         const unsigned col_slices = (unsigned)((n8 / 8 + 255) / 256);
-        // padded columns of dY are zero by construction, so summing n8 columns is safe; only N are written
+        // the pass sums n8 columns but writes only N, so dY's padding columns need not be zero
         // ~8 blocks per SM: with 512 rows per block a 50 000-row dY gave 98 blocks of 512 dependent 16-byte loads per
         // thread -- 2 TB/s, and at the wide nets (N = 2048) the pass cost 72 % of the weight-gradient GEMM it follows
         int64_t rows_per_block = (M + (int64_t)num_sms() * 8 - 1) / ((int64_t)num_sms() * 8);

@@ -18,9 +18,17 @@ value to the set of reals that round to the stored bf16 value, over e.
 
 Measured on an NVIDIA B200 (1000 W power limit), largest over every shape as a fraction of each bound: H 0.105,
 dH 0.354, dz 0.933 (its bound's 2^-8 |dz| term is the bf16 rounding itself), logp_out 0.042, values_out 0.691, gw_head
-0.95 (M = 1: the value tail's one ambiguous activation sits at an end of its interval); wgrad_multi rel-L2 <= 1.1e-6
-against 1e-4.  These maxima, and the file's 18 s run time there, were taken when the file also re-ran the duo shapes in
-the single-tile form and in a CTA-pair variant of it that the library no longer has.
+0.95 (M = 1: the value tail's one ambiguous activation sits at an end of its interval).  These maxima, and the file's
+18 s run time there, were taken when the file also re-ran the duo shapes in the single-tile form and in a CTA-pair
+variant of it that the library no longer has.  wgrad_multi's dW and db, per element against (sqrt(M) + 2) u of their
+sums of magnitudes (check_wgrad), came to at most 0.704 of that bound on the same GPU and power limit: the policy
+head's dW (90 x 256, duo 256x3 net) at M = 129, at an element whose 129 terms dz H are almost all of one sign
+(|sum t| / sum |t| = 0.985: H >= 0 after the ReLU, and that logit's dz column keeps its sign).  Same-signed terms make
+the partial sums grow to sum |t|, so every fp32 rounding is a fraction of the whole sum and the random walk of them
+comes near the sqrt(M) u sum |t| estimate; random-signed terms keep the partial sums near sqrt(M) |t| (the random
+operands of test_bf16_gemm_gpu.py reach 0.0085 on the same kernel).  The policy heads' dW at M = 127..129 give the
+largest values (0.46 to 0.70); the column sums db at most 0.116.  The atomicAdd order moves only the last few
+roundings (three row splits at M = 129).
 
 Layout edges the harness sets up on purpose:
   - x has a row stride past in_dim, and 2 rows past M; both are NaN.  They are outside the x tensor map.
@@ -49,7 +57,7 @@ import torch
 
 from oracle import ref_oracle as O
 from parity_helpers import philox_rows, philox_uniform
-from test_split_kernels_gpu import _prob_bound
+from test_split_kernels_gpu import _prob_bound, gemm_err
 
 pytestmark = pytest.mark.gpu
 
@@ -511,8 +519,10 @@ def check_untouched(net, outs, M, d):
 
 def check_wgrad(items, M, rec):
     """rlppo_wgrad_multi on the stored fused outputs: dW = dy^T x and db = column sums of dy against the fp64
-    contraction of the same stored bf16 operands, rel-L2 < 1e-4 (test_wgrad_multi's bound).  Control: the reference
+    contraction of the same stored bf16 operands, per element: |dW - ref| <= (sqrt(M) + 2) u sum_m |dy x| (the module
+    docstring's e with the contraction over M rows; gemm_err), db likewise with sum_m |dy|.  Control: the reference
     without the rows of the 128-row tile holding row M / 2 (a kernel that skipped one tile) fails it."""
+    bound = (math.sqrt(M) + 2) * U
     t0 = (M // 2) // 128 * 128
     keep = torch.ones(M, dtype=torch.bool, device=DEV)
     keep[t0:t0 + 128] = False
@@ -522,12 +532,12 @@ def check_wgrad(items, M, rec):
         if float(ref.abs().max()) == 0.0:        # a one-action head: dz is identically zero
             assert float(dw.abs().max()) == 0.0 and float(db.abs().max()) == 0.0
             continue
-        e_w = float((dw.double() - ref).norm() / ref.norm())
-        e_b = float((db.double() - ref_db).norm() / ref_db.norm())
-        assert e_w < 1e-4 and e_b < 1e-4, (N, K, e_w, e_b)
-        ctl = a[keep].t() @ b[keep]
-        assert float((dw.double() - ctl).norm() / ctl.norm().clamp_min(1e-300)) >= 1e-4, "wgrad control passed"
-        rec["wgrad rel-L2"] = max(rec.get("wgrad rel-L2", 0.0), e_w, e_b)
+        absum = a.abs().t() @ b.abs() + 1e-300   # (+ 1e-300: an entry with no terms must come out exactly zero)
+        e_w = gemm_err(dw.double(), ref, absum) / bound
+        e_b = gemm_err(db.double(), ref_db, a.abs().sum(0) + 1e-300) / bound
+        assert e_w <= 1.0 and e_b <= 1.0, (N, K, e_w, e_b)
+        assert gemm_err(dw.double(), a[keep].t() @ b[keep], absum) > bound, "wgrad control passed"
+        rec["wgrad"] = max(rec.get("wgrad", 0.0), e_w, e_b)
 
 
 def run_and_check(ops, nets, x, M, d, tag):
